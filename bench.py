@@ -2,7 +2,8 @@
 """bench.py — headline metric of BASELINE.json: rays/sec at 512x512 with 64 coarse + 128 fine samples per ray.
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched under torch.distributed.run)
-    python bench.py --impl reference ...                       (the reference's own implementation on the host cores)
+    python bench.py --impl reference ...                       (the reference algorithm on the host cores)
+    python bench.py ... --dump-outputs DIR                     (also write the last timed step's outputs to DIR/<name>.npy)
 
 Headline (`value`, `e2e`, `roofline`): one step = one full 512x512 frame per GPU (BASELINE config 2; with N GPUs config 5:
 N concurrent frames with different expression codes, all-gathered into one [N,512,512,3] video tensor) => weak scaling,
@@ -14,9 +15,8 @@ value = N*H*W*K / time.  Synthetic per-frame pose / expression / latent / backgr
            background in, 11 floats per ray out, copies inside the timed region (N>1: the same all-gather as `value`).
 `roofline`: dominant kernel = the render kernel; achieved = algorithmic FLOP per launch (1,100,032 FLOP per MLP evaluation x
            (2*Nc+Nf) evaluations per ray x rays) / its CUDA-event time; peak from MEASURED_PEAKS.json.
-`cpu_baseline`: the reference's own run_one_iter_of_nerf (staged copy, oracle/stage_reference.py; kind "reference") — or
-           the oracle port when no reference tree is reachable — on the host cores for a 64x64 crop.
-`gpu_baseline`: the same unmodified reference on this GPU through torch CUDA (TF32 off): what a user of the reference gets.
+`cpu_baseline`: the reference algorithm (oracle/nerface_oracle.py, the bit-exact port of its run_one_iter_of_nerf) on the host
+           cores for a 64x64 crop.
 
 Sub-records in the same JSON line (SURVEY.md §8e, the split `north_star` names):
 `rows`, `rows_1024`: ONE frame (512x512 64c+128f; 1024x1024 128c+256f = BASELINE config 4) sharded by pixel rows over the
@@ -35,6 +35,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -57,11 +58,18 @@ def parse():
     ap.add_argument("--num-coarse", type=int, default=64)
     ap.add_argument("--num-fine", type=int, default=128)
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--no-extras", action="store_true", help="headline only: skip rows / train / gpu_baseline / exact / stress records")
-    ap.add_argument("--extras", default="all", help="comma list out of rows,rows_1024,train,single (exact / stress / gpu_baseline); default all")
+    ap.add_argument("--no-extras", action="store_true", help="headline only: skip rows / train / exact / stress records")
+    ap.add_argument("--extras", default="all", help="comma list out of rows,rows_1024,train,single (exact / stress); default all")
     ap.add_argument("--train-impl", default=os.environ.get("NFB_TRAIN_IMPL", "fused"), choices=["fused", "dropin"])
     ap.add_argument("--no-train-graph", action="store_true", help="fused training step launch by launch instead of one CUDA graph replay")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy, "
+                    "float32: rank 0's 7 per-ray outputs and, with N>1 GPUs, the all-gathered [N,H*W,3] video (--impl ours only)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return a
 
 
 def peaks():
@@ -108,26 +116,14 @@ class ClockSampler(threading.Thread):
 
 
 # ------------------------------------------------------------------------------------------------
-# the reference on the host cores (cpu_baseline / --impl reference) and on the GPU through torch (gpu_baseline)
-def reference_frame_crop(frame_index, H, W, crop, nc, nf, threads, device="cpu"):
-    """(run, rays, kind): the reference algorithm on a crop x crop centre block of the synthetic frame.  kind "reference" =
-    the unmodified reference package (staged copy / /root/reference); "port" = oracle/nerface_oracle.py."""
+# the reference algorithm on the host cores (cpu_baseline / --impl reference)
+def reference_frame_crop(frame_index, H, W, crop, nc, nf, threads):
+    """(run, rays): the reference algorithm (oracle/nerface_oracle.py) on a crop x crop centre block of the synthetic frame."""
     import nerface_oracle as O
-    import ref_loader
-    if device == "cpu":
-        torch.set_num_threads(threads)
+    torch.set_num_threads(threads)
     fr = O.synthetic_frame(frame_index, H, W)
     pc, pf = O.random_init_params(100), O.random_init_params(101)
     r0, c0 = (H - crop) // 2, (W - crop) // 2
-    ref = None
-    try:
-        ref = ref_loader.load_reference()
-    except Exception as e:  # a broken staged copy must not take the bench line down
-        sys.stderr.write(f"reference import failed ({e!r}); using the oracle port\n")
-    if ref is not None:
-        run, rays = ref_loader.reference_renderer(ref, fr, pc, pf if nf > 0 else None, H, W, slice(r0, r0 + crop), slice(c0, c0 + crop),
-                                                  nc, nf, device=device)
-        return run, rays, "reference"
     ro, rd = O.ray_bundle(H, W, fr["intrinsics"], fr["pose"])
     ro, rd = ro[r0:r0 + crop, c0:c0 + crop].contiguous(), rd[r0:r0 + crop, c0:c0 + crop].contiguous()
     bg = fr["bg"][r0:r0 + crop, c0:c0 + crop].reshape(-1, 3)
@@ -136,7 +132,7 @@ def reference_frame_crop(frame_index, H, W, crop, nc, nf, threads, device="cpu")
     def run():
         with torch.no_grad():
             return O.run_one_iter(ro, rd, pc, pf if nf > 0 else None, s, NEAR, FAR, fr["expr"], fr["latent"], bg, "validation")
-    return run, crop * crop, "port"
+    return run, crop * crop
 
 
 def pick_threads(H, W, nc, nf):
@@ -147,7 +143,7 @@ def pick_threads(H, W, nc, nf):
     for th in sorted({cores, 64, 32, 16, 8}):
         if th > cores:
             continue
-        run, _, _ = reference_frame_crop(0, H, W, 16, nc, nf, th)
+        run, _ = reference_frame_crop(0, H, W, 16, nc, nf, th)
         run()
         t0 = time.perf_counter()
         run()
@@ -157,8 +153,7 @@ def pick_threads(H, W, nc, nf):
     return best[0]
 
 
-CPU_SAMPLE = {"reference": "the UNMODIFIED reference run_one_iter_of_nerf (nerf/train_utils.py:165-290, staged copy baseline/_ref, torch CPU FP32)",
-              "port": "oracle/nerface_oracle.py (bit-exact port of the reference, torch CPU FP32)"}
+CPU_SAMPLE = "oracle/nerface_oracle.py (bit-exact port of the reference, torch CPU FP32)"
 
 
 def reference_arm(a):
@@ -166,7 +161,7 @@ def reference_arm(a):
     if rank != 0:
         return
     cores = pick_threads(a.height, a.width, a.num_coarse, a.num_fine)
-    run, rays, kind = reference_frame_crop(0, a.height, a.width, 64, a.num_coarse, a.num_fine, cores)
+    run, rays = reference_frame_crop(0, a.height, a.width, 64, a.num_coarse, a.num_fine, cores)
     for _ in range(max(1, min(a.warmup, 1))):
         run()
     times = []
@@ -181,44 +176,35 @@ def reference_arm(a):
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": f"person_1-shaped eval {a.height}x{a.width}, {a.num_coarse}c+{a.num_fine}f, 76-dim expr + 32-dim latent",
                        "sample": "64x64 centre crop of the frame per step"},
-            "cpu_baseline": {"value": value, "unit": "rays/s", "cores": cores, "host_cores": os.cpu_count(), "kind": kind,
-                             "sample": CPU_SAMPLE[kind] + " on a 64x64 crop per step"},
+            "cpu_baseline": {"value": value, "unit": "rays/s", "cores": cores, "host_cores": os.cpu_count(),
+                             "sample": CPU_SAMPLE + " on a 64x64 crop per step"},
             "e2e": {"value": value, "unit": "rays/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}
     print(json.dumps(line), flush=True)
 
 
-def gpu_baseline(H, W, nc, nf, dev):
-    """The unfused reference on this GPU through torch CUDA, TF32 off (SURVEY.md §8d second baseline): full frame,
-    the shipped YAML's validation chunksize (65536 rays)."""
-    import nerface_oracle as O
-    import ref_loader
-    try:
-        ref = ref_loader.load_reference()
-        if ref is None:
-            return {"unavailable": "no reference tree (baseline/_ref not staged)"}
-        torch.backends.cuda.matmul.allow_tf32 = False
-        torch.backends.cudnn.allow_tf32 = False
-        fr = O.synthetic_frame(0, H, W)
-        run, rays = ref_loader.reference_renderer(ref, fr, O.random_init_params(100), O.random_init_params(101), H, W,
-                                                  slice(0, H), slice(0, W), nc, nf, device=dev, chunksize=65536)
-        run()
-        torch.cuda.synchronize()
-        ts = []
-        for _ in range(2):
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            out = run()
-            e1.record()
-            torch.cuda.synchronize()
-            ts.append(e0.elapsed_time(e1))
-        ms = min(ts)
-        return {"value": rays / (ms * 1e-3), "unit": "rays/s", "ms_per_frame": ms, "kind": "reference",
-                "sample": f"unmodified reference run_one_iter_of_nerf on torch CUDA FP32 (TF32 off), full {H}x{W} frame, {nc}c+{nf}f, "
-                          "chunksize 65536, best of 2 after 1 warm-up",
-                "peak_mem_gb": torch.cuda.max_memory_allocated() / 2 ** 30, "_out": out}
-    except Exception as e:
-        return {"unavailable": repr(e)[:200]}
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, v, n, video=None):
+    """The outputs of one render_camera call as out_dir/<name>.npy (float32, [n] or [n,3]) and, when given, the all-gathered
+    [N,n,3] video as video.npy.  Past DUMP_LIMIT_BYTES in all, a fixed seeded sample of rays (the same for every frame of the
+    video) is written instead, with their indices in ray_index.npy (float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    per_ray = 4 * sum(v[k][:1].numel() for k in NAMES) + (4 * video.shape[0] * video.shape[2] if video is not None else 0)
+    budget = DUMP_LIMIT_BYTES - 4096  # room for the .npy headers
+    idx = None
+    if per_ray * n > budget:
+        keep = budget // (per_ray + 8)
+        idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        np.save(os.path.join(out_dir, "ray_index.npy"), idx.double().numpy())
+        idx = idx.to(v[NAMES[0]].device)
+    for k in NAMES:
+        t = v[k] if idx is None else v[k].index_select(0, idx)
+        np.save(os.path.join(out_dir, k + ".npy"), t.float().cpu().numpy())
+    if video is not None:
+        t = video if idx is None else video.index_select(1, idx)
+        np.save(os.path.join(out_dir, "video.npy"), t.float().cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------------
@@ -509,6 +495,7 @@ def main():
     out_host = torch.empty((11 * n,), dtype=torch.float32).pin_memory()
     video = torch.empty((world, n, 3), device=dev) if world > 1 else None
     rgb_stage = torch.empty((n, 3), device=dev) if world > 1 else None
+    last_out = {}
 
     def step_resident(i, ev=None):
         fr, d = frames[i % len(frames)], dev_frames[i % len(frames)]
@@ -521,6 +508,7 @@ def main():
             ev[1].record()
         if world > 1:
             dist.all_gather_into_tensor(video.view(-1), v["rgb_fine"].reshape(-1))
+        last_out["v"] = v
         return v
 
     def step_host(i):
@@ -562,6 +550,9 @@ def main():
     ms_total, kernel_ms, wall = timed(step_resident, a.steps, kernel_events=True)
     launches = eng.launch_count() - l0
     clocks = sampler.stop() if sampler else None
+    if a.dump_outputs and rank == 0:
+        torch.cuda.synchronize()
+        dump_outputs(a.dump_outputs, last_out["v"], n, video)
     ms_e2e, _, _ = timed(lambda i: step_host(i), a.steps)
 
     # ---- in-run parity (rank 0): two image rows of the last rendered frame against the oracle
@@ -616,21 +607,6 @@ def main():
             extras["exact_mode_rays_per_s"] = 3 * n / (e0.elapsed_time(e1) * 1e-3)
             extras["stress"] = stress_psnr(c, a.precision)
             eng.sync_weights(mc, mf)
-            gb = gpu_baseline(H, W, nc, nf, dev)
-            ref_out = gb.pop("_out", None)
-            if ref_out is not None:  # PSNR / max-abs of OUR frame vs the reference's own CUDA output (same frame 0)
-                fr0, d0 = O.synthetic_frame(0, H, W), None
-                eng.set_frame(fr0["expr"].to(dev), fr0["latent"].to(dev))
-                v = eng.render_camera(fr0["pose"], fr0["intrinsics"], H, W, 0, H, NEAR, FAR, nc, nf,
-                                      background=fr0["bg"].reshape(-1, 3).to(dev).contiguous(), out=out_buf, precision=a.precision)
-                torch.cuda.synchronize()
-                d = (v["rgb_fine"].reshape(H, W, 3) - ref_out[3]).float()
-                mse_f = float((d ** 2).mean())
-                gb["ours_vs_reference_cuda_full_frame"] = {
-                    "psnr_rgb_fine_db": 99.0 if mse_f == 0 else min(99.0, -10.0 * math.log10(mse_f)),
-                    "max_abs": max(float((v[k].reshape(r.shape) - r).abs().max()) for k, r in zip(NAMES, ref_out)), "rays": n}
-                del ref_out
-            extras["gpu_baseline"] = gb
 
     if rank == 0:
         rays_total = n * world * a.steps
@@ -655,15 +631,15 @@ def main():
         cpu = None
         if not a.no_cpu_baseline:
             cores = pick_threads(H, W, nc, nf)
-            run, crays, kind = reference_frame_crop(0, H, W, 64, nc, nf, cores)
+            run, crays = reference_frame_crop(0, H, W, 64, nc, nf, cores)
             run()
             ts = []
             for _ in range(3):
                 t0 = time.perf_counter()
                 run()
                 ts.append(time.perf_counter() - t0)
-            cpu = {"value": crays / (sorted(ts)[1]), "unit": "rays/s", "cores": cores, "kind": kind, "host_cores": os.cpu_count(),
-                   "sample": CPU_SAMPLE[kind] + ", best of 8/16/32/64/all intra-op threads, 64x64 centre crop, median of 3"}
+            cpu = {"value": crays / (sorted(ts)[1]), "unit": "rays/s", "cores": cores, "host_cores": os.cpu_count(),
+                   "sample": CPU_SAMPLE + ", best of 8/16/32/64/all intra-op threads, 64x64 centre crop, median of 3"}
         line = {
             "metric": "rays/sec at 512x512 (64c+128f samples)", "value": value, "unit": "rays/s", "n_gpus": world,
             "steps": a.steps, "warmup": a.warmup, "ms_per_step": ms_total / a.steps, "higher_is_better": True,

@@ -1,7 +1,7 @@
 """Golden vectors for the post-render products (SURVEY.md §8f rank 4), produced by the UNMODIFIED reference functions of
 eval_transformed_rays.py — torch_normal_map (:84-119), cast_to_image (:184-192), cast_to_disparity_image (:195-198) — on the
 disparity / weights / colours the oracle renders for a synthetic 64x64 frame with opaque-stress weights (so the disparity map
-has structure and w_last crosses the 0.22 cleaning threshold).  Build container only (needs /root/reference or the staged copy).
+has structure and w_last crosses the 0.22 cleaning threshold).  Needs the copy oracle/stage_reference.py stages into oracle/_ref.
 
     python oracle/make_golden_products.py        ->  tests/golden_products/frame_products_64.npz
 """

@@ -1,7 +1,7 @@
 """Import the UNMODIFIED reference `nerf` package (test / baseline infrastructure only — never from the product).
 
-Looks for the reference tree at /root/reference (build container) and then at baseline/_ref (the byte-for-byte copy
-staged by oracle/stage_reference.py, which is what exists on the GPU box).  The package is loaded under the alias
+Looks for the reference tree in oracle/_ref (the byte-for-byte copy staged by oracle/stage_reference.py; a script may point
+CANDIDATES elsewhere).  The package is loaded under the alias
 `nerf_reference`, so it never collides with this repository's drop-in package, which is importable as `nerf`.
 
 Hot-path-unused dependencies that are absent from the image (SURVEY.md §8c: pytorch3d, torchsearchsorted, imageio) get
@@ -15,7 +15,7 @@ import types
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-CANDIDATES = ["/root/reference", os.path.join(ROOT, "baseline", "_ref")]
+CANDIDATES = [os.path.join(ROOT, "oracle", "_ref")]
 NP = os.path.join("nerface_code", "nerf-pytorch")
 
 

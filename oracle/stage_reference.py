@@ -1,20 +1,18 @@
-"""Stage the UNMODIFIED reference files of the hot path for the GPU box (test / baseline infrastructure, not product).
+"""Stage the UNMODIFIED reference files of the hot path (golden-data and tooling infrastructure, not product).
 
-`/root/reference` exists only in the build container; the GPU box receives a snapshot of this repository.  This
-recipe copies — byte for byte, nothing edited — the reference's `nerf` package, the two CLI scripts that call the
-path and the shipped paper-model YAML into `baseline/_ref/` (git-ignored: reference sources never enter this
-repository's history; NOT gpurun-ignored: the directory travels with the snapshot).  It is the offline "install" of a
-reference that has no setup.py.  Users of the staged copy:
+This recipe copies — byte for byte, nothing edited — the reference's `nerf` package, the two CLI scripts that call the
+path and the shipped paper-model YAML from a reference checkout into `oracle/_ref/` (git-ignored: reference sources never
+enter this repository's history; the directory can be carried to a GPU machine together with a copy of the tree).  It is
+the offline "install" of a reference that has no setup.py.  Users of the staged copy (through oracle/ref_loader.py):
 
-  * bench.py --impl reference and the `cpu_baseline` / `gpu_baseline` legs (`kind: "reference"`): the reference's own
-    run_one_iter_of_nerf on the host cores / on the B200 through torch CUDA with TF32 off;
-  * tests: the CPU oracle against the live reference functions;
-  * run_reference_script.py: the unmodified train_transformed_rays.py / eval_transformed_rays.py with this repo's
-    drop-in `nerf` package first on sys.path.
+  * run_reference_script.py (tools/run_reference_clis.py): the unmodified train_transformed_rays.py /
+    eval_transformed_rays.py with this repo's drop-in `nerf` package first on sys.path;
+  * oracle/make_golden_reference_checks.py --ref oracle/_ref --cuda-products: the reference's post-render functions on a GPU.
 
-    python oracle/stage_reference.py [--ref /root/reference]
+    python oracle/stage_reference.py --ref PATH_TO_REFERENCE_CHECKOUT
 
-`__graft_entry__.build()` runs it whenever /root/reference is present.
+Run it by hand where the reference tree is present; the build does not run it, and no test needs the staged copy (the tests
+compare with golden data made by oracle/make_golden_reference_checks.py).
 """
 import argparse
 import hashlib
@@ -24,7 +22,7 @@ import shutil
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-DEST = os.path.join(ROOT, "baseline", "_ref")
+DEST = os.path.join(ROOT, "oracle", "_ref")
 NP = os.path.join("nerface_code", "nerf-pytorch")
 FILES = [os.path.join(NP, "nerf", f) for f in (
     "__init__.py", "cfgnode.py", "load_blender.py", "load_flame.py", "load_llff.py", "models.py", "nerf_helpers.py",
@@ -33,9 +31,9 @@ FILES = [os.path.join(NP, "nerf", f) for f in (
     os.path.join(NP, "config", "dave", "dave_dvp_lcode_fixed_bg_512_paper_model.yml")]
 
 
-def stage(ref_root="/root/reference", dest=DEST):
+def stage(ref_root, dest=DEST):
     """Copy FILES from ref_root to dest (same relative paths) + MANIFEST.json with their sha256.  Returns dest, or None
-    when the reference tree is absent (GPU box: the staged copy made in the build container is used as is)."""
+    when the reference tree is absent."""
     if not os.path.isdir(os.path.join(ref_root, NP)):
         return None
     manifest = {}
@@ -52,7 +50,7 @@ def stage(ref_root="/root/reference", dest=DEST):
 
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
-    ap.add_argument("--ref", default="/root/reference")
+    ap.add_argument("--ref", required=True, help="root of the reference checkout (the directory holding nerface_code/)")
     a = ap.parse_args()
     d = stage(a.ref)
     print(d if d else f"{a.ref} not found: nothing staged")

@@ -1,11 +1,14 @@
 """Pins the floating-point reference of the fused backward kernels (tests/torch_reference.py: render_at_depths, what
 tests/test_backward_gpu.py compares the CUDA gradients with) to the UNMODIFIED reference's own autograd: the training loss of
-train_transformed_rays.py:355-389 (mse of the coarse and the fine colour against the target) is back-propagated through the live
+train_transformed_rays.py:355-389 (mse of the coarse and the fine colour against the target) back-propagated through the
 reference's run_one_iter_of_nerf (mode "train", perturbation and sigma noise on, background image) and through render_at_depths at
 the depths the reference sampled; parameter gradients of both networks and the latent-code gradient must agree to FP32 rounding.
 
 So the chain for SURVEY.md §8 row a11 is: CUDA backward  <->  torch_reference (GPU tests)  <->  reference autograd (this file).
-Needs the reference tree (/root/reference or the staged copy baseline/_ref); CPU only."""
+The reference's rays, draws, outputs, loss and gradients are stored in tests/golden/reference_checks/backward.npz by
+oracle/make_golden_reference_checks.py: the latent gradient and the small parameter gradients in full, each larger one as its
+largest magnitude, its sum of squares and a seeded sample of entries.  CPU only."""
+import math
 import os
 import sys
 
@@ -17,45 +20,33 @@ import nerface_oracle as O
 import torch_reference as TR
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle"))
-import make_golden as MG  # noqa: E402  (only its Recorder of torch.rand / torch.randn draws)
-import ref_loader  # noqa: E402
-
-pytestmark = pytest.mark.skipif(ref_loader.reference_root() is None, reason="no reference tree (run oracle/stage_reference.py)")
+import make_golden_reference_checks as G  # noqa: E402
 
 
-@pytest.mark.parametrize("stress,white,use_bg", [(False, False, True), (True, False, True), (True, True, False)],
-                         ids=["random_init", "opaque_stress", "opaque_stress_white_nobg"])
-def test_torch_reference_gradients_equal_reference_autograd(stress, white, use_bg, monkeypatch):
-    ref = ref_loader.load_reference()
-    # `sigma_a[:, -1] += 1e-6` (volume_rendering_utils.py:53) writes into the output of F.relu in place, which torch >= 2 refuses to
-    # differentiate through; the one patch BASELINE.md §4 names for gradient baselines (ref_loader.load_reference(relu_clone=True),
-    # also what the launcher of the unmodified train script installs): F.relu returns a copy — same values, same gradients.
+@pytest.mark.parametrize("name", list(G.BACKWARD_CASES))
+def test_torch_reference_gradients_equal_reference_autograd(name, monkeypatch):
+    stress, white, use_bg = G.BACKWARD_CASES[name]
+    gold = np.load(os.path.join(G.OUT, "backward.npz"))
+    g = lambda k: torch.from_numpy(gold[f"{name}/{k}"])  # noqa: E731
+    # the reference's gradients were taken with F.relu returning a copy (`sigma_a[:, -1] += 1e-6`, volume_rendering_utils.py:53,
+    # writes into its output in place, which torch >= 2 refuses to differentiate through; BASELINE.md §4): same values, same gradients
     orig_relu = torch.nn.functional.relu
     monkeypatch.setattr(torch.nn.functional, "relu", lambda x, *a, **k: orig_relu(x).clone())
     H, W, nc, nf, near, far = 2, 5, 64, 64, 0.2, 0.8
     s = O.Sampling(nc, nf, True, 0.1, white, 2048)
     fr = O.synthetic_frame(31, H, W)
     pc, pf = O.random_init_params(100, stress), O.random_init_params(101, stress)
-    ro, rd = ref.get_ray_bundle(H, W, np.array(fr["intrinsics"]), fr["pose"][:3, :4])
-    ro, rd = ro.reshape(-1, 3).clone(), rd.reshape(-1, 3).clone()
+    ro, rd = g("ro"), g("rd")
+    o_ro, o_rd = O.ray_bundle(H, W, fr["intrinsics"], fr["pose"])
+    assert torch.equal(ro, o_ro.reshape(-1, 3)) and torch.equal(rd, o_rd.reshape(-1, 3))
     n = ro.shape[0]
     bg = fr["bg"].reshape(-1, 3) if use_bg else None
     target = torch.rand(n, 3, generator=torch.Generator().manual_seed(5))
-
-    # ---- the reference: forward in train mode with gradients, the script's loss, autograd
-    mc, mf = ref_loader.build_model(ref, pc), ref_loader.build_model(ref, pf)
-    lat_ref = fr["latent"].clone().requires_grad_(True)
-    cfg = ref_loader.make_cfg(ref, nc, nf, True, 0.1, white, 2048, "train", near, far)
-    torch.manual_seed(77)
-    with MG.Recorder() as rec:
-        out = ref.run_one_iter_of_nerf(H, W, fr["intrinsics"], mc, mf, ro.clone(), rd.clone(), cfg, mode="train",
-                                       encode_position_fn=ref.get_embedding_function(10, True, True),
-                                       encode_direction_fn=ref.get_embedding_function(4, False, True),
-                                       expressions=fr["expr"], background_prior=bg, latent_code=lat_ref)
-    loss_ref = torch.nn.functional.mse_loss(out[0][..., :3], target) + torch.nn.functional.mse_loss(out[3][..., :3], target)
-    loss_ref.backward()
-    draws = [t for _, t in rec.draws]
-    assert len(draws) == 4  # rand[N,Nc], randn[N,Nc], rand[N,Nf], randn[N,Nc+Nf] (train_utils.py:69-76, 105-119)
+    out = [g(f"out{i}") for i in range(7)]
+    loss_ref = float(gold[f"{name}/loss"])
+    # rand[N,Nc], randn[N,Nc], rand[N,Nf], randn[N,Nc+Nf] (train_utils.py:69-76, 105-119)
+    draws = [g(f"draw{j}") for j in range(4)]
+    assert f"{name}/draw4" not in gold
     noise = O.Noise(t_rand=draws[0], n_c=draws[1], u=draws[2], n_f=draws[3])
 
     # ---- the depths the reference sampled (the oracle reproduces the forward bit for bit, test_oracle_vs_reference_cpu.py)
@@ -64,7 +55,7 @@ def test_torch_reference_gradients_equal_reference_autograd(stress, white, use_b
     with torch.no_grad():
         o_out = O.render_chunk(rays, pc, pf, s, fr["expr"], fr["latent"], bg, noise, extras=ex)
     for a, b in zip(out, o_out):
-        assert torch.equal(a.detach(), b)
+        assert torch.equal(a, b)
 
     # ---- the backward tests' floating-point reference at those depths
     lc = {k: v.clone().requires_grad_(True) for k, v in pc.items()}
@@ -73,26 +64,35 @@ def test_torch_reference_gradients_equal_reference_autograd(stress, white, use_b
     got = TR.render_at_depths(rays, lc, lf, fr["expr"], lat, ex["z_coarse"], ex["z_fine"], near, far, 0.1,
                               {"n_c": noise.n_c, "n_f": noise.n_f}, white, bg, None)
     for i in (0, 1, 2, 3, 4, 5, 6):
-        assert float((got[i].detach() - out[i].detach()).abs().max()) <= 2e-6 * max(1.0, float(out[i].detach().abs().max())), i
+        assert float((got[i].detach() - out[i]).abs().max()) <= 2e-6 * max(1.0, float(out[i].abs().max())), i
     loss = torch.nn.functional.mse_loss(got[0], target) + torch.nn.functional.mse_loss(got[3], target)
-    assert abs(float(loss.detach()) - float(loss_ref.detach())) <= 1e-7
+    assert abs(float(loss.detach()) - loss_ref) <= 1e-7
     loss.backward()
 
-    def close(a, b, what):
-        scale = max(float(b.abs().max()), 1e-12)
+    def close(a, b, what, scale=None):
+        scale = max(float(b.abs().max()), 1e-12) if scale is None else scale
         assert float((a - b).abs().max()) <= 2e-5 * scale, (what, float((a - b).abs().max()), scale)
 
-    n_checked = 0
-    for leaves, model, tag in ((lc, mc, "coarse"), (lf, mf, "fine")):
-        named = dict(model.named_parameters())
-        for k in TR.PARAM_ORDER:
-            g_ref = named[k].grad
-            if k.startswith("layers_dir.3"):  # built by the reference model but never used by its forward (models.py:257)
-                assert g_ref is None and leaves[k].grad is None
+    # max |g_ours - g_ref| <= 2e-5 max|g_ref| over every entry implies it on the stored entries, for the largest magnitudes and,
+    # summed over the n entries, |  ||g_ours|| - ||g_ref||  | <= sqrt(n) 2e-5 max|g_ref|
+    max_abs, sum_sq, stored = gold[f"{name}/grad_max_abs"], gold[f"{name}/grad_sum_sq"], torch.from_numpy(gold[f"{name}/grad_sample"])
+    n_checked, at = 0, 0
+    for m_i, (leaves, tag) in enumerate(((lc, "coarse"), (lf, "fine"))):
+        for k, pname in enumerate(TR.PARAM_ORDER):
+            grad = leaves[pname].grad
+            if pname.startswith("layers_dir.3"):  # built by the reference model but never used by its forward (models.py:257)
+                assert np.isnan(max_abs[m_i, k]) and grad is None
                 continue
-            assert g_ref is not None and leaves[k].grad is not None, (tag, k)
-            close(leaves[k].grad, g_ref, (tag, k))
+            assert not np.isnan(max_abs[m_i, k]) and grad is not None, (tag, pname)
+            flat, scale = grad.reshape(-1), max(float(max_abs[m_i, k]), 1e-12)
+            idx = G.grad_sample_index(flat.numel(), k)
+            close(flat[idx], stored[at:at + idx.numel()], (tag, pname, "entries"), scale)
+            at += idx.numel()
+            assert abs(float(flat.abs().max()) - float(max_abs[m_i, k])) <= 2e-5 * scale, (tag, pname, "max")
+            norm, norm_ref = math.sqrt(float((flat.double() ** 2).sum())), math.sqrt(float(sum_sq[m_i, k]))
+            assert abs(norm - norm_ref) <= 2e-5 * scale * math.sqrt(flat.numel()), (tag, pname, "norm", norm, norm_ref)
             n_checked += 1
-    assert n_checked == 2 * 24
-    close(lat.grad, lat_ref.grad, "latent")
-    assert float(lat_ref.grad.abs().max()) > 0
+    assert n_checked == 2 * 24 and at == stored.numel()
+    lat_ref = g("grad_latent")
+    close(lat.grad, lat_ref, "latent")
+    assert float(lat_ref.abs().max()) > 0

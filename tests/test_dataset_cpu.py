@@ -49,31 +49,21 @@ def test_round_trip_through_load_flame_data(tmp_path, built_lib):
 
 
 def test_loader_matches_the_reference_loader(tmp_path, built_lib):
-    """nerf.load_flame_data against the UNMODIFIED reference loader (nerf/load_flame.py:40-211, staged copy / live tree) on the
-    same synthetic dataset: every returned member equal, for the train and the test-only call, with and without half_res."""
+    """nerf.load_flame_data against the UNMODIFIED reference loader (nerf/load_flame.py:40-211) on the same synthetic dataset:
+    every returned member equal, for the train and the test-only call, with and without half_res.  The reference loader's
+    members are stored as digests of their values in tests/golden/reference_checks/dataset.json
+    (oracle/make_golden_reference_checks.py)."""
     import sys
 
-    import cv2
-    import numpy as np
-    import torch
-
-    import ref_loader
-    ref = ref_loader.load_reference()
-    if ref is None:
-        import pytest
-        pytest.skip("no reference tree (baseline/_ref not staged)")
-    sys.modules["imageio"].imread = lambda p: cv2.imread(p, cv2.IMREAD_UNCHANGED)[..., ::-1]
+    sys.path.insert(0, os.path.join(ROOT, "oracle"))
+    import make_golden_reference_checks as G
     import nerf
+    with open(os.path.join(G.OUT, "dataset.json")) as f:
+        gold = json.load(f)["calls"]
     _writer().write_dataset(str(tmp_path), 32, 3, 1, 4)
-    for kw in (dict(half_res=False, testskip=1, test=True), dict(half_res=True, testskip=1), dict(half_res=False, testskip=2)):
-        a, b = ref.load_flame_data(str(tmp_path), **kw), nerf.load_flame_data(str(tmp_path), **kw)
-        assert len(a) == len(b) == 8
-        for x, y in zip(a, b):
-            if torch.is_tensor(x):
-                assert x.shape == y.shape and float((x.float() - y.float()).abs().max()) == 0.0
-            elif isinstance(x, list) and len(x) == 3 and not isinstance(x[0], np.ndarray):
-                assert x[0] == y[0] and x[1] == y[1] and np.array_equal(np.asarray(x[2]), np.asarray(y[2]))
-            elif isinstance(x, list):
-                assert all(np.array_equal(p, q) for p, q in zip(x, y))
-            else:
-                assert x is None and y is None
+    assert [c["kwargs"] for c in gold] == G.LOADER_CALLS
+    for call in gold:
+        got = nerf.load_flame_data(str(tmp_path), **call["kwargs"])
+        assert len(got) == len(call["members"]) == 8
+        for i, (want, y) in enumerate(zip(call["members"], got)):
+            assert G.describe(y) == want, (call["kwargs"], i)

@@ -1,10 +1,10 @@
-"""The oracle against the UNMODIFIED reference executed LIVE (CPU), on configurations the golden fixtures do not hold: the
-smallest sample counts the kernels accept, a single fine sample, ragged chunk sizes, perturbation without noise, white
-background without a background image, the direction-ablation input with every stochastic option on.  Every output must be
-bit-identical — the same statement oracle/make_golden.py prints for the eight committed cases.
+"""The oracle against the UNMODIFIED reference on configurations the golden fixtures do not hold: the smallest sample counts the
+kernels accept, a single fine sample, ragged chunk sizes, perturbation without noise, white background without a background
+image, the direction-ablation input with every stochastic option on.  Every output must be bit-identical — the same statement
+oracle/make_golden.py prints for the eight committed cases.
 
-Needs the reference tree (/root/reference in the build container, the staged byte-for-byte copy baseline/_ref on the GPU box,
-oracle/stage_reference.py); skipped when neither is present.  CPU only."""
+What the reference computed (rays, the torch.rand / torch.randn draws it made, its outputs) is stored in
+tests/golden/reference_checks/oracle_cases.npz by oracle/make_golden_reference_checks.py.  CPU only."""
 import os
 import sys
 
@@ -15,81 +15,43 @@ import torch
 import nerface_oracle as O
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle"))
-import make_golden as MG  # noqa: E402
-import ref_loader  # noqa: E402
+import make_golden_reference_checks as G  # noqa: E402
 
-pytestmark = pytest.mark.skipif(ref_loader.reference_root() is None, reason="no reference tree (run oracle/stage_reference.py)")
-
-# name: (H, W, Sampling(nc, nf, perturb, noise_std, white_bkgd, chunksize), mode, use_bg, use_fine, stress, ablation)
-CASES = {
-    "min_coarse_3c5f": (3, 4, O.Sampling(3, 5, False, 0.0, False, 65536), "validation", True, True, True, False),
-    "one_fine_sample": (2, 5, O.Sampling(64, 1, False, 0.0, False, 65536), "validation", True, True, False, False),
-    "ragged_chunks_train": (5, 3, O.Sampling(16, 8, True, 0.2, False, 7), "train", True, True, True, False),
-    "perturb_only_white_nobg": (4, 4, O.Sampling(40, 72, True, 0.0, True, 65536), "validation", False, True, True, False),
-    "noise_only_coarse_only": (4, 3, O.Sampling(24, 0, False, 0.3, False, 5), "train", True, False, False, False),
-    # chunk size divides the ray count: with a ragged last chunk the reference itself raises (every chunk takes the FIRST chunk's
-    # ablation directions, train_utils.py:82 — the quirk the oracle and the kernels reproduce)
-    "ablation_all_stochastic": (3, 5, O.Sampling(32, 48, True, 0.1, False, 5), "validation", True, True, True, True),
-}
+CASES = G.ORACLE_CASES
 
 
 @pytest.fixture(scope="module")
-def ref():
+def gold():
     assert torch.get_float32_matmul_precision() == "highest"
-    return ref_loader.load_reference()  # module `nerf_reference`: does not shadow the drop-in `nerf` other tests import
+    return np.load(os.path.join(G.OUT, "oracle_cases.npz"))
 
 
 @pytest.mark.parametrize("name", list(CASES))
-def test_oracle_is_bit_identical_to_the_live_reference(ref, name):
+def test_oracle_is_bit_identical_to_the_live_reference(gold, name):
     H, W, s, mode, use_bg, use_fine, stress, ablation = CASES[name]
+    g = lambda k: torch.from_numpy(gold[f"{name}/{k}"])  # noqa: E731
     ci = 200 + list(CASES).index(name)
     near, far = 0.2, 0.8
     pc = O.random_init_params(300 + ci, stress)
     pf = O.random_init_params(400 + ci, stress) if use_fine else None
     fr = O.synthetic_frame(ci, H, W)
-    ro, rd = ref.get_ray_bundle(H, W, np.array(fr["intrinsics"]), fr["pose"][:3, :4])
+    ro, rd = g("ro"), g("rd")
     o_ro, o_rd = O.ray_bundle(H, W, fr["intrinsics"], fr["pose"])
     assert torch.equal(ro, o_ro) and torch.equal(rd, o_rd)
     if mode == "train":  # the trainer passes flat gathered rays (train_transformed_rays.py:320-326)
         ro, rd = ro.reshape(-1, 3).clone(), rd.reshape(-1, 3).clone()
     bg = fr["bg"].reshape(-1, 3) if use_bg else None
-    rd_abl = None
-    if ablation:
-        fr2 = O.synthetic_frame(ci + 50, H, W)
-        _, rd_abl = ref.get_ray_bundle(H, W, np.array(fr2["intrinsics"]), fr2["pose"][:3, :4])
-    mc = ref_loader.build_model(ref, pc)
-    mf = ref_loader.build_model(ref, pf) if use_fine else None
-    cfg = ref_loader.make_cfg(ref, s.num_coarse, s.num_fine, s.perturb, s.noise_std, s.white_bkgd, s.chunksize, mode, near, far)
-    torch.manual_seed(4321 + ci)
-    with torch.no_grad(), MG.Recorder() as rec:
-        want = ref.run_one_iter_of_nerf(H, W, fr["intrinsics"], mc, mf, ro.clone(), rd.clone(), cfg, mode=mode,
-                                        encode_position_fn=ref.get_embedding_function(10, True, True),
-                                        encode_direction_fn=ref.get_embedding_function(4, False, True),
-                                        expressions=fr["expr"], background_prior=bg, latent_code=fr["latent"],
-                                        ray_directions_ablation=rd_abl)
+    rd_abl = g("rd_ablation") if ablation else None
     # the recorded draws, split back into the per-chunk order the reference made them in (train_utils.py:69-76, 105-119)
-    n_rays = H * W
-    it = iter(rec.draws)
-    noises = []
-    for st in range(0, n_rays, s.chunksize):
-        nz = O.Noise()
-        if s.perturb:
-            nz.t_rand = next(it)[1]
-        if s.noise_std > 0:
-            nz.n_c = next(it)[1]
-        if s.num_fine > 0:
-            if s.perturb:
-                nz.u = next(it)[1]
-            if s.noise_std > 0:
-                nz.n_f = next(it)[1]
-        noises.append(nz)
-    assert next(it, None) is None, "the reference drew more random tensors than the oracle's model of it consumes"
+    noises = G.split_draws([g(f"draw{j}") for j in range(int(gold[f"{name}/n_draws"]))], s, H * W)
     with torch.no_grad():
         got = O.run_one_iter(ro, rd, pc, pf, s, near, far, fr["expr"], fr["latent"], bg, mode, noise_per_chunk=noises,
                              rd_ablation=rd_abl)
-    assert len(got) == len(want)
-    for i, (a, b) in enumerate(zip(want, got)):
-        assert (a is None) == (b is None), i
-        if a is not None:
+    assert len(got) == int(gold[f"{name}/arity"])
+    for i, b in enumerate(got):
+        key = f"{name}/out{i}"
+        assert (key not in gold) == (b is None), i
+        if b is not None:
+            a = g(f"out{i}")
             assert a.shape == b.shape, (i, a.shape, b.shape)
             assert torch.equal(a, b), (name, i, float((a - b).abs().max()))

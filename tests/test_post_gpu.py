@@ -95,8 +95,13 @@ def test_ray_sampler_numpy_lockstep_and_device_rng(env):
 
 def test_frame_products_match_the_reference_functions(env):
     """cast_to_image / torch_normal_map(clean=True) / cast_to_disparity_image bytes against the reference functions' outputs on the
-    same FP32 inputs (golden, made with CPU torch: NFB_PRODUCTS_LIKE_TORCH_CPU).  And, in the default mode, against the reference
-    functions executed with torch CUDA on this box (what the unmodified eval script runs here) at 64x64 and 512x512."""
+    same FP32 inputs: with NFB_PRODUCTS_LIKE_TORCH_CPU against the functions run with CPU torch, in full at 64x64 (golden_products)
+    and as digests of the whole frame at 64x64 and 512x512; in the default mode against the functions run with torch CUDA on a
+    B200 (what the unmodified eval script computes on a GPU), as digests at 64x64 and 512x512 (golden/reference_checks/products.json,
+    oracle/make_golden_reference_checks.py)."""
+    import json
+    import sys
+
     nerf, ray_sampler, dev = env
     g = np.load(GOLD)
     rgb, disp, w_last = (torch.from_numpy(g[k]).to(dev) for k in ("rgb", "disp", "w_last"))
@@ -109,20 +114,14 @@ def test_frame_products_match_the_reference_functions(env):
         assert got.shape == ref.shape and got.dtype == np.uint8, name
         bad = int((got != ref).sum())
         assert bad == 0, (name, bad, int(np.abs(got.astype(int) - ref.astype(int)).max()))
-    import ref_loader
-    ev = ref_loader.load_eval_script()
-    if ev is not None:
-        for H in (64, 512):
-            gen = torch.Generator().manual_seed(H)
-            d = (torch.rand(H, H, generator=gen) * 4 + 1).to(dev)
-            w = (torch.rand(H, H, generator=gen) ** 3).to(dev)
-            c = torch.rand(H, H, 3, generator=gen).to(dev) * 1.2 - 0.1
-            intr = np.array([1200.0 * H / 512, 1150.0 * H / 512, 0.52, 0.47])
-            ref_n = ev.torch_normal_map(d.clone(), intr, w.clone(), clean=True).cpu().numpy().astype("uint8")
-            ref_d = ev.cast_to_disparity_image(d)
-            ref_c = ev.cast_to_image(c, "blender")
-            got_c, got_n, got_d = ray_sampler.frame_products(c, d, w, list(intr), want_disparity=True)
-            for name, got, ref in (("rgb", got_c, np.asarray(ref_c)), ("normals", got_n, ref_n), ("disparity", got_d, ref_d)):
-                got = got.cpu().numpy()
-                bad = int((got != ref).sum())
-                assert bad == 0, (H, name, bad, ref.size, int(np.abs(got.astype(int) - ref.astype(int)).max()))
+    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle"))
+    import make_golden_reference_checks as G
+    with open(os.path.join(G.OUT, "products.json")) as f:
+        digests = json.load(f)
+    for H in G.PRODUCT_SIZES:
+        c, d, w, intr = (t.to(dev) if torch.is_tensor(t) else t for t in G.product_inputs(H))
+        for backend, like_cpu in (("cpu", True), ("cuda", False)):
+            got = ray_sampler.frame_products(c, d, w, list(intr), want_disparity=True, like_torch_cpu=like_cpu)
+            for name, t in zip(("rgb", "normals", "disparity"), got):
+                t, want = t.cpu().numpy(), digests[backend][str(H)][name]
+                assert t.dtype == np.uint8 and list(t.shape) == want["shape"] and G.sha256(t) == want["sha256"], (backend, H, name)

@@ -6,7 +6,7 @@
 
 through 4d-facial-avatars_b200/run_reference_script.py, which only puts this repository's drop-in `nerf` package first on
 sys.path (and, under torchrun, shards run_one_iter_of_nerf over the ranks — nerf/parallel.py).  The script bodies come from the
-reference tree (/root/reference here, the staged byte-for-byte copy baseline/_ref on the GPU box); the dataset is synthetic
+reference tree (the byte-for-byte copy oracle/stage_reference.py stages into oracle/_ref); the dataset is synthetic
 (tools/make_synthetic_dataset.py); the YAML is the shipped paper-model config with only paths and iteration counts replaced.
 
     python tools/run_reference_clis.py --out gpurun_out/cli --gpus 1 --iters 40
@@ -42,7 +42,7 @@ def main():
     train_py, eval_py = ref_loader.script_path("train_transformed_rays.py"), ref_loader.script_path("eval_transformed_rays.py")
     yml = ref_loader.script_path(os.path.join("config", "dave", "dave_dvp_lcode_fixed_bg_512_paper_model.yml"))
     if not train_py or not os.path.exists(train_py):
-        sys.exit("no reference tree: run oracle/stage_reference.py in the build container first")
+        sys.exit("no reference tree: run oracle/stage_reference.py --ref PATH_TO_REFERENCE_CHECKOUT first")
     out = os.path.abspath(a.out)
     data, logs = os.path.join(out, "data"), os.path.join(out, "logs")
     os.makedirs(out, exist_ok=True)
