@@ -37,8 +37,6 @@ struct NfbHandle {
   bool frame_set = false;
   bool use_render2 = true;
   bool use_render3 = true;
-  bool train_render2 = false;   // training forward on the two-tile kernel (NFB_TRAIN_KERNEL=v6)
-  bool train_render3 = false;   // training forward on the pipelined kernel (NFB_TRAIN_KERNEL=v7); default: the one-tile kernel
   long long launches = 0;
   // cached torch.linspace(0,1,n) tables on the device
   float* lin_c = nullptr; int lin_c_n = 0;
@@ -142,14 +140,6 @@ static int create_impl(NfbHandle* h, const cudaDeviceProp& prop) {
     const char* k = std::getenv("NFB_KERNEL");
     h->use_render2 = !(k && std::strcmp(k, "v4") == 0);
     h->use_render3 = h->use_render2 && !(k && std::strcmp(k, "v6") == 0);  // NFB_KERNEL=v6: two tiles in flight, passes not pipelined
-    // The training forward defaults to the one-tile kernel: with the record stores the two-tile kernel's row warps spill
-    // (216 B) and it is slower there (measured 1.46 ms vs 1.01 ms per 2048-ray forward); NFB_TRAIN_KERNEL=v6 selects it.
-    const char* tk = std::getenv("NFB_TRAIN_KERNEL");
-    h->train_render2 = tk && std::strcmp(tk, "v6") == 0;
-    // Both two-stream kernels have SAVE variants whose records are bit-identical to the one-tile kernel's, and both are SLOWER
-    // there (2048 rays, 64c+64f: v4 0.77 ms, v6 1.46 ms, v7 1.26 ms): the record is written as 16-bit transposed stores, 2304 per
-    // row thread and tile, and with two streams the same eight row warps issue twice as many per unit of time.
-    h->train_render3 = h->use_render3 && tk && std::strcmp(tk, "v7") == 0;
   }
   return NFB_OK;
 }
@@ -402,11 +392,11 @@ static int render_impl(NfbHandle* h, const NfbRays* rays, const NfbSampling* sm,
     tr.n_rays = rays->n_rays; tr.nc = nc; tr.nf = nf; tr.rays_per_unit = p.rays_per_unit; tr.tiles_c = p.tiles_c;
     tr.tiles_f = p.tiles_f; tr.n_units = p.n_units; tr.has_bg = rays->background != nullptr; tr.white_bkgd = p.white_bkgd;
   }
-  // fast-mode evaluation runs the two-tiles-in-flight kernel (the training forward only on request, see nfb_create); exact
-  // mode (hi+lo operands need twice the TMEM columns) and the layer probe run the one-tile kernel
-  const bool saving = train && !h->tr.chunked;
-  const bool two_tile = h->use_render2 && !exact && !p.dbg_act && (!saving || h->train_render2);
-  const bool pipelined = h->use_render3 && !exact && !p.dbg_act && (!saving || h->train_render3) && nfb::render3_supports(p);
+  // fast-mode evaluation runs a two-tiles-in-flight kernel; exact mode (hi+lo operands need twice the TMEM columns), the
+  // training forward (only the one-tile kernel writes the activation records) and the layer probe run the one-tile kernel
+  const bool saving = p.save_rec != nullptr;
+  const bool two_tile = h->use_render2 && !exact && !p.dbg_act && !saving;
+  const bool pipelined = two_tile && h->use_render3 && nfb::render3_supports(p);
   if (pipelined) NFB_CUDA(nfb::launch_render3(p, h->num_sms, st, &h->launches));
   else if (two_tile) NFB_CUDA(nfb::launch_render2(p, h->num_sms, st, &h->launches));
   else NFB_CUDA(nfb::launch_render(p, exact ? 1 : 0, h->num_sms, st, &h->launches));
@@ -511,9 +501,7 @@ int nfb_render_backward(NfbHandle* h, const NfbOutGrads* og, const float* const 
       p.w_last = so + 10 * cn;
       p.save_rec = tr.rec; p.save_dnorm = tr.dnorm; p.save_raw_c = tr.raw_c; p.save_raw_f = tr.raw_f;
       p.dbg_z_c = tr.z_c; p.dbg_z_f = tr.z_f;
-      if (h->train_render3 && tr.precision == 0 && nfb::render3_supports(p)) NFB_CUDA(nfb::launch_render3(p, h->num_sms, st, &h->launches));
-      else if (h->train_render2 && tr.precision == 0) NFB_CUDA(nfb::launch_render2(p, h->num_sms, st, &h->launches));
-      else NFB_CUDA(nfb::launch_render(p, tr.precision, h->num_sms, st, &h->launches));
+      NFB_CUDA(nfb::launch_render(p, tr.precision, h->num_sms, st, &h->launches));
       rc = backward_rays(begin, n, n_units);
       if (rc) return rc;
     }

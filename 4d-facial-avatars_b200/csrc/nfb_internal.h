@@ -117,7 +117,7 @@ cudaError_t launch_adam(float* p, float* g, float* m, float* v, long long n, flo
 // precision: 0 = fast (x1), 1 = exact (x3).  num_sms = CTAs to launch at most.
 cudaError_t launch_render(const RenderParams& p, int precision, int num_sms, cudaStream_t st, long long* launches);
 cudaError_t render_kernel_setup();  // opt-in to the large dynamic shared memory size
-// Two-tiles-in-flight kernel (nfb_render2.cu): fast mode, evaluation (no training records, no layer probe / phase timers).
+// Two-tiles-in-flight kernel (nfb_render2.cu): fast-mode evaluation (the training forward and the layer probe run launch_render).
 cudaError_t render2_kernel_setup();
 cudaError_t launch_render2(const RenderParams& p, int num_sms, cudaStream_t st, long long* launches);
 // Two tiles in flight + software-pipelined passes (nfb_render3.cu): fast-mode evaluation of the configurations its fixed

@@ -374,47 +374,13 @@ __global__ void __launch_bounds__(SAVE ? kThreadsSave : kThreads, 1) render_kern
       // ---- per-ray constants
       if (etid < R) {
         RayP& rp = rayp[etid];
-        const int g = unit * R + etid;
-        rp.valid = g < p.n_rays;
-        rp.gidx = g;
-        if (rp.valid) {
-          float o0, o1, o2, d0, d1, d2;
-          if (p.o) {
-            o0 = p.o[3 * g]; o1 = p.o[3 * g + 1]; o2 = p.o[3 * g + 2];
-            d0 = p.d[3 * g]; d1 = p.d[3 * g + 1]; d2 = p.d[3 * g + 2];
-          } else {  // get_ray_bundle (nerf_helpers.py:111-122), same operation order in FP32
-            const int pj = p.row_begin + g / p.width, pi = g % p.width;
-            const float cx = __fdiv_rn(__fsub_rn((float)pi, p.wcx), p.fx);
-            const float cy = -__fdiv_rn(__fsub_rn((float)pj, p.hcy), p.fy);
-            d0 = __fadd_rn(__fadd_rn(__fmul_rn(cx, p.pose[0]), __fmul_rn(cy, p.pose[1])), __fmul_rn(-1.f, p.pose[2]));
-            d1 = __fadd_rn(__fadd_rn(__fmul_rn(cx, p.pose[4]), __fmul_rn(cy, p.pose[5])), __fmul_rn(-1.f, p.pose[6]));
-            d2 = __fadd_rn(__fadd_rn(__fmul_rn(cx, p.pose[8]), __fmul_rn(cy, p.pose[9])), __fmul_rn(-1.f, p.pose[10]));
-            o0 = p.pose[3]; o1 = p.pose[7]; o2 = p.pose[11];
-          }
-          rp.o[0] = o0; rp.o[1] = o1; rp.o[2] = o2;
-          rp.d[0] = d0; rp.d[1] = d1; rp.d[2] = d2;
-          rp.dnorm = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(d0, d0), __fmul_rn(d1, d1)), __fmul_rn(d2, d2)));
-          if (has_bg) { rp.bg[0] = p.bg[3 * g]; rp.bg[1] = p.bg[3 * g + 1]; rp.bg[2] = p.bg[3 * g + 2]; }
-          rp.dz = p.dir_z ? p.dir_z[g] : d2;
-          if constexpr (SAVE) p.save_dnorm[g] = rp.dnorm;
-        } else {
-          for (int k = 0; k < 3; ++k) { rp.o[k] = 0.f; rp.d[k] = 0.f; rp.bg[k] = 0.f; }
-          rp.dnorm = 0.f;
-          rp.dz = 0.f;
+        load_ray(p, unit * R + etid, rp);
+        if constexpr (SAVE) {
+          if (rp.valid) p.save_dnorm[rp.gidx] = rp.dnorm;
         }
       }
       named_bar_sync(kRowBarrier, kRowThreads);
-      // direction encoder input is (d_z, near, far): run_network reads ray_batch[..., -3:] (train_utils.py:14);
-      // one accurate sincos per thread
-      if (etid < R * 12) {
-        const int rr = etid / 12, k = etid - rr * 12, f = k / 3, c = k - f * 3;
-        RayP& rp = rayp[rr];
-        const float v = (c == 0) ? rp.dz : (c == 1 ? p.near_ : p.far_);
-        float sn, cs;
-        sincosf(v * (float)(1 << f), &sn, &cs);
-        rp.ped[6 * f + c] = rp.valid ? sn : 0.f;
-        rp.ped[6 * f + 3 + c] = rp.valid ? cs : 0.f;
-      }
+      dir_encoding(p, rayp, R, etid);
       named_bar_sync(kRowBarrier, kRowThreads);
       tm.lap(0);
 
@@ -437,23 +403,7 @@ __global__ void __launch_bounds__(SAVE ? kThreadsSave : kThreads, 1) render_kern
           float z = 0.f;
           if (live) {
             if (pass == 0) {
-              const float tc = p.t_coarse[i];
-              z = __fadd_rn(__fmul_rn(p.near_, __fsub_rn(1.f, tc)), __fmul_rn(p.far_, tc));
-              if (p.perturb) {  // stratified jitter (train_utils.py:69-76)
-                float lower = z, upper = z;
-                if (i > 0) {
-                  const float tp = p.t_coarse[i - 1];
-                  const float zp = __fadd_rn(__fmul_rn(p.near_, __fsub_rn(1.f, tp)), __fmul_rn(p.far_, tp));
-                  lower = __fmul_rn(0.5f, __fadd_rn(z, zp));
-                }
-                if (i < S - 1) {
-                  const float tn = p.t_coarse[i + 1];
-                  const float zn = __fadd_rn(__fmul_rn(p.near_, __fsub_rn(1.f, tn)), __fmul_rn(p.far_, tn));
-                  upper = __fmul_rn(0.5f, __fadd_rn(zn, z));
-                }
-                const float tr = rp.valid ? p.t_rand[(size_t)rp.gidx * p.nc + i] : 0.f;
-                z = __fadd_rn(lower, __fmul_rn(__fsub_rn(upper, lower), tr));
-              }
+              z = coarse_depth(p, rp, i, S);
               if (ch == 0) carry_z[prow] = z;
             } else {
               z = carry_z[prow];
@@ -461,52 +411,9 @@ __global__ void __launch_bounds__(SAVE ? kThreadsSave : kThreads, 1) render_kern
           }
           // positional encoding of o + d*z: 63 lanes + 1 zero pad, FP16 (hi[,lo]) into the swizzled PE buffer.
           // The two threads of a row write lanes [0,32) and [32,64) respectively.
-          const float px = __fadd_rn(rp.o[0], __fmul_rn(rp.d[0], z));
-          const float py = __fadd_rn(rp.o[1], __fmul_rn(rp.d[1], z));
-          const float pz = __fadd_rn(rp.o[2], __fmul_rn(rp.d[2], z));
           float f[32];
-          if (ch == 0) {  // lanes 0..31: xyz, frequencies 0..3, sin of frequency 4, cos(x), cos(y) of frequency 4
-            f[0] = px; f[1] = py; f[2] = pz;
-#pragma unroll
-            for (int fr = 0; fr < 4; ++fr) {
-              const float sc = (float)(1 << fr);
-              pe_sincos<EXACT>(px * sc, f[3 + 6 * fr + 0], f[3 + 6 * fr + 3]);
-              pe_sincos<EXACT>(py * sc, f[3 + 6 * fr + 1], f[3 + 6 * fr + 4]);
-              pe_sincos<EXACT>(pz * sc, f[3 + 6 * fr + 2], f[3 + 6 * fr + 5]);
-            }
-            float cz;
-            pe_sincos<EXACT>(px * 16.f, f[27], f[30]);
-            pe_sincos<EXACT>(py * 16.f, f[28], f[31]);
-            pe_sincos<EXACT>(pz * 16.f, f[29], cz);
-          } else {        // lanes 32..63: cos(z) of frequency 4, frequencies 5..9, zero pad
-            float sz;
-            pe_sincos<EXACT>(pz * 16.f, sz, f[0]);
-#pragma unroll
-            for (int fr = 5; fr < 10; ++fr) {
-              const float sc = (float)(1 << fr);
-              const int b = 6 * fr - 29;  // lane 3 + 6*fr, minus 32
-              pe_sincos<EXACT>(px * sc, f[b + 0], f[b + 3]);
-              pe_sincos<EXACT>(py * sc, f[b + 1], f[b + 4]);
-              pe_sincos<EXACT>(pz * sc, f[b + 2], f[b + 5]);
-            }
-            f[31] = 0.f;
-          }
-#pragma unroll
-          for (int qq = 0; qq < 4; ++qq) {
-            uint32_t hi[4], lo[4];
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-              const float a = f[qq * 8 + 2 * e], b = f[qq * 8 + 2 * e + 1];
-              hi[e] = pack_f16x2(a, b);
-              if constexpr (EXACT) {
-                const float2 hf = unpack_f16x2(hi[e]);
-                lo[e] = pack_f16x2(a - hf.x, b - hf.y);
-              }
-            }
-            const int off = row * 128 + (((ch * 4 + qq) ^ (row & 7)) << 4);
-            *reinterpret_cast<uint4*>(pe_hi + off) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-            if constexpr (EXACT) *reinterpret_cast<uint4*>(pe_lo + off) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-          }
+          pe_lanes<EXACT>(rp, z, ch, f);
+          store_pe_row<EXACT>(f, pe_hi, pe_lo, row, ch);
           if (p.dbg_act && p.dbg_act_step == -1 && unit == 0 && pass == 0 && t == 0) {
 #pragma unroll
             for (int k = 0; k < 32; ++k) p.dbg_act[row * 256 + ch * 32 + k] = f[k];
@@ -605,22 +512,8 @@ __global__ void __launch_bounds__(SAVE ? kThreadsSave : kThreads, 1) render_kern
                   float* dr = pass ? p.dbg_raw_f : p.dbg_raw_c;
                   if (dr) reinterpret_cast<float4*>(dr)[(size_t)rp.gidx * S + i] = make_float4(r0, r1, r2, sigma_raw);
                 }
-                float sig = sigma_raw;
-                if (p.noise_std > 0.f && rp.valid)
-                  sig = __fadd_rn(sig, __fmul_rn((pass ? p.noise_f : p.noise_c)[(size_t)rp.gidx * S + i], p.noise_std));
-                const float sig_in = sig;  // what the ReLU sees (volume_rendering_utils.py:52)
-                sig = fmaxf(sig, 0.f);
-                float4 pre;
-                if (i == S - 1) {
-                  sig = __fadd_rn(sig, 1e-6f);
-                  if (has_bg) { pre.x = rp.bg[0]; pre.y = rp.bg[1]; pre.z = rp.bg[2]; }
-                }
-                if (!(has_bg && i == S - 1)) {
-                  pre.x = 1.f / (1.f + expf(-r0));
-                  pre.y = 1.f / (1.f + expf(-r1));
-                  pre.z = 1.f / (1.f + expf(-r2));
-                }
-                pre.w = sig;
+                float sig_in;
+                const float4 pre = colour_sigma(p, rp, has_bg, r0, r1, r2, sigma_raw, pass, S, i, sig_in);
                 carry_raw[prow] = pre;
                 if constexpr (SAVE) {  // what the compositing backward needs: colour (or bg) and the ReLU input
                   if (rp.valid) reinterpret_cast<float4*>(pass ? p.save_raw_f : p.save_raw_c)[(size_t)rp.gidx * S + i] = make_float4(pre.x, pre.y, pre.z, sig_in);
@@ -712,37 +605,8 @@ __global__ void __launch_bounds__(SAVE ? kThreadsSave : kThreads, 1) render_kern
 
         // ---- inverse-CDF resampling (nerf_helpers.py:344-387) on weights[1:-1] over the mid-point bins
         __syncwarp();
-        const int nb = p.nc - 1;   // bins / cdf entries
-        const int nw = p.nc - 2;   // interior weights
-        if (ew < R) {
-          const float* w = scr_w + ew * p.nc;
-          const float* zc = carry_z + ew * p.nc;
-          float* cdf = scr_cdf + ew * p.nc;
-          float* bins = scr_bins + ew * p.nc;
-          for (int k = lane; k < nb; k += 32) bins[k] = __fmul_rn(0.5f, __fadd_rn(zc[k + 1], zc[k]));
-          const int per = (nw + 31) >> 5;
-          const int k0 = lane * per;
-          float part = 0.f;
-          for (int j = 0; j < per; ++j)
-            if (k0 + j < nw) part += __fadd_rn(w[k0 + j + 1], 1e-5f);
-          const float total = warp_sum(part);
-          float psum = 0.f;
-          for (int j = 0; j < per; ++j)
-            if (k0 + j < nw) psum += __fdiv_rn(__fadd_rn(w[k0 + j + 1], 1e-5f), total);
-          float incl = psum;
-#pragma unroll
-          for (int o = 1; o < 32; o <<= 1) {
-            const float tt = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= o) incl += tt;
-          }
-          float run = incl - psum;  // exclusive prefix of this lane's block
-          if (lane == 0) cdf[0] = 0.f;
-          for (int j = 0; j < per; ++j)
-            if (k0 + j < nw) {
-              run += __fdiv_rn(__fadd_rn(w[k0 + j + 1], 1e-5f), total);
-              cdf[k0 + j + 1] = run;
-            }
-        }
+        const int nb = p.nc - 1;
+        if (ew < R) build_cdf(scr_w + ew * p.nc, carry_z + ew * p.nc, scr_cdf + ew * p.nc, scr_bins + ew * p.nc, p.nc, lane);
         named_bar_sync(kRowBarrier, kRowThreads);
         tm.lap(5);
         // cat(z_coarse, z_samples) per ray into scr_sort (stride s_fine)
@@ -754,52 +618,18 @@ __global__ void __launch_bounds__(SAVE ? kThreadsSave : kThreads, 1) render_kern
             val = carry_z[rr * p.nc + i];
           } else {
             const int j = i - p.nc;
-            const float* cdf = scr_cdf + rr * p.nc;
-            const float* bins = scr_bins + rr * p.nc;
             const float u = p.perturb ? (rayp[rr].valid ? p.u_rand[(size_t)rayp[rr].gidx * p.nf + j] : 0.f) : p.u_fine[j];
-            int lo = 0, hi = nb;  // searchsorted(..., right=True): number of cdf entries <= u
-            while (lo < hi) {
-              const int mid = (lo + hi) >> 1;
-              if (cdf[mid] <= u) lo = mid + 1; else hi = mid;
-            }
-            const int below = max(0, lo - 1), above = min(nb - 1, lo);
-            const float cb = cdf[below], ca = cdf[above];
-            float den = __fsub_rn(ca, cb);
-            if (den < 1e-5f) den = 1.f;
-            const float tt = __fdiv_rn(__fsub_rn(u, cb), den);
-            val = __fadd_rn(bins[below], __fmul_rn(tt, __fsub_rn(bins[above], bins[below])));
+            val = sample_pdf(scr_cdf + rr * p.nc, scr_bins + rr * p.nc, nb, u);
           }
           scr_sort[k] = val;
         }
         named_bar_sync(kRowBarrier, kRowThreads);
         tm.lap(6);
-        // ---- torch.sort(cat(z, z_samples)) (train_utils.py:126) as a rank merge: the coarse depths are sorted, the
-        //      samples need not be (stochastic u), so an element's rank = (# coarse before it, by binary search)
-        //      + (# samples before it, counted).  Ties: coarse first, then samples by index — equal values make any
-        //      tie order give the same sorted array.
+        // ---- torch.sort(cat(z, z_samples)) (train_utils.py:126) as a rank merge
         for (int k = etid; k < R * SF; k += kRowThreads) {
           const int rr = k / SF, i = k - rr * SF;
-          const float* zc = scr_sort + rr * SF;
-          const float* zs = zc + p.nc;
-          const float v = zc[i];
-          int rank;
-          if (i < p.nc) {
-            rank = i;
-            for (int j = 0; j < p.nf; ++j) rank += (zs[j] < v) ? 1 : 0;
-          } else {
-            const int jm = i - p.nc;
-            int lo = 0, hi = p.nc;  // # coarse depths <= v
-            while (lo < hi) {
-              const int mid = (lo + hi) >> 1;
-              if (zc[mid] <= v) lo = mid + 1; else hi = mid;
-            }
-            rank = lo;
-            for (int j = 0; j < p.nf; ++j) {
-              const float y = zs[j];
-              rank += (y < v || (y == v && j < jm)) ? 1 : 0;
-            }
-          }
-          carry_z[rr * SF + rank] = v;
+          const float* z = scr_sort + rr * SF;
+          carry_z[rr * SF + merge_rank(z, p.nc, p.nf, i)] = z[i];
         }
         named_bar_sync(kRowBarrier, kRowThreads);
         tm.lap(7);
@@ -891,28 +721,12 @@ cudaError_t render_kernel_setup() {
 }
 
 cudaError_t launch_render(const RenderParams& p, int precision, int num_sms, cudaStream_t st, long long* launches) {
-  int grid = p.n_units < num_sms ? p.n_units : num_sms;
-  if (grid <= 0) return cudaSuccess;
-  grid = (grid + kCluster - 1) / kCluster * kCluster;        // whole clusters
-  if (grid > num_sms) grid = num_sms / kCluster * kCluster;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(p.save_rec != nullptr ? kThreadsSave : kThreads);
-  cfg.dynamicSmemBytes = kSmemBytes;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = kCluster;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  const bool save = p.save_rec != nullptr;  // training forward: also writes the per-tile activation records
-  cudaError_t e;
-  if (precision == 1) e = save ? cudaLaunchKernelEx(&cfg, render_kernel<true, true>, p) : cudaLaunchKernelEx(&cfg, render_kernel<true, false>, p);
-  else e = save ? cudaLaunchKernelEx(&cfg, render_kernel<false, true>, p) : cudaLaunchKernelEx(&cfg, render_kernel<false, false>, p);
-  ++*launches;
-  return e != cudaSuccess ? e : cudaGetLastError();
+  if (p.save_rec) {  // training forward: also writes the per-tile activation records
+    return precision == 1 ? launch_clustered(render_kernel<true, true>, p, kCluster, kThreadsSave, kSmemBytes, num_sms, st, launches)
+                          : launch_clustered(render_kernel<false, true>, p, kCluster, kThreadsSave, kSmemBytes, num_sms, st, launches);
+  }
+  return precision == 1 ? launch_clustered(render_kernel<true, false>, p, kCluster, kThreads, kSmemBytes, num_sms, st, launches)
+                        : launch_clustered(render_kernel<false, false>, p, kCluster, kThreads, kSmemBytes, num_sms, st, launches);
 }
 
 }  // namespace nfb

@@ -1,4 +1,4 @@
-// nfb_render2.cu — the render path with TWO tiles in flight per SM (fast mode: evaluation; training variant on request).
+// nfb_render2.cu — the render path with TWO tiles in flight per SM (fast mode, evaluation).
 //
 // Same reference path and same per-tile algebra as nfb_render.cu (see its header for the reference citations); what
 // changes is how the tensor core is kept busy.  With one tile per SM the epilogue -> MMA hand-off of every step is
@@ -32,7 +32,6 @@
 #include "nfb_layout.h"
 #include "nfb_ptx.cuh"
 #include "nfb_render_common.cuh"
-#include "nfb_save.cuh"
 #include "nfb_tile2.cuh"
 
 namespace nfb {
@@ -43,14 +42,10 @@ using namespace t2;
 using Timer = PhaseTimer;
 
 constexpr int kRowsMax = 512;  // sample rows of one pass of one stream
-#ifndef NFB_V6_HELPER
-#define NFB_V6_HELPER 1
-#endif
-// Warp 3 (otherwise idle) computes the positional encoding of the NEXT fine-pass tile of both streams while the row warps
-// run the current tile's epilogues; with 0 the row warps do it themselves after step 3 (tensor core idle meanwhile).
-constexpr bool kHelper = NFB_V6_HELPER != 0;
 // Warps: 0 = weight producer, 1 / 2 = MMA issuer of stream X / Y (different SM sub-partitions; one warp issuing both streams
-// in turn measured 4.37 M rays/s against 4.51 M), 3 = idle, 4..11 = row warps.  12 warps still allow 168 registers per thread.
+// in turn measured 4.37 M rays/s against 4.51 M), 3 = helper, 4..11 = row warps.  12 warps still allow 168 registers per thread.
+// The helper computes the positional encoding of the NEXT fine-pass tile of both streams while the row warps run the current
+// tile's epilogues (in the coarse pass the row warps do it after step 3).
 constexpr int kRowWarp0 = 4;
 constexpr int kThreads = (kRowWarp0 + 8) * 32;
 constexpr int kRowThreads = 256;
@@ -79,85 +74,28 @@ static_assert(kSmemBytes <= 232448, "exceeds the 227 KB per-CTA shared memory li
 
 // Sample depth + positional encoding of tile t of stream x -> PE buffer x (63 lanes + zero pad, FP16, swizzled).
 __device__ __forceinline__ void prologue_fn(const RenderParams& p, const RayP* __restrict__ rayp, float* __restrict__ carry_z,
-                                                 uint8_t* __restrict__ pe_base, int x, int t, int pass, int S, int rows, int R,
-                                                 int row, int ch, uint8_t* __restrict__ rec /* training record of this tile or null */) {
-    const int prow = t * 128 + row;
-    const bool live = prow < rows;
-    const int r = live ? prow / S : 0;
-    const int i = live ? prow - r * S : 0;
-    const RayP& rp = rayp[x * R + r];
-    float z = 0.f;
-    if (live) {
-      if (pass == 0) {
-        const float tc = p.t_coarse[i];
-        z = __fadd_rn(__fmul_rn(p.near_, __fsub_rn(1.f, tc)), __fmul_rn(p.far_, tc));
-        if (p.perturb) {  // stratified jitter (train_utils.py:69-76)
-          float lower = z, upper = z;
-          if (i > 0) {
-            const float tp = p.t_coarse[i - 1];
-            const float zp = __fadd_rn(__fmul_rn(p.near_, __fsub_rn(1.f, tp)), __fmul_rn(p.far_, tp));
-            lower = __fmul_rn(0.5f, __fadd_rn(z, zp));
-          }
-          if (i < S - 1) {
-            const float tn = p.t_coarse[i + 1];
-            const float zn = __fadd_rn(__fmul_rn(p.near_, __fsub_rn(1.f, tn)), __fmul_rn(p.far_, tn));
-            upper = __fmul_rn(0.5f, __fadd_rn(zn, z));
-          }
-          const float tr = rp.valid ? p.t_rand[(size_t)rp.gidx * p.nc + i] : 0.f;
-          z = __fadd_rn(lower, __fmul_rn(__fsub_rn(upper, lower), tr));
-        }
-        if (ch == 0) carry_z[x * kRowsMax + prow] = z;
-      } else {
-        z = carry_z[x * kRowsMax + prow];
-      }
+                                            uint8_t* __restrict__ pe_base, int x, int t, int pass, int S, int rows, int R, int row,
+                                            int ch) {
+  const int prow = t * 128 + row;
+  const bool live = prow < rows;
+  const int r = live ? prow / S : 0;
+  const int i = live ? prow - r * S : 0;
+  const RayP& rp = rayp[x * R + r];
+  float z = 0.f;
+  if (live) {
+    if (pass == 0) {
+      z = coarse_depth(p, rp, i, S);
+      if (ch == 0) carry_z[x * kRowsMax + prow] = z;
+    } else {
+      z = carry_z[x * kRowsMax + prow];
     }
-    const float px = __fadd_rn(rp.o[0], __fmul_rn(rp.d[0], z));
-    const float py = __fadd_rn(rp.o[1], __fmul_rn(rp.d[1], z));
-    const float pz = __fadd_rn(rp.o[2], __fmul_rn(rp.d[2], z));
-    float f[32];
-    if (ch == 0) {  // lanes 0..31: xyz, frequencies 0..3, sin of frequency 4, cos(x), cos(y) of frequency 4
-      f[0] = px; f[1] = py; f[2] = pz;
-#pragma unroll
-      for (int fr = 0; fr < 4; ++fr) {
-        const float sc = (float)(1 << fr);
-        pe_sincos<false>(px * sc, f[3 + 6 * fr + 0], f[3 + 6 * fr + 3]);
-        pe_sincos<false>(py * sc, f[3 + 6 * fr + 1], f[3 + 6 * fr + 4]);
-        pe_sincos<false>(pz * sc, f[3 + 6 * fr + 2], f[3 + 6 * fr + 5]);
-      }
-      float cz;
-      pe_sincos<false>(px * 16.f, f[27], f[30]);
-      pe_sincos<false>(py * 16.f, f[28], f[31]);
-      pe_sincos<false>(pz * 16.f, f[29], cz);
-    } else {        // lanes 32..63: cos(z) of frequency 4, frequencies 5..9, zero pad
-      float sz;
-      pe_sincos<false>(pz * 16.f, sz, f[0]);
-#pragma unroll
-      for (int fr = 5; fr < 10; ++fr) {
-        const float sc = (float)(1 << fr);
-        const int b = 6 * fr - 29;
-        pe_sincos<false>(px * sc, f[b + 0], f[b + 3]);
-        pe_sincos<false>(py * sc, f[b + 1], f[b + 4]);
-        pe_sincos<false>(pz * sc, f[b + 2], f[b + 5]);
-      }
-      f[31] = 0.f;
-    }
-    uint8_t* pe = pe_base + x * (kTileM * 128);
-    uint32_t hh[16];
-#pragma unroll
-    for (int qq = 0; qq < 4; ++qq) {
-#pragma unroll
-      for (int e = 0; e < 4; ++e) hh[qq * 4 + e] = pack_f16x2(f[qq * 8 + 2 * e], f[qq * 8 + 2 * e + 1]);
-      const int off = row * 128 + (((ch * 4 + qq) ^ (row & 7)) << 4);
-      *reinterpret_cast<uint4*>(pe + off) = make_uint4(hh[qq * 4], hh[qq * 4 + 1], hh[qq * 4 + 2], hh[qq * 4 + 3]);
-    }
-    fence_proxy_async_smem();
-    if (rec) store_t32(rec + kRecPE + img_row_base(64, row), row, 32 * ch, hh);  // transposed FP16 image for the weight gradients
+  }
+  float f[32];
+  pe_lanes<false>(rp, z, ch, f);
+  store_pe_row<false>(f, pe_base + x * (kTileM * 128), nullptr, row, ch);
+  fence_proxy_async_smem();
 }
 
-// SAVE = training forward: also writes the per-tile activation records (nfb_layout.h kRec*), the per-sample colours / ReLU
-// inputs of sigma and |d| that nfb_render_backward reads.  Records are indexed like the one-tile kernel's: the stream x of
-// super-unit U is unit 2U + x there.
-template <bool SAVE>
 __global__ void __launch_bounds__(kThreads, 1) render2_kernel(const __grid_constant__ RenderParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   const uint32_t smem_base = smem_u32(smem);
@@ -196,7 +134,6 @@ __global__ void __launch_bounds__(kThreads, 1) render2_kernel(const __grid_const
   tc_fence_after_sync();
   const uint32_t tmem_base = *tmem_ptr_s;
   const uint32_t cta_rank = cluster_ctarank();
-  constexpr uint16_t kAllCtas = (1u << kCluster) - 1;
 
   const int first_in_cluster = (int)blockIdx.x - (int)cta_rank;
   const int n_iter = (p.n_units - first_in_cluster + (int)gridDim.x - 1) / (int)gridDim.x;  // n_units = super-units of 2R rays
@@ -229,7 +166,7 @@ __global__ void __launch_bounds__(kThreads, 1) render2_kernel(const __grid_const
     const uint32_t gate = bar_gate + x * 8;
     for (int it = 0; it < n_iter; ++it) {
       for (int t = 0; t < tiles_per_unit; ++t) {
-        const bool fine_t = kHelper && t >= p.tiles_c;  // fine-pass tiles: PE buffer handshake with the helper warp
+        const bool fine_t = t >= p.tiles_c;  // fine-pass tiles: PE buffer handshake with the helper warp
         if (fine_t && t > p.tiles_c) {                  // its encoding was written by the helper, not by the row warps
           mbar_wait(bar_peready + x * 8, ph_per);
           ph_per ^= 1;
@@ -251,7 +188,7 @@ __global__ void __launch_bounds__(kThreads, 1) render2_kernel(const __grid_const
         for_each_group(group, std::make_integer_sequence<int, kNumGroups>{});
       }
     }
-  } else if (kHelper && warp == 3) {
+  } else if (warp == 3) {
     // ============================== helper: encoding of the next fine-pass tile ==============================
     if (p.nf > 0) {
       const RayP* rayp = reinterpret_cast<const RayP*>(smem + kOffRay);
@@ -259,21 +196,15 @@ __global__ void __launch_bounds__(kThreads, 1) render2_kernel(const __grid_const
       const int R = p.rays_per_unit, S = p.s_fine, rows = R * S, n_tiles = p.tiles_f;
       uint32_t ph_free0 = 0, ph_free1 = 0;
       for (int it = 0; it < n_iter; ++it) {
-        const int unit = blockIdx.x + it * gridDim.x;
         for (int t = 0; t < n_tiles; ++t) {
 #pragma unroll
           for (int x = 0; x < 2; ++x) {
             if (x == 0) { mbar_wait(bar_pefree, ph_free0); ph_free0 ^= 1; }
             else        { mbar_wait(bar_pefree + 8, ph_free1); ph_free1 ^= 1; }
             if (t + 1 < n_tiles) {
-              uint8_t* rec = nullptr;
-              if constexpr (SAVE) {
-                const int u4 = 2 * unit + x;
-                if (u4 * R < p.n_rays) rec = p.save_rec + ((size_t)u4 * tiles_per_unit + p.tiles_c + (t + 1)) * kRecBytes;
-              }
               for (int k = 0; k < 8; ++k) {  // 128 rows x 2 lane halves = 256 thread-tasks for 32 threads
                 const int idx = k * 32 + lane;
-                prologue_fn(p, rayp, carry_z, smem + kOffPe, x, t + 1, 1, S, rows, R, idx & 127, idx >> 7, rec);
+                prologue_fn(p, rayp, carry_z, smem + kOffPe, x, t + 1, 1, S, rows, R, idx & 127, idx >> 7);
               }
               __syncwarp();  // every lane has fenced its generic-proxy stores (inside prologue_fn)
               if (lane == 0) mbar_arrive(bar_peready + x * 8);
@@ -307,48 +238,9 @@ __global__ void __launch_bounds__(kThreads, 1) render2_kernel(const __grid_const
     for (int it = 0; it < n_iter; ++it) {
       const int unit = blockIdx.x + it * gridDim.x;
       tm.lap(39);
-      // ---- per-ray constants (ray slot qy = x * R + r)
-      if (etid < RR) {
-        RayP& rp = rayp[etid];
-        const int g = unit * RR + etid;
-        rp.valid = g < p.n_rays;
-        rp.gidx = g;
-        if (rp.valid) {
-          float o0, o1, o2, d0, d1, d2;
-          if (p.o) {
-            o0 = p.o[3 * g]; o1 = p.o[3 * g + 1]; o2 = p.o[3 * g + 2];
-            d0 = p.d[3 * g]; d1 = p.d[3 * g + 1]; d2 = p.d[3 * g + 2];
-          } else {  // get_ray_bundle (nerf_helpers.py:111-122), same operation order in FP32
-            const int pj = p.row_begin + g / p.width, pi = g % p.width;
-            const float cx = __fdiv_rn(__fsub_rn((float)pi, p.wcx), p.fx);
-            const float cy = -__fdiv_rn(__fsub_rn((float)pj, p.hcy), p.fy);
-            d0 = __fadd_rn(__fadd_rn(__fmul_rn(cx, p.pose[0]), __fmul_rn(cy, p.pose[1])), __fmul_rn(-1.f, p.pose[2]));
-            d1 = __fadd_rn(__fadd_rn(__fmul_rn(cx, p.pose[4]), __fmul_rn(cy, p.pose[5])), __fmul_rn(-1.f, p.pose[6]));
-            d2 = __fadd_rn(__fadd_rn(__fmul_rn(cx, p.pose[8]), __fmul_rn(cy, p.pose[9])), __fmul_rn(-1.f, p.pose[10]));
-            o0 = p.pose[3]; o1 = p.pose[7]; o2 = p.pose[11];
-          }
-          rp.o[0] = o0; rp.o[1] = o1; rp.o[2] = o2;
-          rp.d[0] = d0; rp.d[1] = d1; rp.d[2] = d2;
-          rp.dnorm = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(d0, d0), __fmul_rn(d1, d1)), __fmul_rn(d2, d2)));
-          if (has_bg) { rp.bg[0] = p.bg[3 * g]; rp.bg[1] = p.bg[3 * g + 1]; rp.bg[2] = p.bg[3 * g + 2]; }
-          rp.dz = p.dir_z ? p.dir_z[g] : d2;
-          if constexpr (SAVE) p.save_dnorm[g] = rp.dnorm;
-        } else {
-          for (int k = 0; k < 3; ++k) { rp.o[k] = 0.f; rp.d[k] = 0.f; rp.bg[k] = 0.f; }
-          rp.dnorm = 0.f;
-          rp.dz = 0.f;
-        }
-      }
+      if (etid < RR) load_ray(p, unit * RR + etid, rayp[etid]);  // ray slot qy = x * R + r
       named_bar_sync(kRowBarrier, kRowThreads);
-      if (etid < RR * 12) {  // direction encoder input (d_z, near, far), train_utils.py:14
-        const int rr = etid / 12, k = etid - rr * 12, f = k / 3, c = k - f * 3;
-        RayP& rp = rayp[rr];
-        const float v = (c == 0) ? rp.dz : (c == 1 ? p.near_ : p.far_);
-        float sn, cs;
-        sincosf(v * (float)(1 << f), &sn, &cs);
-        rp.ped[6 * f + c] = rp.valid ? sn : 0.f;
-        rp.ped[6 * f + 3 + c] = rp.valid ? cs : 0.f;
-      }
+      dir_encoding(p, rayp, RR, etid);
       named_bar_sync(kRowBarrier, kRowThreads);
       tm.lap(0);
 
@@ -361,15 +253,7 @@ __global__ void __launch_bounds__(kThreads, 1) render2_kernel(const __grid_const
         if (p.nf > 0 || it == 0)  // bias block of this pass's network (published by the barrier after the first prologue)
           for (int k = etid; k < kBiasFloats; k += kRowThreads) bias_s[k] = p.bias[pass][k];
 
-        // training record of tile t of stream x in this pass (null outside SAVE mode / beyond the last real unit)
-        auto tile_rec = [&](int x, int t) -> uint8_t* {
-          if constexpr (SAVE) {
-            const int u4 = 2 * unit + x;  // unit index in the one-tile kernel's numbering
-            if (u4 * R < p.n_rays) return p.save_rec + ((size_t)u4 * tiles_per_unit + (pass ? p.tiles_c : 0) + t) * kRecBytes;
-          }
-          return nullptr;
-        };
-        auto prologue = [&](int x, int t) { prologue_fn(p, rayp, carry_z, smem + kOffPe, x, t, pass, S, rows, R, row, ch, tile_rec(x, t)); };
+        auto prologue = [&](int x, int t) { prologue_fn(p, rayp, carry_z, smem + kOffPe, x, t, pass, S, rows, R, row, ch); };
 
         prologue(0, 0);
         prologue(1, 0);
@@ -385,28 +269,6 @@ __global__ void __launch_bounds__(kThreads, 1) render2_kernel(const __grid_const
           if (lane == 0) {  // PE buffers of tile t are in place: first half-step of both streams may start
             mbar_arrive(bar_gate);
             mbar_arrive(bar_gate + 8);
-          }
-          uint8_t* rec0 = tile_rec(0, t);
-          uint8_t* rec1 = tile_rec(1, t);
-          if constexpr (SAVE) {  // direction encoding of each row's ray as a transposed image: features [16 ch, 16 ch + 16)
-#pragma unroll
-            for (int x = 0; x < 2; ++x) {
-              uint8_t* rec = x ? rec1 : rec0;
-              if (rec) {
-                const RayP& rq = rayp[x * R + r];
-                uint8_t* img = rec + kRecPEd + img_row_base(32, row);
-                const uint32_t cr = (uint32_t)((row & 63) >> 3);
-#pragma unroll
-                for (int e = 0; e < 8; ++e) {
-                  const int ka = 16 * ch + 2 * e, kb = ka + 1;
-                  const float a = (live && rq.valid && ka < kDimDir) ? rq.ped[ka] : 0.f;
-                  const float b = (live && rq.valid && kb < kDimDir) ? rq.ped[kb] : 0.f;
-                  const uint32_t w = pack_f16x2(a, b);
-                  *reinterpret_cast<uint16_t*>(img + ka * 128 + ((cr ^ (uint32_t)(ka & 7)) << 4)) = (uint16_t)(w & 0xFFFFu);
-                  *reinterpret_cast<uint16_t*>(img + kb * 128 + ((cr ^ (uint32_t)(kb & 7)) << 4)) = (uint16_t)(w >> 16);
-                }
-              }
-            }
           }
           if (t == 0) {
             // per-ray additive term of layers_dir.0: W[:, 256:280] . PE_dir; thread = (output feature `row`, rays ch and ch+2)
@@ -428,115 +290,24 @@ __global__ void __launch_bounds__(kThreads, 1) render2_kernel(const __grid_const
           uint32_t keep0[32], keep1[32];  // half-0 results of streams X / Y, held until P is dead
           float sigma_raw0 = 0.f, sigma_raw1 = 0.f;
           for (int s = 0; s < kNumSteps; ++s) {
-            const StepInfo si = step_info(s);
-            const int c0 = 64 * ch;
+            const float* bias_s = bias_n + step_info(s).bias_off;
             if (s == 6 && t == 0) named_bar_sync(kRowBarrier, kRowThreads);  // dirbias written by all threads
             for (int h = 0; h < num_halves(s); ++h) {
 #pragma unroll
               for (int x = 0; x < 2; ++x) {
                 const uint32_t t_p = t_lane + (uint32_t)x * 256u;
-                const uint32_t t_q = t_p + 128u;
                 if (x == 0) { mbar_wait(bar_accfull, ph_acc0); ph_acc0 ^= 1; }
                 else        { mbar_wait(bar_accfull + 8, ph_acc1); ph_acc1 ^= 1; }
                 tc_fence_after_sync();
                 tm.lap(10 + s);
-                uint32_t (&keep)[32] = x ? keep1 : keep0;
-                uint32_t hh[32];          // half-1 / single-half result (SAVE: written to the record after the gate)
-                int save_k0 = -1;         // SAVE: first feature of the 64 this event produced, -1: nothing to record
-                bool save_keep = false;   // SAVE: the 64 features are in `keep` (half 0) instead of `hh`
-                bool arrived = false;
-                float& sigma_raw = x ? sigma_raw1 : sigma_raw0;
-                const RayP& rp = rayp[x * R + r];
-                if (s <= 5) {
-                  if (h == 0) {  // outputs [64 ch, +64) of features 0..127 -> registers (gate signalled inside)
-                    epi_load64_early(t_q + c0, smem_u32(bias_n + si.bias_off + c0), 0u, keep, bar_gate + x * 8, lane);
-                    arrived = true;
-                    save_k0 = c0; save_keep = true;
-                  } else {       // P_x is dead: store half 0 (K atom ch), convert half 1 (K atom 2 + ch)
-                    store32(t_p + 32 * ch, keep);
-                    epi_load64(t_q + c0, smem_u32(bias_n + si.bias_off + 128 + c0), 0u, hh);
-                    store32(t_p + 64 + 32 * ch, hh);
-                    tmem_wait_st();
-                    save_k0 = 128 + c0;
-                  }
-                } else if (s == 6) {
-                  if (h == 0) {
-                    epi_load64_early(t_q + c0, smem_u32(bias_n + si.bias_off + c0), smem_u32(dirbias + (x * R + r) * 128 + c0), keep,
-                                     bar_gate + x * 8, lane);
-                    arrived = true;
-                    save_k0 = c0; save_keep = true;
-                  } else {  // sigma = column 0 of the 16-wide second half; then g0 becomes the operand (K = 128)
-                    if (ch == 0) {
-                      uint32_t v[4];
-                      tmem_ld4(t_q, v);
-                      tmem_wait_ld();
-                      sigma_raw = __uint_as_float(v[0]) + bias_n[si.bias_off + 128];
-                    }
-                    store32(t_p + 32 * ch, keep);
-                    tmem_wait_st();
-                  }
-                } else if (s <= 8) {  // 128 -> 128 layers: the MMAs that read P have completed
-                  epi_load64(t_q + c0, smem_u32(bias_n + si.bias_off + c0), 0u, hh);
-                  store32(t_p + 32 * ch, hh);
-                  tmem_wait_st();
-                  save_k0 = c0;
-                } else if (ch == 0) {
-                  // fc_rgb output: colour and sigma per sample for compositing (volume_rendering_utils.py:29-33, 41-53)
-                  uint32_t v[4];
-                  tmem_ld4(t_q, v);
-                  tmem_wait_ld();
-                  const float* b = bias_n + si.bias_off;
-                  if (live) {
-                    const float r0 = __uint_as_float(v[0]) + b[0], r1 = __uint_as_float(v[1]) + b[1], r2 = __uint_as_float(v[2]) + b[2];
-                    if (rp.valid) {
-                      float* dr = pass ? p.dbg_raw_f : p.dbg_raw_c;
-                      if (dr) reinterpret_cast<float4*>(dr)[(size_t)rp.gidx * S + i] = make_float4(r0, r1, r2, sigma_raw);
-                    }
-                    float sig = sigma_raw;
-                    if (p.noise_std > 0.f && rp.valid)
-                      sig = __fadd_rn(sig, __fmul_rn((pass ? p.noise_f : p.noise_c)[(size_t)rp.gidx * S + i], p.noise_std));
-                    const float sig_in = sig;  // what the ReLU sees (volume_rendering_utils.py:52)
-                    sig = fmaxf(sig, 0.f);
-                    float4 pre;
-                    if (i == S - 1) {
-                      sig = __fadd_rn(sig, 1e-6f);
-                      if (has_bg) { pre.x = rp.bg[0]; pre.y = rp.bg[1]; pre.z = rp.bg[2]; }
-                    }
-                    if (!(has_bg && i == S - 1)) {
-                      pre.x = 1.f / (1.f + expf(-r0));
-                      pre.y = 1.f / (1.f + expf(-r1));
-                      pre.z = 1.f / (1.f + expf(-r2));
-                    }
-                    pre.w = sig;
-                    carry_raw[x * kRowsMax + prow] = pre;
-                    if constexpr (SAVE) {  // what the compositing backward needs: colour (or bg) and the ReLU input
-                      if (rp.valid) reinterpret_cast<float4*>(pass ? p.save_raw_f : p.save_raw_c)[(size_t)rp.gidx * S + i] = make_float4(pre.x, pre.y, pre.z, sig_in);
-                    }
-                  }
-                }
-                if (s < kNumSteps - 1 && !arrived) {  // Q_x has been read (and, after a step's last half, P_x holds the next operand)
-                  tc_fence_before_sync();
-                  __syncwarp();
-                  if (lane == 0) mbar_arrive(bar_gate + x * 8);
-                }
-                if constexpr (SAVE) {  // after the gate: activation image + ReLU mask of the 64 features this event produced
-                  uint8_t* rec = x ? rec1 : rec0;
-                  if (rec && save_k0 >= 0) {
-                    uint32_t a[16], b[16];
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) { a[j] = save_keep ? keep[j] : hh[j]; b[j] = save_keep ? keep[16 + j] : hh[16 + j]; }
-                    uint8_t* img = rec + rec_x_off(s) + img_row_base(rec_width(s), row);
-                    store_t32(img, row, save_k0, a);
-                    store_t32(img, row, save_k0 + 32, b);
-                    *reinterpret_cast<uint2*>(reinterpret_cast<uint32_t*>(rec + kRecMask) + (s * 128 + row) * 8 + (save_k0 >> 5)) =
-                        make_uint2(relu_mask32(a), relu_mask32(b));
-                  }
-                }
+                epilogue_event(p, s, h, t_p, t_p + 128u, bar_gate + x * 8, bias_s, dirbias + (x * R + r) * 128, x ? keep1 : keep0,
+                               x ? sigma_raw1 : sigma_raw0, rayp[x * R + r], has_bg, live, pass, S, i, ch, lane,
+                               carry_raw + x * kRowsMax + prow, pass ? p.dbg_raw_f : p.dbg_raw_c);
                 tm.lap(20 + s);
               }
             }
-            if (s == 3 && t + 1 < n_tiles && !(kHelper && pass == 1)) {  // both PE buffers are free: encode the next tile pair
-                                                                         // under steps 4..9 (fine pass: the helper warp does it)
+            if (s == 3 && t + 1 < n_tiles && pass == 0) {  // both PE buffers are free: encode the next tile pair under steps
+                                                           // 4..9 (fine pass: the helper warp does it)
               prologue(0, t + 1);
               prologue(1, t + 1);
               tm.lap(2);
@@ -583,37 +354,10 @@ __global__ void __launch_bounds__(kThreads, 1) render2_kernel(const __grid_const
         // ---- inverse-CDF resampling (nerf_helpers.py:344-387) on weights[1:-1] over the mid-point bins
         __syncwarp();
         const int nb = p.nc - 1;
-        const int nw = p.nc - 2;
         if (ew < RR) {
           const int x = ew / R, rr = ew - x * R;
           const int base = x * kRowsMax + rr * p.nc;
-          const float* w = scr_w + base;
-          const float* zc = carry_z + base;
-          float* cdf = scr_cdf + base;
-          float* bins = scr_bins + base;
-          for (int k = lane; k < nb; k += 32) bins[k] = __fmul_rn(0.5f, __fadd_rn(zc[k + 1], zc[k]));
-          const int per = (nw + 31) >> 5;
-          const int k0 = lane * per;
-          float part = 0.f;
-          for (int j = 0; j < per; ++j)
-            if (k0 + j < nw) part += __fadd_rn(w[k0 + j + 1], 1e-5f);
-          const float total = warp_sum(part);
-          float psum = 0.f;
-          for (int j = 0; j < per; ++j)
-            if (k0 + j < nw) psum += __fdiv_rn(__fadd_rn(w[k0 + j + 1], 1e-5f), total);
-          float incl = psum;
-#pragma unroll
-          for (int o = 1; o < 32; o <<= 1) {
-            const float tt = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= o) incl += tt;
-          }
-          float run = incl - psum;
-          if (lane == 0) cdf[0] = 0.f;
-          for (int j = 0; j < per; ++j)
-            if (k0 + j < nw) {
-              run += __fdiv_rn(__fadd_rn(w[k0 + j + 1], 1e-5f), total);
-              cdf[k0 + j + 1] = run;
-            }
+          build_cdf(scr_w + base, carry_z + base, scr_cdf + base, scr_bins + base, p.nc, lane);
         }
         named_bar_sync(kRowBarrier, kRowThreads);
         tm.lap(5);
@@ -627,50 +371,19 @@ __global__ void __launch_bounds__(kThreads, 1) render2_kernel(const __grid_const
             val = carry_z[x * kRowsMax + rr * p.nc + i];
           } else {
             const int j = i - p.nc;
-            const float* cdf = scr_cdf + x * kRowsMax + rr * p.nc;
-            const float* bins = scr_bins + x * kRowsMax + rr * p.nc;
             const float u = p.perturb ? (rayp[qy].valid ? p.u_rand[(size_t)rayp[qy].gidx * p.nf + j] : 0.f) : p.u_fine[j];
-            int lo = 0, hi = nb;  // searchsorted(..., right=True)
-            while (lo < hi) {
-              const int mid = (lo + hi) >> 1;
-              if (cdf[mid] <= u) lo = mid + 1; else hi = mid;
-            }
-            const int below = max(0, lo - 1), above = min(nb - 1, lo);
-            const float cb = cdf[below], ca = cdf[above];
-            float den = __fsub_rn(ca, cb);
-            if (den < 1e-5f) den = 1.f;
-            const float tt = __fdiv_rn(__fsub_rn(u, cb), den);
-            val = __fadd_rn(bins[below], __fmul_rn(tt, __fsub_rn(bins[above], bins[below])));
+            val = sample_pdf(scr_cdf + x * kRowsMax + rr * p.nc, scr_bins + x * kRowsMax + rr * p.nc, nb, u);
           }
           scr_sort[x * kRowsMax + rr * SF + i] = val;
         }
         named_bar_sync(kRowBarrier, kRowThreads);
         tm.lap(6);
-        // ---- torch.sort(cat(z, z_samples)) (train_utils.py:126) as a rank merge (see nfb_render.cu)
+        // ---- torch.sort(cat(z, z_samples)) (train_utils.py:126) as a rank merge
         for (int k = etid; k < RR * SF; k += kRowThreads) {
           const int qy = k / SF, i = k - qy * SF;
           const int x = qy / R, rr = qy - x * R;
-          const float* zc = scr_sort + x * kRowsMax + rr * SF;
-          const float* zs = zc + p.nc;
-          const float v = zc[i];
-          int rank;
-          if (i < p.nc) {
-            rank = i;
-            for (int j = 0; j < p.nf; ++j) rank += (zs[j] < v) ? 1 : 0;
-          } else {
-            const int jm = i - p.nc;
-            int lo = 0, hi = p.nc;
-            while (lo < hi) {
-              const int mid = (lo + hi) >> 1;
-              if (zc[mid] <= v) lo = mid + 1; else hi = mid;
-            }
-            rank = lo;
-            for (int j = 0; j < p.nf; ++j) {
-              const float y = zs[j];
-              rank += (y < v || (y == v && j < jm)) ? 1 : 0;
-            }
-          }
-          carry_z[x * kRowsMax + rr * SF + rank] = v;
+          const float* z = scr_sort + x * kRowsMax + rr * SF;
+          carry_z[x * kRowsMax + rr * SF + merge_rank(z, p.nc, p.nf, i)] = z[i];
         }
         named_bar_sync(kRowBarrier, kRowThreads);
         tm.lap(7);
@@ -717,35 +430,14 @@ int debug_prog_v6(int index, uint32_t* out) {  // host copy of the two-tile prog
 }
 
 cudaError_t render2_kernel_setup() {
-  cudaError_t e = cudaFuncSetAttribute(v6::render2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, v6::kSmemBytes);
-  if (e != cudaSuccess) return e;
-  return cudaFuncSetAttribute(v6::render2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, v6::kSmemBytes);
+  return cudaFuncSetAttribute(v6::render2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, v6::kSmemBytes);
 }
 
 // `p` is prepared for the one-tile kernel (n_units = units of R rays); here a unit of work is 2R rays.
 cudaError_t launch_render2(const RenderParams& p_in, int num_sms, cudaStream_t st, long long* launches) {
   RenderParams p = p_in;
   p.n_units = (p_in.n_rays + 2 * p_in.rays_per_unit - 1) / (2 * p_in.rays_per_unit);
-  int grid = p.n_units < num_sms ? p.n_units : num_sms;
-  if (grid <= 0) return cudaSuccess;
-  grid = (grid + v6::kCluster - 1) / v6::kCluster * v6::kCluster;
-  if (grid > num_sms) grid = num_sms / v6::kCluster * v6::kCluster;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(v6::kThreads);
-  cfg.dynamicSmemBytes = v6::kSmemBytes;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = v6::kCluster;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  cudaError_t e = p.save_rec ? cudaLaunchKernelEx(&cfg, v6::render2_kernel<true>, p)   // training forward: writes the records
-                             : cudaLaunchKernelEx(&cfg, v6::render2_kernel<false>, p);
-  ++*launches;
-  return e != cudaSuccess ? e : cudaGetLastError();
+  return launch_clustered(v6::render2_kernel, p, v6::kCluster, v6::kThreads, v6::kSmemBytes, num_sms, st, launches);
 }
 
 }  // namespace nfb

@@ -35,7 +35,6 @@
 #include "nfb_layout.h"
 #include "nfb_ptx.cuh"
 #include "nfb_render_common.cuh"
-#include "nfb_save.cuh"
 #include "nfb_tile2.cuh"
 
 namespace nfb {
@@ -103,72 +102,16 @@ template <int N> __device__ __forceinline__ void reg_inc() { asm volatile("setma
 // Positional encoding of sample row `row` (lane half `ch`) of tile t of one stream -> PE buffer (63 lanes + zero pad, FP16,
 // 128-byte swizzled).  z comes from the stream's depth buffer; rows beyond the pass encode depth 0 of ray 0 (never read back).
 __device__ __forceinline__ void encode_row(const RayP* __restrict__ rays_x /* the stream's R rays */, const float* __restrict__ z_x,
-                                           uint8_t* __restrict__ pe, int t, int S, int rows, int row, int ch,
-                                           uint8_t* __restrict__ rec /* training record of the tile, or null */) {
+                                           uint8_t* __restrict__ pe, int t, int S, int rows, int row, int ch) {
   const int prow = t * 128 + row;
   const bool live = prow < rows;
   const int r = live ? prow / S : 0;
-  const RayP& rp = rays_x[r];
   const float z = live ? z_x[prow] : 0.f;
-  const float px = __fadd_rn(rp.o[0], __fmul_rn(rp.d[0], z));
-  const float py = __fadd_rn(rp.o[1], __fmul_rn(rp.d[1], z));
-  const float pz = __fadd_rn(rp.o[2], __fmul_rn(rp.d[2], z));
   float f[32];
-  if (ch == 0) {  // lanes 0..31: xyz, frequencies 0..3, sin of frequency 4, cos(x), cos(y) of frequency 4
-    f[0] = px; f[1] = py; f[2] = pz;
-#pragma unroll
-    for (int fr = 0; fr < 4; ++fr) {
-      const float sc = (float)(1 << fr);
-      pe_sincos<false>(px * sc, f[3 + 6 * fr + 0], f[3 + 6 * fr + 3]);
-      pe_sincos<false>(py * sc, f[3 + 6 * fr + 1], f[3 + 6 * fr + 4]);
-      pe_sincos<false>(pz * sc, f[3 + 6 * fr + 2], f[3 + 6 * fr + 5]);
-    }
-    float cz;
-    pe_sincos<false>(px * 16.f, f[27], f[30]);
-    pe_sincos<false>(py * 16.f, f[28], f[31]);
-    pe_sincos<false>(pz * 16.f, f[29], cz);
-  } else {        // lanes 32..63: cos(z) of frequency 4, frequencies 5..9, zero pad
-    float sz;
-    pe_sincos<false>(pz * 16.f, sz, f[0]);
-#pragma unroll
-    for (int fr = 5; fr < 10; ++fr) {
-      const float sc = (float)(1 << fr);
-      const int b = 6 * fr - 29;
-      pe_sincos<false>(px * sc, f[b + 0], f[b + 3]);
-      pe_sincos<false>(py * sc, f[b + 1], f[b + 4]);
-      pe_sincos<false>(pz * sc, f[b + 2], f[b + 5]);
-    }
-    f[31] = 0.f;
-  }
-  uint32_t hh[16];
-#pragma unroll
-  for (int qq = 0; qq < 4; ++qq) {
-#pragma unroll
-    for (int e = 0; e < 4; ++e) hh[qq * 4 + e] = pack_f16x2(f[qq * 8 + 2 * e], f[qq * 8 + 2 * e + 1]);
-    const int off = row * 128 + (((ch * 4 + qq) ^ (row & 7)) << 4);
-    *reinterpret_cast<uint4*>(pe + off) = make_uint4(hh[qq * 4], hh[qq * 4 + 1], hh[qq * 4 + 2], hh[qq * 4 + 3]);
-  }
-  if (rec) {  // training: the same 32 lanes as a transposed FP16 image for the weight gradients, and the row's ray's direction
-              // encoding (features [16 ch, 16 ch + 16) of 24) replicated per sample
-    store_t32(rec + kRecPE + img_row_base(64, row), row, 32 * ch, hh);
-    uint8_t* img = rec + kRecPEd + img_row_base(32, row);
-    const uint32_t cr = (uint32_t)((row & 63) >> 3);
-#pragma unroll
-    for (int e = 0; e < 8; ++e) {
-      const int ka = 16 * ch + 2 * e, kb = ka + 1;
-      const float a = (live && rp.valid && ka < kDimDir) ? rp.ped[ka] : 0.f;
-      const float b = (live && rp.valid && kb < kDimDir) ? rp.ped[kb] : 0.f;
-      const uint32_t w = pack_f16x2(a, b);
-      *reinterpret_cast<uint16_t*>(img + ka * 128 + ((cr ^ (uint32_t)(ka & 7)) << 4)) = (uint16_t)(w & 0xFFFFu);
-      *reinterpret_cast<uint16_t*>(img + kb * 128 + ((cr ^ (uint32_t)(kb & 7)) << 4)) = (uint16_t)(w >> 16);
-    }
-  }
+  pe_lanes<false>(rays_x[r], z, ch, f);
+  store_pe_row<false>(f, pe, nullptr, row, ch);
 }
 
-// SAVE = training forward: also writes the per-tile activation records (nfb_layout.h kRec*), per-sample (colour, ReLU input of
-// sigma), depths and |d| that nfb_render_backward reads — the same records as the one-tile kernel (unit 2U + x there = stream x
-// of unit U here).
-template <bool SAVE>
 __global__ void __launch_bounds__(kThreads, 1) render3_kernel(const __grid_constant__ RenderParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   const uint32_t smem_base = smem_u32(smem);
@@ -217,14 +160,6 @@ __global__ void __launch_bounds__(kThreads, 1) render3_kernel(const __grid_const
   const int first_in_cluster = (int)blockIdx.x - (int)cta_rank;
   const int n_iter = (p.n_units - first_in_cluster + (int)gridDim.x - 1) / (int)gridDim.x;  // units of work (2R rays) of this CTA
   const int Tc = p.tiles_c, Tf = p.tiles_f;
-  // training record of tile t of `pass` of stream x of unit iteration `it` (null outside SAVE mode / beyond the last real ray)
-  auto tile_rec = [&](int it, int pass, int x, int t) -> uint8_t* {
-    if constexpr (SAVE) {
-      const int u4 = 2 * ((int)blockIdx.x + it * (int)gridDim.x) + x;  // unit index in the one-tile kernel's numbering
-      if (u4 * p.rays_per_unit < p.n_rays) return p.save_rec + ((size_t)u4 * (Tc + Tf) + (pass ? Tc : 0) + t) * kRecBytes;
-    }
-    return nullptr;
-  };
 
   // The job sequence every role walks (JobIt):  block b = -1: C(0);  block b >= 0: C(b+1) (if it exists), then F(b, 0..Tf-1).
   // A job is (u = the unit's iteration index, pass 0/1, t = tile pair of the pass).
@@ -302,13 +237,10 @@ __global__ void __launch_bounds__(kThreads, 1) render3_kernel(const __grid_const
       mbar_wait(bar_peready + 8, ph_per);
       ph_per ^= 1;
 
-      uint8_t* rec0 = tile_rec(u, pass, 0, t);
-      uint8_t* rec1 = tile_rec(u, pass, 1, t);
       uint32_t keep0[32], keep1[32];  // half-0 results of streams X / Y, held until P is dead
       float sigma_raw0 = 0.f, sigma_raw1 = 0.f;
       for (int s = 0; s < kNumSteps; ++s) {
-        const StepInfo si = step_info(s);
-        const int c0 = 64 * ch;
+        const float* bias_s = bias_n + step_info(s).bias_off;
         if (s == kNumSteps - 1 && t == 0) {  // about to overwrite the pass's (colour, sigma) buffer: previous unit composited?
           if (pass == 0) { mbar_wait(bar_rawfree, ph_rawfree0 ^ 1); ph_rawfree0 ^= 1; }
           else           { mbar_wait(bar_rawfree + 8, ph_rawfree1 ^ 1); ph_rawfree1 ^= 1; }
@@ -317,98 +249,12 @@ __global__ void __launch_bounds__(kThreads, 1) render3_kernel(const __grid_const
 #pragma unroll
           for (int x = 0; x < 2; ++x) {
             const uint32_t t_p = t_lane + (uint32_t)x * 256u;
-            const uint32_t t_q = t_p + 128u;
             if (x == 0) { mbar_wait(bar_accfull, ph_acc0); ph_acc0 ^= 1; }
             else        { mbar_wait(bar_accfull + 8, ph_acc1); ph_acc1 ^= 1; }
             tc_fence_after_sync();
-            uint32_t (&keep)[32] = x ? keep1 : keep0;
-            uint32_t hh[32];
-            bool arrived = false;
-            int save_k0 = -1;         // SAVE: first feature of the 64 this event produced, -1: nothing to record
-            bool save_keep = false;   // SAVE: the 64 features are in `keep` (half 0) instead of `hh`
-            float& sigma_raw = x ? sigma_raw1 : sigma_raw0;
-            const RayP& rp = rayp[x * R + r];
-            if (s <= 5) {
-              if (h == 0) {  // outputs [64 ch, +64) of features 0..127 -> registers (gate signalled inside)
-                epi_load64_early(t_q + c0, smem_u32(bias_n + si.bias_off + c0), 0u, keep, bar_gate + x * 8, lane);
-                arrived = true;
-                save_k0 = c0; save_keep = true;
-              } else {       // P_x is dead: store half 0 (K atom ch), convert half 1 (K atom 2 + ch)
-                store32(t_p + 32 * ch, keep);
-                epi_load64(t_q + c0, smem_u32(bias_n + si.bias_off + 128 + c0), 0u, hh);
-                store32(t_p + 64 + 32 * ch, hh);
-                tmem_wait_st();
-                save_k0 = 128 + c0;
-              }
-            } else if (s == 6) {
-              if (h == 0) {
-                epi_load64_early(t_q + c0, smem_u32(bias_n + si.bias_off + c0), smem_u32(dirbias + (x * R + r) * 128 + c0), keep,
-                                 bar_gate + x * 8, lane);
-                arrived = true;
-                save_k0 = c0; save_keep = true;
-              } else {  // sigma = column 0 of the 16-wide second half; then g0 becomes the operand (K = 128)
-                if (ch == 0) {
-                  uint32_t v[4];
-                  tmem_ld4(t_q, v);
-                  tmem_wait_ld();
-                  sigma_raw = __uint_as_float(v[0]) + bias_n[si.bias_off + 128];
-                }
-                store32(t_p + 32 * ch, keep);
-                tmem_wait_st();
-              }
-            } else if (s <= 8) {  // 128 -> 128 layers: the MMAs that read P have completed
-              epi_load64(t_q + c0, smem_u32(bias_n + si.bias_off + c0), 0u, hh);
-              store32(t_p + 32 * ch, hh);
-              tmem_wait_st();
-              save_k0 = c0;
-            } else if (ch == 0) {
-              // fc_rgb output: colour and sigma per sample for compositing (volume_rendering_utils.py:29-33, 41-53)
-              uint32_t v[4];
-              tmem_ld4(t_q, v);
-              tmem_wait_ld();
-              const float* b = bias_n + si.bias_off;
-              if (live) {
-                const float r0 = __uint_as_float(v[0]) + b[0], r1 = __uint_as_float(v[1]) + b[1], r2 = __uint_as_float(v[2]) + b[2];
-                float sig = sigma_raw;
-                if (p.noise_std > 0.f && rp.valid)
-                  sig = __fadd_rn(sig, __fmul_rn((pass ? p.noise_f : p.noise_c)[(size_t)rp.gidx * S + i], p.noise_std));
-                const float sig_in = sig;  // what the ReLU sees (volume_rendering_utils.py:52)
-                sig = fmaxf(sig, 0.f);
-                float4 pre;
-                if (i == S - 1) {
-                  sig = __fadd_rn(sig, 1e-6f);
-                  if (has_bg) { pre.x = rp.bg[0]; pre.y = rp.bg[1]; pre.z = rp.bg[2]; }
-                }
-                if (!(has_bg && i == S - 1)) {
-                  pre.x = 1.f / (1.f + expf(-r0));
-                  pre.y = 1.f / (1.f + expf(-r1));
-                  pre.z = 1.f / (1.f + expf(-r2));
-                }
-                pre.w = sig;
-                raw[x * raw_stride + prow] = pre;
-                if constexpr (SAVE) {  // what the compositing backward needs: colour (or bg) and the ReLU input
-                  if (rp.valid) reinterpret_cast<float4*>(pass ? p.save_raw_f : p.save_raw_c)[(size_t)rp.gidx * S + i] = make_float4(pre.x, pre.y, pre.z, sig_in);
-                }
-              }
-            }
-            if (s < kNumSteps - 1 && !arrived) {  // Q_x has been read (and, after a step's last half, P_x holds the next operand)
-              tc_fence_before_sync();
-              __syncwarp();
-              if (lane == 0) mbar_arrive(bar_gate + x * 8);
-            }
-            if constexpr (SAVE) {  // after the gate: activation image + ReLU mask of the 64 features this event produced
-              uint8_t* rec = x ? rec1 : rec0;
-              if (rec && save_k0 >= 0) {
-                uint32_t a[16], b[16];
-#pragma unroll
-                for (int j = 0; j < 16; ++j) { a[j] = save_keep ? keep[j] : hh[j]; b[j] = save_keep ? keep[16 + j] : hh[16 + j]; }
-                uint8_t* img = rec + rec_x_off(s) + img_row_base(rec_width(s), row);
-                store_t32(img, row, save_k0, a);
-                store_t32(img, row, save_k0 + 32, b);
-                *reinterpret_cast<uint2*>(reinterpret_cast<uint32_t*>(rec + kRecMask) + (s * 128 + row) * 8 + (save_k0 >> 5)) =
-                    make_uint2(relu_mask32(a), relu_mask32(b));
-              }
-            }
+            epilogue_event(p, s, h, t_p, t_p + 128u, bar_gate + x * 8, bias_s, dirbias + (x * R + r) * 128, x ? keep1 : keep0,
+                           x ? sigma_raw1 : sigma_raw0, rayp[x * R + r], has_bg, live, pass, S, i, ch, lane, raw + x * raw_stride + prow,
+                           nullptr);
           }
         }
       }
@@ -437,7 +283,6 @@ __global__ void __launch_bounds__(kThreads, 1) render3_kernel(const __grid_const
     const float4* raw_f = reinterpret_cast<const float4*>(smem + kOffRawF);
     const int R = p.rays_per_unit, RR = 2 * R;
     const int nc = p.nc, nf = p.nf, SF = p.s_fine;
-    const bool has_bg = p.bg != nullptr;
     int P2 = 1;                                   // fine samples of one ray padded to a power of two for the bitonic network
     while (P2 < nf) P2 <<= 1;
     uint32_t ph_pefree = 1;                       // first wait passes: nothing has read the PE buffers yet
@@ -448,47 +293,9 @@ __global__ void __launch_bounds__(kThreads, 1) render3_kernel(const __grid_const
     auto ray_setup = [&](int it) {
       RayP* rayp = rayp_all + (it % 3) * 4;
       const int unit = blockIdx.x + it * gridDim.x;
-      if (stid < RR) {
-        RayP& rp = rayp[stid];
-        const int g = unit * RR + stid;
-        rp.valid = g < p.n_rays;
-        rp.gidx = g;
-        if (rp.valid) {
-          float o0, o1, o2, d0, d1, d2;
-          if (p.o) {
-            o0 = p.o[3 * g]; o1 = p.o[3 * g + 1]; o2 = p.o[3 * g + 2];
-            d0 = p.d[3 * g]; d1 = p.d[3 * g + 1]; d2 = p.d[3 * g + 2];
-          } else {  // get_ray_bundle (nerf_helpers.py:111-122), same operation order in FP32
-            const int pj = p.row_begin + g / p.width, pi = g % p.width;
-            const float cx = __fdiv_rn(__fsub_rn((float)pi, p.wcx), p.fx);
-            const float cy = -__fdiv_rn(__fsub_rn((float)pj, p.hcy), p.fy);
-            d0 = __fadd_rn(__fadd_rn(__fmul_rn(cx, p.pose[0]), __fmul_rn(cy, p.pose[1])), __fmul_rn(-1.f, p.pose[2]));
-            d1 = __fadd_rn(__fadd_rn(__fmul_rn(cx, p.pose[4]), __fmul_rn(cy, p.pose[5])), __fmul_rn(-1.f, p.pose[6]));
-            d2 = __fadd_rn(__fadd_rn(__fmul_rn(cx, p.pose[8]), __fmul_rn(cy, p.pose[9])), __fmul_rn(-1.f, p.pose[10]));
-            o0 = p.pose[3]; o1 = p.pose[7]; o2 = p.pose[11];
-          }
-          rp.o[0] = o0; rp.o[1] = o1; rp.o[2] = o2;
-          rp.d[0] = d0; rp.d[1] = d1; rp.d[2] = d2;
-          rp.dnorm = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(d0, d0), __fmul_rn(d1, d1)), __fmul_rn(d2, d2)));
-          if (has_bg) { rp.bg[0] = p.bg[3 * g]; rp.bg[1] = p.bg[3 * g + 1]; rp.bg[2] = p.bg[3 * g + 2]; }
-          rp.dz = p.dir_z ? p.dir_z[g] : d2;
-          if constexpr (SAVE) p.save_dnorm[g] = rp.dnorm;
-        } else {
-          for (int k = 0; k < 3; ++k) { rp.o[k] = 0.f; rp.d[k] = 0.f; rp.bg[k] = 0.f; }
-          rp.dnorm = 0.f;
-          rp.dz = 0.f;
-        }
-      }
+      if (stid < RR) load_ray(p, unit * RR + stid, rayp[stid]);
       sbar();
-      if (stid < RR * 12) {  // direction encoder input (d_z, near, far), train_utils.py:14
-        const int rr = stid / 12, k = stid - rr * 12, f = k / 3, c = k - f * 3;
-        RayP& rp = rayp[rr];
-        const float v = (c == 0) ? rp.dz : (c == 1 ? p.near_ : p.far_);
-        float sn, cs;
-        sincosf(v * (float)(1 << f), &sn, &cs);
-        rp.ped[6 * f + c] = rp.valid ? sn : 0.f;
-        rp.ped[6 * f + 3 + c] = rp.valid ? cs : 0.f;
-      }
+      dir_encoding(p, rayp, RR, stid);
       sbar();
     };
     // per-ray additive term of layers_dir.0 of network `pass`: W[:, 256:280] . PE_dir; thread = output feature
@@ -513,28 +320,7 @@ __global__ void __launch_bounds__(kThreads, 1) render3_kernel(const __grid_const
       for (int k = stid; k < RR * nc; k += kSamplerThreads) {
         const int e = k / nc, i = k - e * nc;
         const int x = e / R, rr = e - x * R;
-        const RayP& rp = rayp[e];
-        const float tc = p.t_coarse[i];
-        float z = __fadd_rn(__fmul_rn(p.near_, __fsub_rn(1.f, tc)), __fmul_rn(p.far_, tc));
-        if (p.perturb) {
-          float lower = z, upper = z;
-          if (i > 0) {
-            const float tp = p.t_coarse[i - 1];
-            const float zp = __fadd_rn(__fmul_rn(p.near_, __fsub_rn(1.f, tp)), __fmul_rn(p.far_, tp));
-            lower = __fmul_rn(0.5f, __fadd_rn(z, zp));
-          }
-          if (i < nc - 1) {
-            const float tn = p.t_coarse[i + 1];
-            const float zn = __fadd_rn(__fmul_rn(p.near_, __fsub_rn(1.f, tn)), __fmul_rn(p.far_, tn));
-            upper = __fmul_rn(0.5f, __fadd_rn(zn, z));
-          }
-          const float tr = rp.valid ? p.t_rand[(size_t)rp.gidx * nc + i] : 0.f;
-          z = __fadd_rn(lower, __fmul_rn(__fsub_rn(upper, lower), tr));
-        }
-        zc[x * kRowsC + rr * nc + i] = z;
-        if constexpr (SAVE) {
-          if (rp.valid) p.dbg_z_c[(size_t)rp.gidx * nc + i] = z;  // depths of the coarse pass for the compositing backward
-        }
+        zc[x * kRowsC + rr * nc + i] = coarse_depth(p, rayp[e], i, nc);
       }
     };
     // positional encoding of tile t of `pass` of both streams into the PE buffers, each after its previous reader is done
@@ -549,7 +335,7 @@ __global__ void __launch_bounds__(kThreads, 1) render3_kernel(const __grid_const
         uint8_t* pe = smem + kOffPe + x * (kTileM * 128);
         for (int k = 0; k < 2; ++k) {  // 128 rows x 2 lane halves = 256 thread-tasks for 128 threads
           const int idx = k * kSamplerThreads + stid;
-          encode_row(rayp + x * R, z_x, pe, t, S, rows, idx & 127, idx >> 7, tile_rec(it, pass, x, t));
+          encode_row(rayp + x * R, z_x, pe, t, S, rows, idx & 127, idx >> 7);
         }
         fence_proxy_async_smem();  // generic-proxy stores -> visible to the tensor core's async-proxy reads
         __syncwarp();
@@ -607,37 +393,11 @@ __global__ void __launch_bounds__(kThreads, 1) render3_kernel(const __grid_const
       composite_pass(it, 0);
       // ---- inverse-CDF resampling (nerf_helpers.py:344-387) on weights[1:-1] over the mid-point bins
       __syncwarp();
-      const int nb = nc - 1, nw = nc - 2;
+      const int nb = nc - 1;
       if (sw < RR) {
         const int x = sw / R, rr = sw - x * R;
         const int base = x * kRowsC + rr * nc;
-        const float* w = scr_w + base;
-        const float* z = zc + base;
-        float* cdf = scr_cdf + base;
-        float* bins = scr_bins + base;
-        for (int k = lane; k < nb; k += 32) bins[k] = __fmul_rn(0.5f, __fadd_rn(z[k + 1], z[k]));
-        const int per = (nw + 31) >> 5;
-        const int k0 = lane * per;
-        float part = 0.f;
-        for (int j = 0; j < per; ++j)
-          if (k0 + j < nw) part += __fadd_rn(w[k0 + j + 1], 1e-5f);
-        const float total = warp_sum(part);
-        float psum = 0.f;
-        for (int j = 0; j < per; ++j)
-          if (k0 + j < nw) psum += __fdiv_rn(__fadd_rn(w[k0 + j + 1], 1e-5f), total);
-        float incl = psum;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-          const float tt = __shfl_up_sync(0xffffffffu, incl, o);
-          if (lane >= o) incl += tt;
-        }
-        float run = incl - psum;
-        if (lane == 0) cdf[0] = 0.f;
-        for (int j = 0; j < per; ++j)
-          if (k0 + j < nw) {
-            run += __fdiv_rn(__fadd_rn(w[k0 + j + 1], 1e-5f), total);
-            cdf[k0 + j + 1] = run;
-          }
+        build_cdf(scr_w + base, zc + base, scr_cdf + base, scr_bins + base, nc, lane);
       }
       sbar();
       if (stid == 0) mbar_arrive(bar_rawfree);  // the coarse (colour, sigma) buffer may be overwritten by C(it + 1)
@@ -648,20 +408,8 @@ __global__ void __launch_bounds__(kThreads, 1) render3_kernel(const __grid_const
         float val = CUDART_INF_F;
         if (j < nf) {
           const int x = e / R, rr = e - x * R;
-          const float* cdf = scr_cdf + x * kRowsC + rr * nc;
-          const float* bins = scr_bins + x * kRowsC + rr * nc;
           const float u = p.perturb ? (rayp[e].valid ? p.u_rand[(size_t)rayp[e].gidx * nf + j] : 0.f) : p.u_fine[j];
-          int lo = 0, hi = nb;  // searchsorted(..., right=True)
-          while (lo < hi) {
-            const int mid = (lo + hi) >> 1;
-            if (cdf[mid] <= u) lo = mid + 1; else hi = mid;
-          }
-          const int below = max(0, lo - 1), above = min(nb - 1, lo);
-          const float cb = cdf[below], ca = cdf[above];
-          float den = __fsub_rn(ca, cb);
-          if (den < 1e-5f) den = 1.f;
-          const float tt = __fdiv_rn(__fsub_rn(u, cb), den);
-          val = __fadd_rn(bins[below], __fmul_rn(tt, __fsub_rn(bins[above], bins[below])));
+          val = sample_pdf(scr_cdf + x * kRowsC + rr * nc, scr_bins + x * kRowsC + rr * nc, nb, u);
         }
         scr_sort[k] = val;
       }
@@ -709,12 +457,6 @@ __global__ void __launch_bounds__(kThreads, 1) render3_kernel(const __grid_const
         zf[x * kRowsF + rr * SF + rank] = v;
       }
       sbar();
-      if constexpr (SAVE) {  // sorted depths of the fine pass for the compositing backward
-        for (int k = stid; k < RR * SF; k += kSamplerThreads) {
-          const int e = k / SF, i = k - e * SF;
-          if (rayp[e].valid) p.dbg_z_f[(size_t)rayp[e].gidx * SF + i] = zf[(e / R) * kRowsF + (e - (e / R) * R) * SF + i];
-        }
-      }
     };
     auto finish_fine = [&](int it) {  // F(it) complete -> composite it, then its buffers are free
       mbar_wait(bar_rawready + 8, ph_rawready1);
@@ -770,19 +512,17 @@ int debug_jobs_v7(int n_iter, int tc, int tf, int index, uint32_t* out) {
 }
 
 cudaError_t render3_kernel_setup() {
-  cudaError_t e = cudaFuncSetAttribute(v7::render3_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, v7::kSmemBytes);
-  if (e != cudaSuccess) return e;
-  return cudaFuncSetAttribute(v7::render3_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, v7::kSmemBytes);
+  return cudaFuncSetAttribute(v7::render3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, v7::kSmemBytes);
 }
 
 // Configurations the pipelined kernel's fixed shared-memory budget covers (nfb_api.cu falls back to nfb_render2.cu otherwise).
+// It has no training variant and none of the debug outputs.
 bool render3_supports(const RenderParams& p) {
-  if (p.nf <= 0 || p.nc < 3) return false;
+  if (p.nf <= 0 || p.nc < 3 || p.save_rec) return false;
   const int R = p.rays_per_unit;
   int p2 = 1;
   while (p2 < p.nf) p2 <<= 1;
   const bool fits = R * p.nc <= v7::kRowsC && R * p.s_fine <= v7::kRowsF && 2 * R * p2 <= v7::kSortMax && !p.dbg_act && !p.prof;
-  if (p.save_rec) return fits && !p.dbg_raw_c && !p.dbg_raw_f;  // training forward: depths go to dbg_z_c / dbg_z_f, the rest is in the records
   return fits && !p.dbg_z_c && !p.dbg_raw_c && !p.dbg_z_f && !p.dbg_raw_f;
 }
 
@@ -790,25 +530,7 @@ bool render3_supports(const RenderParams& p) {
 cudaError_t launch_render3(const RenderParams& p_in, int num_sms, cudaStream_t st, long long* launches) {
   RenderParams p = p_in;
   p.n_units = (p_in.n_rays + 2 * p_in.rays_per_unit - 1) / (2 * p_in.rays_per_unit);
-  int grid = p.n_units < num_sms ? p.n_units : num_sms;
-  if (grid <= 0) return cudaSuccess;
-  grid = (grid + t2::kCluster - 1) / t2::kCluster * t2::kCluster;
-  if (grid > num_sms) grid = num_sms / t2::kCluster * t2::kCluster;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(v7::kThreads);
-  cfg.dynamicSmemBytes = v7::kSmemBytes;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = t2::kCluster;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  cudaError_t e = p.save_rec ? cudaLaunchKernelEx(&cfg, v7::render3_kernel<true>, p) : cudaLaunchKernelEx(&cfg, v7::render3_kernel<false>, p);
-  ++*launches;
-  return e != cudaSuccess ? e : cudaGetLastError();
+  return launch_clustered(v7::render3_kernel, p, t2::kCluster, v7::kThreads, v7::kSmemBytes, num_sms, st, launches);
 }
 
 }  // namespace nfb

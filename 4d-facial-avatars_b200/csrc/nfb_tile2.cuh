@@ -1,6 +1,6 @@
 // nfb_tile2.cuh — machinery shared by the kernels that keep TWO tiles in flight per SM (nfb_render2.cu: v6, nfb_render3.cu: v7):
 // the per-tile-pair weight program (one LOAD per ring slot), the compile-time-unrolled MMA issue code of one stream, the
-// weight producer's loop body and the epilogue helpers that move a 64-column accumulator chunk through registers.
+// weight producer's loop body and the epilogue of one half-step of one stream.
 // See the header of nfb_render2.cu for the TMEM layout (P_x operand / Q_x accumulator per stream) and the half-step order.
 #pragma once
 #include <cuda_fp16.h>
@@ -23,14 +23,6 @@ constexpr int kRingBytes = kNumSlots * kSlotBytes;
 #define NFB_V6_CLUSTER 2
 #endif
 constexpr int kCluster = NFB_V6_CLUSTER;  // CTAs sharing every weight half-unit through one multicast L2 read
-#ifndef NFB_V6_ISSUE_UNITS
-#define NFB_V6_ISSUE_UNITS 2
-#endif
-#ifndef NFB_V6_ISSUE_INSIDE
-#define NFB_V6_ISSUE_INSIDE 0
-#endif
-constexpr int kIssueUnits = NFB_V6_ISSUE_UNITS;     // weight loads (4 MMAs each) per elected MMA block
-constexpr int kIssueInside = NFB_V6_ISSUE_INSIDE;   // 1: one elected block per half-step group, weights awaited inside it
 
 // Half-steps.  Step s (nfb_layout.h) has 1 or 2 halves; half h covers weight rows [h * nh0, h * nh0 + N_h).
 __host__ __device__ constexpr int num_halves(int s) { return step_info(s).nh1 > 0 ? 2 : 1; }
@@ -138,34 +130,17 @@ template <class F, int... G>
 __device__ __forceinline__ void for_each_group(F& f, std::integer_sequence<int, G...>) {
   (f(std::integral_constant<int, G>{}), ...);
 }
-// loads [I, I + N) of one group.  kIssueInside == 0: kIssueUnits loads per elected block, the whole warp waits for their
-// weights first.  kIssueInside == 1: the group's loads in ONE elected block, the elected lane waits for each load's weights
-// right before its MMAs (the first MMAs are issued while later weights are still arriving).
-template <int I, int K>
-__device__ __forceinline__ void wait_loads(const IssueCtx& c) {
-  if constexpr (K > 0) {
-    mbar_wait(c.bar_full + (I % kNumSlots) * 8, (uint32_t)((I / kNumSlots) & 1));
-    wait_loads<I + 1, K - 1>(c);
-  }
-}
-template <int I, int K, bool WAIT>
-__device__ __forceinline__ void mma_loads(const IssueCtx& c) {
-  if constexpr (K > 0) {
-    if constexpr (WAIT) mbar_wait(c.bar_full + (I % kNumSlots) * 8, (uint32_t)((I / kNumSlots) & 1));
-    issue_load_mmas<I>(c);
-    mma_loads<I + 1, K - 1, WAIT>(c);
-  }
-}
+// loads [I, I + N) of one group, two loads (8 MMAs) per elected block: the whole warp waits for their weights first.
 template <int I, int N>
 __device__ __forceinline__ void issue_loads(const IssueCtx& c) {
   if constexpr (N > 0) {
-    constexpr int K = kIssueInside ? N : (N < kIssueUnits ? N : kIssueUnits);
-    if constexpr (!kIssueInside) {
-      wait_loads<I, K>(c);
-      tc_fence_after_sync();
-    }
+    constexpr int K = N < 2 ? N : 2;
+    mbar_wait(c.bar_full + (I % kNumSlots) * 8, (uint32_t)((I / kNumSlots) & 1));
+    if constexpr (K == 2) mbar_wait(c.bar_full + ((I + 1) % kNumSlots) * 8, (uint32_t)(((I + 1) / kNumSlots) & 1));
+    tc_fence_after_sync();
     if (elect_one()) {
-      mma_loads<I, K, kIssueInside != 0>(c);
+      issue_load_mmas<I>(c);
+      if constexpr (K == 2) issue_load_mmas<I + 1>(c);
       if constexpr (kLoads.l[I + K - 1].last != 0) umma_commit(c.bar_accfull);
     }
     __syncwarp();
@@ -205,6 +180,64 @@ __device__ __forceinline__ void store32(uint32_t t_p, const uint32_t (&h)[32]) {
   for (int j = 0; j < 16; ++j) { a[j] = h[j]; b[j] = h[16 + j]; }
   tmem_st16(t_p, a);
   tmem_st16(t_p + 16, b);
+}
+
+// Epilogue of half h of step s of one stream for this thread's row (its TMEM lane) and columns [64 ch, 64 ch + 64).  t_p / t_q:
+// the stream's operand P / accumulator Q at this lane; gate: the stream's gate barrier; bias: the step's bias block.  A half-0 result is HELD in `keep` until
+// half 1, when P is dead.  Step 6 adds the per-ray direction term dir_row (of the row's ray rp) and leaves sigma's raw value in
+// sigma_raw; step 9 turns it and the colour into what compositing needs -> *pre (live rows; dbg_raw, when not null, gets the raw
+// outputs).  Signals the gate once Q has been read (and P holds the next operand), except after the last step.
+__device__ __forceinline__ void epilogue_event(const RenderParams& p, int s, int h, uint32_t t_p, uint32_t t_q, uint32_t gate,
+                                               const float* bias, const float* dir_row, uint32_t (&keep)[32], float& sigma_raw,
+                                               const RayP& rp, bool has_bg, bool live, int pass, int S, int i, int ch, int lane,
+                                               float4* pre, float* dbg_raw) {
+  const int c0 = 64 * ch;
+  uint32_t hh[32];
+  bool arrived = false;
+  if (s <= 5) {
+    if (h == 0) {  // outputs [64 ch, +64) of features 0..127 -> registers (gate signalled inside)
+      epi_load64_early(t_q + c0, smem_u32(bias + c0), 0u, keep, gate, lane);
+      arrived = true;
+    } else {       // P is dead: store half 0 (K atom ch), convert half 1 (K atom 2 + ch)
+      store32(t_p + 32 * ch, keep);
+      epi_load64(t_q + c0, smem_u32(bias + 128 + c0), 0u, hh);
+      store32(t_p + 64 + 32 * ch, hh);
+      tmem_wait_st();
+    }
+  } else if (s == 6) {
+    if (h == 0) {
+      epi_load64_early(t_q + c0, smem_u32(bias + c0), smem_u32(dir_row + c0), keep, gate, lane);
+      arrived = true;
+    } else {  // sigma = column 0 of the 16-wide second half; then g0 becomes the operand (K = 128)
+      if (ch == 0) {
+        uint32_t v[4];
+        tmem_ld4(t_q, v);
+        tmem_wait_ld();
+        sigma_raw = __uint_as_float(v[0]) + bias[128];
+      }
+      store32(t_p + 32 * ch, keep);
+      tmem_wait_st();
+    }
+  } else if (s <= 8) {  // 128 -> 128 layers: the MMAs that read P have completed
+    epi_load64(t_q + c0, smem_u32(bias + c0), 0u, hh);
+    store32(t_p + 32 * ch, hh);
+    tmem_wait_st();
+  } else if (ch == 0) {  // fc_rgb output
+    uint32_t v[4];
+    tmem_ld4(t_q, v);
+    tmem_wait_ld();
+    if (live) {
+      const float r0 = __uint_as_float(v[0]) + bias[0], r1 = __uint_as_float(v[1]) + bias[1], r2 = __uint_as_float(v[2]) + bias[2];
+      if (dbg_raw && rp.valid) reinterpret_cast<float4*>(dbg_raw)[(size_t)rp.gidx * S + i] = make_float4(r0, r1, r2, sigma_raw);
+      float sig_in;
+      *pre = colour_sigma(p, rp, has_bg, r0, r1, r2, sigma_raw, pass, S, i, sig_in);
+    }
+  }
+  if (s < kNumSteps - 1 && !arrived) {
+    tc_fence_before_sync();
+    __syncwarp();
+    if (lane == 0) mbar_arrive(gate);
+  }
 }
 
 // Weight producer: the 54 loads of one tile pair from the packed stream `base` into the ring (whole warp; elected lane issues).

@@ -262,68 +262,3 @@ def test_parameter_gradients(ctx):
     e = rel_err(ctx.glat, ctx.lat.grad)
     print(f"latent: rel {e:.2e}; worst parameter rel {worst:.2e}")
     assert e < 1e-2
-
-
-@pytest.mark.parametrize("kernel", ["v6", "v7"])
-def test_training_forward_two_tile_matches_one_tile(built_lib, monkeypatch, kernel):
-    """Fast mode: the two-tile kernel (NFB_TRAIN_KERNEL=v6) and the pipelined kernel (v7, the default training forward where its
-    shared-memory budget covers the sample counts) also have training (SAVE) variants; the one-tile kernel's SAVE variant
-    (NFB_TRAIN_KERNEL=v4) is the reference here.  Both accumulate every output element over the same K sequence, so
-    outputs and the saved state (activation images, masks, encodings, colours, depths) must agree bit for bit, and the
-    gradients computed from them to summation order (atomics)."""
-    import nerf
-    from nerf import _engine
-    dev = torch.device("cuda", 0)
-    n, nc, nf = 37, 64, 128
-    fr = O.synthetic_frame(9, 6, 8)
-    ro, rd = O.ray_bundle(6, 8, fr["intrinsics"], fr["pose"])
-    ro, rd = ro.reshape(-1, 3)[:n].contiguous().to(dev), rd.reshape(-1, 3)[:n].contiguous().to(dev)
-    bg = fr["bg"].reshape(-1, 3)[:n].contiguous().to(dev)
-    s = O.Sampling(nc, nf, True, 0.1, False, 2048)
-    noise = O.draw_noise(n, s, torch.Generator().manual_seed(3))
-    nz = dict(t_rand=noise.t_rand.to(dev), n_c=noise.n_c.to(dev), u=noise.u.to(dev), n_f=noise.n_f.to(dev))
-    models = []
-    for seed in (100, 101):
-        m = nerf.models.ConditionalBlendshapePaperNeRFModel(num_encoding_fn_xyz=10, num_encoding_fn_dir=4,
-                                                            include_input_xyz=True, include_input_dir=False)
-        m.load_state_dict(O.random_init_params(seed, True))
-        models.append(m.to(dev))
-    mc, mf = models
-    expr, latent = fr["expr"].to(dev), fr["latent"].to(dev)
-    gouts = [torch.randn(n, 3, generator=torch.Generator().manual_seed(11)).to(dev), None, None,
-             torch.randn(n, 3, generator=torch.Generator().manual_seed(12)).to(dev), None, None, None]
-    params_c = [dict(mc.named_parameters())[k] for k in TR.PARAM_ORDER]
-    params_f = [dict(mf.named_parameters())[k] for k in TR.PARAM_ORDER]
-
-    def run(engine):
-        engine.sync_weights(mc, mf)
-        engine.set_frame(expr, latent)
-        out = engine.render(ro, rd, 0.2, 0.8, nc, nf, perturb=True, noise_std=0.1, background=bg, noise=nz, precision="fast", train=True)
-        torch.cuda.synchronize()
-        d = engine.train_debug()
-        nt = int(d.n_tiles)
-        rec = dev_tensor(d.records, (nt, d.record_bytes // 2), "<i2").clone()
-        state = dict(z_c=dev_tensor(d.z_coarse, (n, nc)).clone(), z_f=dev_tensor(d.z_fine, (n, nc + nf)).clone(),
-                     raw_c=dev_tensor(d.raw_coarse, (n, nc, 4)).clone(), raw_f=dev_tensor(d.raw_fine, (n, nc + nf, 4)).clone())
-        grads = engine.backward(gouts, params_c, params_f)
-        torch.cuda.synchronize()
-        return out, rec, state, grads
-
-    monkeypatch.setenv("NFB_TRAIN_KERNEL", kernel)
-    out2, rec2, st2, g2 = run(_engine.Renderer(dev))                 # two-tile / pipelined training forward
-    monkeypatch.setenv("NFB_TRAIN_KERNEL", "v4")
-    out1, rec1, st1, g1 = run(_engine.Renderer(dev))                 # one-tile training forward
-    for k in ("rgb_coarse", "disp_coarse", "acc_coarse", "rgb_fine", "disp_fine", "acc_fine", "w_last"):
-        assert torch.equal(out1[k], out2[k]), k
-    for k in st1:
-        assert torch.equal(st1[k], st2[k]), k
-    x_side = REC["mask"] // 2                                        # halfwords: encodings + activation images
-    assert torch.equal(rec1[:, :x_side], rec2[:, :x_side])
-    m1 = rec1.view(torch.uint8).reshape(rec1.shape[0], -1)[:, REC["mask"]:REC["mask"] + 9 * 128 * 32].view(torch.int32).reshape(-1, 9, 128, 8)
-    m2 = rec2.view(torch.uint8).reshape(rec2.shape[0], -1)[:, REC["mask"]:REC["mask"] + 9 * 128 * 32].view(torch.int32).reshape(-1, 9, 128, 8)
-    assert torch.equal(m1[:, :6], m2[:, :6]) and torch.equal(m1[:, 6:, :, :4], m2[:, 6:, :, :4])   # 128-wide layers: 4 words
-    for a, b in zip(g1[0] + g1[1] + [g1[2]], g2[0] + g2[1] + [g2[2]]):
-        if a is None:
-            assert b is None
-            continue
-        assert float((a - b).abs().max()) <= 1e-5 * float(a.abs().max()) + 1e-12

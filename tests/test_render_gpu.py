@@ -146,6 +146,42 @@ def test_sample_counts_against_oracle(env, precision, nc, nf):
         assert err < 1e-4, (name, err)
 
 
+def test_fast_kernels_agree_bit_for_bit(env, monkeypatch):
+    """Fast mode: the one-tile kernel (NFB_KERNEL=v4; evaluation and training forward), the two-tile kernel (v6) and the
+    pipelined kernel (v7) accumulate every output element over the same K sequence with the same per-sample arithmetic, so
+    all seven outputs agree bit for bit.  100c+60f is outside the pipelined kernel's shared-memory budget (it falls back to
+    v6), so only v4 and v6 are compared there; 128c+256f has two coarse tiles and one ray per stream."""
+    nerf, _engine, dev = env
+    engines = {}
+    for k in ("v4", "v6", "v7"):
+        monkeypatch.setenv("NFB_KERNEL", k)
+        engines[k] = _engine.Renderer(dev)
+    mc, mf = make_model(nerf, O.random_init_params(100, True), dev), make_model(nerf, O.random_init_params(101, True), dev)
+    cases = [(37, 64, 128, ("v6", "v7", "train")), (13, 100, 60, ("v6",)), (13, 128, 256, ("v6", "v7"))]
+    for n, nc, nf, others in cases:
+        fr = O.synthetic_frame(9, 6, 8)
+        ro, rd = O.ray_bundle(6, 8, fr["intrinsics"], fr["pose"])
+        ro, rd = ro.reshape(-1, 3)[:n].contiguous().to(dev), rd.reshape(-1, 3)[:n].contiguous().to(dev)
+        bg = fr["bg"].reshape(-1, 3)[:n].contiguous().to(dev)
+        noise = O.draw_noise(n, O.Sampling(nc, nf, True, 0.1, False, 2048), torch.Generator().manual_seed(3))
+        nz = dict(t_rand=noise.t_rand.to(dev), n_c=noise.n_c.to(dev), u=noise.u.to(dev), n_f=noise.n_f.to(dev))
+
+        def run(kernel):
+            eng = engines["v4" if kernel == "train" else kernel]
+            eng.sync_weights(mc, mf)
+            eng.set_frame(fr["expr"].to(dev), fr["latent"].to(dev))
+            out = eng.render(ro, rd, 0.2, 0.8, nc, nf, perturb=True, noise_std=0.1, background=bg, noise=nz, precision="fast",
+                             train=kernel == "train")
+            torch.cuda.synchronize()
+            return out
+
+        ref = run("v4")
+        for kernel in others:
+            out = run(kernel)
+            for name in NAMES:
+                assert torch.equal(ref[name], out[name]), (n, nc, nf, kernel, name)
+
+
 def test_in_kernel_ray_generation_matches_explicit_rays(env):
     nerf, _engine, dev = env
     H, W = 16, 24
