@@ -46,7 +46,7 @@ struct NfbHandle {
   size_t bg_cap = 0, out_cap = 0;
   // training state: what nfb_render_forward_train saved for nfb_render_backward (grow-only buffers)
   struct Train {
-    uint8_t* rec = nullptr; size_t rec_tiles = 0;       // per-tile activation records (nfb_layout.h kRec*)
+    uint8_t* rec = nullptr; size_t rec_tiles = 0;       // per-tile activation records (nfb_layout.h kRec*), rec_tiles = bytes
     float* draw = nullptr; size_t draw_tiles = 0;       // [tiles][128][4]
     float *z_c = nullptr, *raw_c = nullptr, *z_f = nullptr, *raw_f = nullptr, *dnorm = nullptr;
     size_t cap_zc = 0, cap_rawc = 0, cap_zf = 0, cap_rawf = 0, cap_dn = 0;
@@ -55,6 +55,7 @@ struct NfbHandle {
     float* cond = nullptr;                              // [108] conditioning vector of the frame the forward rendered
     int n_rays = 0, nc = 0, nf = 0, rays_per_unit = 0, tiles_c = 0, tiles_f = 0, n_units = 0, has_bg = 0, white_bkgd = 0;
     bool valid = false;
+    bool exact_grad = false;     // NFB_PREC_EXACT_GRAD: 2 MiB hi+lo records, exact chain and weight-gradient kernels
     // chunked mode (the records of the whole call would exceed the memory budget): the forward only produced the outputs; the
     // backward re-runs the training forward chunk by chunk from the saved launch parameters (the caller keeps the inputs alive)
     bool chunked = false;
@@ -125,6 +126,7 @@ static int create_impl(NfbHandle* h, const cudaDeviceProp& prop) {
     NFB_CUDA(dev_alloc(&nb.w3c, 256 * nfb::kDimCond));
     NFB_CUDA(dev_alloc(&nb.wd0b_t, nfb::kDimDir * 128));
     NFB_CUDA(dev_alloc(&nb.stream_bwd, nfb::kBwdStreamBytes));
+    NFB_CUDA(dev_alloc(&nb.stream_bwd_x3, nfb::kBwdStreamBytesX3));
     NFB_CUDA(dev_alloc(&h->tr.acc[n], nfb::kAccFloats));
   }
   NFB_CUDA(dev_alloc(&h->tr.scal, 4));
@@ -173,6 +175,7 @@ int nfb_destroy(NfbHandle* h) {
     nfb::NetBuffers& nb = h->net[n];
     cudaFree(nb.stream_x1); cudaFree(nb.stream_x3); cudaFree(nb.w6); cudaFree(nb.b6); cudaFree(nb.bias_static);
     cudaFree(nb.bias_frame); cudaFree(nb.w0c); cudaFree(nb.w3c); cudaFree(nb.wd0b_t); cudaFree(nb.stream_bwd);
+    cudaFree(nb.stream_bwd_x3);
     cudaFree(h->tr.acc[n]);
   }
   cudaFree(h->tr.rec); cudaFree(h->tr.draw); cudaFree(h->tr.z_c); cudaFree(h->tr.raw_c); cudaFree(h->tr.z_f); cudaFree(h->tr.raw_f);
@@ -283,10 +286,10 @@ static size_t train_budget(NfbHandle* h) {
   return h->train_budget = budget;
 }
 
-// (Re)size the buffers a training launch over n rays / `tiles` tiles writes.
+// (Re)size the buffers a training launch over n rays / `tiles` tiles writes (records of tr.exact_grad's size).
 static int ensure_train_buffers(NfbHandle::Train& tr, size_t n, size_t tiles, int nc, int nf) {
   int rc;
-  if ((rc = ensure_cap(&tr.rec, &tr.rec_tiles, tiles * nfb::kRecBytes))) return rc;
+  if ((rc = ensure_cap(&tr.rec, &tr.rec_tiles, tiles * (size_t)nfb::rec_stride(tr.exact_grad)))) return rc;
   if ((rc = ensure_cap(&tr.draw, &tr.draw_tiles, tiles * 512))) return rc;
   if ((rc = ensure_cap(&tr.z_c, &tr.cap_zc, n * nc))) return rc;
   if ((rc = ensure_cap(&tr.raw_c, &tr.cap_rawc, n * nc * 4))) return rc;
@@ -307,7 +310,7 @@ static int render_impl(NfbHandle* h, const NfbRays* rays, const NfbSampling* sm,
   const int nc = sm->num_coarse, nf = sm->num_fine;
   if (nc < 3 || nf < 0 || nc + nf > 512) return NFB_ERR_UNSUPPORTED;
   if (sm->lindisp) return NFB_ERR_UNSUPPORTED;
-  if (sm->precision != NFB_PREC_FAST && sm->precision != NFB_PREC_EXACT) return NFB_ERR_INVALID;
+  if (sm->precision != NFB_PREC_FAST && sm->precision != NFB_PREC_EXACT && sm->precision != NFB_PREC_EXACT_GRAD) return NFB_ERR_INVALID;
   if (!h->net[0].loaded || (nf > 0 && !h->net[1].loaded) || !h->frame_set) return NFB_ERR_STATE;
   if (!out->rgb_coarse || !out->disp_coarse || !out->acc_coarse) return NFB_ERR_INVALID;
   if (nf > 0 && (!out->rgb_fine || !out->disp_fine || !out->acc_fine)) return NFB_ERR_INVALID;
@@ -352,7 +355,7 @@ static int render_impl(NfbHandle* h, const NfbRays* rays, const NfbSampling* sm,
     }
   }
   if (noise) { p.t_rand = noise->t_rand; p.noise_c = noise->sigma_noise_c; p.u_rand = noise->u; p.noise_f = noise->sigma_noise_f; }
-  const bool exact = sm->precision == NFB_PREC_EXACT;
+  const bool exact = sm->precision != NFB_PREC_FAST;  // NFB_PREC_EXACT_GRAD renders with the exact kernels too
   for (int n = 0; n < 2; ++n) {
     p.wstream[n] = exact ? h->net[n].stream_x3 : h->net[n].stream_x1;
     p.bias[n] = h->net[n].bias_frame;
@@ -369,19 +372,21 @@ static int render_impl(NfbHandle* h, const NfbRays* rays, const NfbSampling* sm,
     // Saved for nfb_render_backward: per-tile activation records, sample depths, (colour, ReLU input of sigma), |d|.
     NfbHandle::Train& tr = h->tr;
     tr.valid = false;
+    tr.exact_grad = sm->precision == NFB_PREC_EXACT_GRAD;
+    const size_t rec_bytes = (size_t)nfb::rec_stride(tr.exact_grad);
     const size_t n = (size_t)rays->n_rays, tiles_per_unit = (size_t)(p.tiles_c + p.tiles_f), tiles = (size_t)p.n_units * tiles_per_unit;
     int rc;
-    tr.chunked = tiles * nfb::kRecBytes > train_budget(h);
+    tr.chunked = tiles * rec_bytes > train_budget(h);
     if (tr.chunked) {
       // e.g. a whole frame rendered with gradients enabled: 1.5-2 MiB of records per ray.  Keep the launch parameters, produce
       // the outputs with the evaluation kernel now, and let the backward re-run the training forward in chunks that fit.
       if (!rays->o) { g_last_cuda_error = "training forward over budget needs explicit rays (o, d)"; return NFB_ERR_UNSUPPORTED; }
-      size_t units = train_budget(h) / nfb::kRecBytes / tiles_per_unit;
+      size_t units = train_budget(h) / rec_bytes / tiles_per_unit;
       units &= ~(size_t)1;  // whole two-tile units of work
       if (units < 2) units = 2;
       tr.chunk_rays = (int)(units * p.rays_per_unit);
       tr.full = p;
-      tr.precision = exact ? 1 : 0;
+      tr.precision = tr.exact_grad ? 2 : (exact ? 1 : 0);
     } else if ((rc = ensure_train_buffers(tr, n, tiles, nc, nf))) return rc;
     // a later nfb_set_frame (e.g. a validation render before the backward) must not change what the backward differentiates
     NFB_CUDA(cudaMemcpyAsync(tr.cond, h->cond, nfb::kDimCond * sizeof(float), cudaMemcpyDeviceToDevice, st));
@@ -399,7 +404,7 @@ static int render_impl(NfbHandle* h, const NfbRays* rays, const NfbSampling* sm,
   const bool pipelined = two_tile && h->use_render3 && nfb::render3_supports(p);
   if (pipelined) NFB_CUDA(nfb::launch_render3(p, h->num_sms, st, &h->launches));
   else if (two_tile) NFB_CUDA(nfb::launch_render2(p, h->num_sms, st, &h->launches));
-  else NFB_CUDA(nfb::launch_render(p, exact ? 1 : 0, h->num_sms, st, &h->launches));
+  else NFB_CUDA(nfb::launch_render(p, (saving && h->tr.exact_grad) ? 2 : (exact ? 1 : 0), h->num_sms, st, &h->launches));
   if (train) h->tr.valid = true;
   return NFB_OK;
 }
@@ -454,16 +459,17 @@ int nfb_render_backward(NfbHandle* h, const NfbOutGrads* og, const float* const 
     nfb::ChainParams c;
     c.n_units = n_units; c.tiles_c = tr.tiles_c; c.tiles_f = tr.tiles_f;
     c.rec = tr.rec; c.draw = tr.draw; c.scal = tr.scal;
-    c.wstream[0] = h->net[0].stream_bwd;
-    c.wstream[1] = fine ? h->net[1].stream_bwd : h->net[0].stream_bwd;
-    NFB_CUDA(nfb::launch_chain(c, h->num_sms, st, &h->launches));
+    const int fn = fine ? 1 : 0;
+    c.wstream[0] = tr.exact_grad ? h->net[0].stream_bwd_x3 : h->net[0].stream_bwd;
+    c.wstream[1] = tr.exact_grad ? h->net[fn].stream_bwd_x3 : h->net[fn].stream_bwd;
+    NFB_CUDA(nfb::launch_chain(c, tr.exact_grad, h->num_sms, st, &h->launches));
     {
       nfb::DwParams d = {};
       d.rec = tr.rec; d.n_units = n_units; d.tpu = tr.tiles_c + tr.tiles_f;
       d.t_base[0] = 0; d.t_cnt[0] = tr.tiles_c;
       d.t_base[1] = tr.tiles_c; d.t_cnt[1] = fine ? tr.tiles_f : 0;
       d.acc[0] = tr.acc[0]; d.acc[1] = tr.acc[1]; d.scal = tr.scal;
-      NFB_CUDA(nfb::launch_dw(d, h->num_sms, st, &h->launches));  // both networks in one launch
+      NFB_CUDA(nfb::launch_dw(d, tr.exact_grad, h->num_sms, st, &h->launches));  // both networks in one launch
     }
     return NFB_OK;
   };
@@ -515,7 +521,7 @@ int nfb_train_debug(NfbHandle* h, NfbTrainDebug* out) {
   if (!h || !out) return NFB_ERR_INVALID;
   if (!h->tr.valid || h->tr.chunked) return NFB_ERR_STATE;  // chunked: the buffers only ever hold one chunk
   const NfbHandle::Train& tr = h->tr;
-  out->records = tr.rec; out->n_tiles = (long long)tr.n_units * (tr.tiles_c + tr.tiles_f); out->record_bytes = nfb::kRecBytes;
+  out->records = tr.rec; out->n_tiles = (long long)tr.n_units * (tr.tiles_c + tr.tiles_f); out->record_bytes = (int32_t)nfb::rec_stride(tr.exact_grad);
   out->d_raw = tr.draw; out->acc_coarse = tr.acc[0]; out->acc_fine = tr.acc[1]; out->acc_floats = nfb::kAccFloats;
   out->scale = tr.scal; out->z_coarse = tr.z_c; out->raw_coarse = tr.raw_c; out->z_fine = tr.z_f; out->raw_fine = tr.raw_f;
   out->tiles_coarse = tr.tiles_c; out->tiles_fine = tr.tiles_f; out->rays_per_unit = tr.rays_per_unit;
@@ -646,6 +652,8 @@ int nfb_debug_schedule(int which, int index, uint32_t* out, int out_words) {
     case 2: return nfb::debug_prog_chain(index, out);
     case 3: return nfb::debug_jobs_dw(index, out);
     case 4: return index < 0 ? 1 : nfb::debug_dw_split(out);  // in/out: {num_sms, tiles 0, tiles 1} -> {parts0, parts1, groups}
+    case 5: return nfb::debug_prog_chain_exact(index, out);
+    case 6: return nfb::debug_stages_dw_exact(index, out);
     default:
       if (which >= 1000) {  // 1000 + n_iter * 100 + Tc * 10 + Tf: the pipelined kernel's job sequence
         const int w = which - 1000;

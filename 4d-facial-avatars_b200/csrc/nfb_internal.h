@@ -20,6 +20,7 @@ struct NetBuffers {
   float* w3c = nullptr;          // [256,108] conditioning columns of layers_xyz.3
   float* wd0b_t = nullptr;       // [24,128] direction columns of layers_dir.0, transposed
   uint8_t* stream_bwd = nullptr; // kBwdStreamBytes: transposed FP16 weights for the backward chain (nfb_train.cu)
+  uint8_t* stream_bwd_x3 = nullptr;  // kBwdStreamBytesX3: the same as hi unit, lo unit, ... (exact-gradient chain)
   bool loaded = false;
 };
 
@@ -77,7 +78,7 @@ struct ChainParams {
   uint8_t* rec;
   const float* draw;
   const float* scal;            // [0] = loss scale, [1] = 1 / scale
-  const uint8_t* wstream[2];    // backward weight streams (coarse, fine)
+  const uint8_t* wstream[2];    // backward weight streams (coarse, fine): stream_bwd, or stream_bwd_x3 for the exact-gradient chain
 };
 struct DwParams {  // ONE launch covers both networks: the first parts[0] * groups CTAs work on network 0, the rest on network 1
   const uint8_t* rec;
@@ -93,11 +94,14 @@ int debug_prog_v6(int index, uint32_t* out);
 int debug_jobs_v7(int n_iter, int tc, int tf, int index, uint32_t* out);
 int debug_prog_chain(int index, uint32_t* out);
 int debug_jobs_dw(int index, uint32_t* out);
+int debug_prog_chain_exact(int index, uint32_t* out);
+int debug_stages_dw_exact(int index, uint32_t* out);
 int debug_dw_split(uint32_t* io);  // io: {num_sms, tiles net 0, tiles net 1} -> {parts0, parts1, groups}
 cudaError_t train_kernels_setup();
 cudaError_t launch_composite_bwd(const CompBwdParams& q, float* scal, cudaStream_t st, long long* launches);
-cudaError_t launch_chain(const ChainParams& p, int num_sms, cudaStream_t st, long long* launches);
-cudaError_t launch_dw(const DwParams& p, int num_sms, cudaStream_t st, long long* launches);
+// exact_grad: the variants that read / write 2 MiB hi+lo records (after an NFB_PREC_EXACT_GRAD training forward)
+cudaError_t launch_chain(const ChainParams& p, bool exact_grad, int num_sms, cudaStream_t st, long long* launches);
+cudaError_t launch_dw(const DwParams& p, bool exact_grad, int num_sms, cudaStream_t st, long long* launches);
 cudaError_t launch_finalize_all(const float* const params_c[26], float* const grads_c[26], const float* acc_c,
                                 const float* const params_f[26], float* const grads_f[26], const float* acc_f, const float* cond,
                                 float* latent_out, cudaStream_t st, long long* launches);
@@ -114,7 +118,8 @@ cudaError_t launch_loss_grad(const float* rgb_c, const float* rgb_f, const float
 cudaError_t launch_adam_dev(float* p, float* g, float* m, float* v, long long n, void* dev_state, cudaStream_t st, long long* launches);
 cudaError_t launch_adam(float* p, float* g, float* m, float* v, long long n, float lr, float b1, float b2, float eps, int step,
                         float grad_scale, long long reg_off, float reg_w, cudaStream_t st, long long* launches);
-// precision: 0 = fast (x1), 1 = exact (x3).  num_sms = CTAs to launch at most.
+// precision: 0 = fast (x1), 1 = exact (x3), 2 = exact with lo records (training forward of NFB_PREC_EXACT_GRAD; evaluation as 1).
+// num_sms = CTAs to launch at most.
 cudaError_t launch_render(const RenderParams& p, int precision, int num_sms, cudaStream_t st, long long* launches);
 cudaError_t render_kernel_setup();  // opt-in to the large dynamic shared memory size
 // Two-tiles-in-flight kernel (nfb_render2.cu): fast-mode evaluation (the training forward and the layer probe run launch_render).

@@ -119,6 +119,11 @@ constexpr int kRecDY6 = kRecDY0 + 6 * 65536;      // dY6..dY8, 128 features
 constexpr int kRecDRaw = kRecDY6 + 3 * 32768;     // scaled (d rgb_raw[3], d sigma_raw) image, 16 rows (4 used)
 constexpr int kRecBytes = kRecDRaw + 4096;
 static_assert(kRecBytes == (1 << 20), "tile record is 1 MiB");
+// Exact-gradient training (NFB_PREC_EXACT_GRAD): a tile record is 2 MiB.  The first MiB is the record above, byte for byte; the
+// second holds the lo parts  lo = fp16(x - float(hi))  of every image at the same offsets (PE, h0..h5, g0..g2, PEd, dY0..dY8,
+// dRaw), so x = hi + lo to ~2^-21 relative.  The mask region of the lo MiB is unused.
+constexpr int kRecLo = 1 << 20;
+NFB_HD constexpr long long rec_stride(bool exact_grad) { return exact_grad ? 2LL * kRecBytes : (long long)kRecBytes; }
 NFB_HD constexpr int rec_x_off(int layer) { return layer < 6 ? kRecH0 + layer * 65536 : kRecG0 + (layer - 6) * 32768; }
 NFB_HD constexpr int rec_dy_off(int layer) { return layer < 6 ? kRecDY0 + layer * 65536 : kRecDY6 + (layer - 6) * 32768; }
 NFB_HD constexpr int rec_width(int layer) { return layer < 6 ? 256 : 128; }
@@ -147,6 +152,7 @@ NFB_HD constexpr int bwd_step_offset(int s) {
   return off;
 }
 constexpr int kBwdStreamBytes = bwd_step_offset(kBwdSteps);  // 835584
+constexpr int kBwdStreamBytesX3 = 2 * kBwdStreamBytes;       // exact-gradient chain: per unit the hi image, then the lo image
 
 // Weight-gradient accumulators of one network (FP32, float offsets), in the kernel's folded parametrisation.
 constexpr int kAcc0 = 0;                       // [256][64]   d W0[:, PE lanes]

@@ -1,7 +1,7 @@
 // nfb_pack.cu — load-time, per-optimizer-step and per-frame preparation kernels (not on the per-ray hot path):
 //   * fold_feat_kernel : fc_feat pre-multiplied into fc_alpha and layers_dir.0[:, :256] (FP64 accumulate), both networks
 //   * repack_kernel    : ONE launch per weight update, both networks: FP32 weights -> FP16 hi/lo as the swizzled shared-memory images the
-//                        render kernels bulk-copy (forward streams) and the transposed stream of the backward chain, static
+//                        render kernels bulk-copy (forward streams) and the transposed streams of the backward chain (FP16 and hi/lo), static
 //                        biases, conditioning columns, transposed direction columns
 //   * frame_fold_kernel: per-frame expression/latent fold into the layer-0 / layer-3 biases
 // Reference semantics: nerf/models.py:236-261 (forward), :218-233 (parameter shapes).
@@ -117,8 +117,10 @@ __device__ __forceinline__ void gather_elem(const NetParams& g, int t, float* __
   }
 }
 
-// Backward (transposed) stream: one thread per 16-byte chunk (8 consecutive k) of row n of unit (s, u); element (n, k) = W^T.
-__device__ __forceinline__ void pack_bwd_chunk(const NetParams& a, int s, int u, int idx, uint8_t* __restrict__ dst) {
+// Backward (transposed) streams: one thread per 16-byte chunk (8 consecutive k) of row n of unit (s, u); element (n, k) = W^T.
+// dst: FP16 of W^T; dst_x3: hi then lo per unit (the split of the FP32 value, after the FP64 fold for M1 / m2).
+__device__ __forceinline__ void pack_bwd_chunk(const NetParams& a, int s, int u, int idx, uint8_t* __restrict__ dst,
+                                               uint8_t* __restrict__ dst_x3) {
   const StepInfo si = bwd_step_info(s);
   if (u >= si.k_atoms) return;
   const int rows = si.nh0 + si.nh1;
@@ -127,6 +129,7 @@ __device__ __forceinline__ void pack_bwd_chunk(const NetParams& a, int s, int u,
   const bool op_atom = si.pe_first && u == 0;
   const int hid = u - si.pe_first;  // TMEM atom index
   __align__(16) __half h[8];
+  __align__(16) __half lo[8];
 #pragma unroll
   for (int e = 0; e < 8; ++e) {
     const int kl = c16 * 8 + e;        // k inside the atom
@@ -145,9 +148,13 @@ __device__ __forceinline__ void pack_bwd_chunk(const NetParams& a, int s, int u,
       default: w = a.p[2][kk * 256 + n]; break;                                    // layers_xyz.1
     }
     h[e] = __float2half_rn(w);
+    lo[e] = __float2half_rn(w - __half2float(h[e]));
   }
   const int off = bwd_step_offset(s) + u * rows * 128;
-  *reinterpret_cast<uint4*>(dst + off + n * 128 + ((c16 ^ (n & 7)) << 4)) = *reinterpret_cast<const uint4*>(h);
+  const int inner = n * 128 + ((c16 ^ (n & 7)) << 4);
+  *reinterpret_cast<uint4*>(dst + off + inner) = *reinterpret_cast<const uint4*>(h);
+  *reinterpret_cast<uint4*>(dst_x3 + 2 * off + inner) = *reinterpret_cast<const uint4*>(h);
+  *reinterpret_cast<uint4*>(dst_x3 + 2 * off + rows * 128 + inner) = *reinterpret_cast<const uint4*>(lo);
 }
 
 // Launch 2 re-packs up to two networks: FP32 parameters (+ the fold) -> forward streams (x1, hi/lo x3), transposed backward
@@ -160,7 +167,7 @@ constexpr int kGatherBlocks = (256 * kDimCond + 255) / 256;  // 108
 constexpr int kRepackBlocks = kFwdBlocks + kBwdBlocks + kGatherBlocks;
 struct RepackArgs {
   NetParams net[2];
-  uint8_t *x1[2], *x3[2], *bwd[2];
+  uint8_t *x1[2], *x3[2], *bwd[2], *bwd_x3[2];
   float *bias_static[2], *w0c[2], *w3c[2], *wd0b_t[2];
 };
 __global__ void __launch_bounds__(256) repack_kernel(const RepackArgs a) {
@@ -175,7 +182,7 @@ __global__ void __launch_bounds__(256) repack_kernel(const RepackArgs a) {
   b -= kFwdBlocks;
   if (b < kBwdBlocks) {
     const int s = b / (8 * kMaxBwdUnits), r = b % (8 * kMaxBwdUnits);
-    pack_bwd_chunk(np, s, r / 8, (r % 8) * 256 + threadIdx.x, a.bwd[net]);
+    pack_bwd_chunk(np, s, r / 8, (r % 8) * 256 + threadIdx.x, a.bwd[net], a.bwd_x3[net]);
     return;
   }
   b -= kBwdBlocks;
@@ -239,7 +246,7 @@ cudaError_t launch_repack(NetBuffers* const nb[2], const float* const* const par
     f.net[n].w6 = f.net[n].b6 = nullptr;
     f.w6[n] = nb[n]->w6; f.b6[n] = nb[n]->b6;
     a.net[n].w6 = nb[n]->w6; a.net[n].b6 = nb[n]->b6;
-    a.x1[n] = nb[n]->stream_x1; a.x3[n] = nb[n]->stream_x3; a.bwd[n] = nb[n]->stream_bwd;
+    a.x1[n] = nb[n]->stream_x1; a.x3[n] = nb[n]->stream_x3; a.bwd[n] = nb[n]->stream_bwd; a.bwd_x3[n] = nb[n]->stream_bwd_x3;
     a.bias_static[n] = nb[n]->bias_static; a.w0c[n] = nb[n]->w0c; a.w3c[n] = nb[n]->w3c; a.wd0b_t[n] = nb[n]->wd0b_t;
   }
   fold_feat_kernel<<<dim3(144, 4, n_nets), 256, 0, st>>>(f);

@@ -169,8 +169,13 @@ __device__ __forceinline__ void epi_half(uint32_t t_slice, uint32_t bias, uint32
 }
 
 // ------------------------------------------------------------------------------------------------
-template <bool EXACT, bool SAVE>
+// LO (the exact-gradient training forward, EXACT and SAVE only): the records are 2 MiB and the lo parts of every image go to the
+// second MiB (nfb_layout.h kRecLo) — the savers read the lo columns (+32 of each slice) too, the row warps write the lo PE and PEd
+// images.
+template <bool EXACT, bool SAVE, bool LO = false>
 __global__ void __launch_bounds__(SAVE ? kThreadsSave : kThreads, 1) render_kernel(const __grid_constant__ RenderParams p) {
+  static_assert(!LO || (EXACT && SAVE), "lo records need the exact training forward");
+  constexpr long long kRecStride = rec_stride(LO);
   // Use the dynamic shared array directly (no integer round trip) so the compiler keeps the shared address
   // space and emits LDS/STS instead of generic loads; the swizzled operands need 1024-byte alignment.
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -420,11 +425,19 @@ __global__ void __launch_bounds__(SAVE ? kThreadsSave : kThreads, 1) render_kern
           }
           if constexpr (SAVE) {  // FP16 encoding of this tile as a transposed image (input of layers_xyz.0 / .3 in dW)
             if (unit < p.n_units) {
-              uint8_t* rec = p.save_rec + (size_t)(unit * tiles_per_unit + (pass ? p.tiles_c : 0) + t) * kRecBytes;
+              uint8_t* rec = p.save_rec + (size_t)(unit * tiles_per_unit + (pass ? p.tiles_c : 0) + t) * kRecStride;
               uint32_t hh[16];
 #pragma unroll
               for (int e = 0; e < 16; ++e) hh[e] = pack_f16x2(f[2 * e], f[2 * e + 1]);
               store_t32(rec + kRecPE + img_row_base(64, row), row, 32 * ch, hh);
+              if constexpr (LO) {  // the remainder, rounded as store_pe_row rounds the lo operand of the forward
+#pragma unroll
+                for (int e = 0; e < 16; ++e) {
+                  const float2 h = unpack_f16x2(hh[e]);
+                  hh[e] = pack_f16x2(f[2 * e] - h.x, f[2 * e + 1] - h.y);
+                }
+                store_t32(rec + kRecLo + kRecPE + img_row_base(64, row), row, 32 * ch, hh);
+              }
             }
           }
           fence_proxy_async_smem();  // make the generic-proxy PE stores visible to the tensor core
@@ -443,7 +456,7 @@ __global__ void __launch_bounds__(SAVE ? kThreadsSave : kThreads, 1) render_kern
           uint8_t* rec = nullptr;  // this tile's training record (SAVE mode, real units only)
           if constexpr (SAVE) {
             if (unit < p.n_units) {
-              rec = p.save_rec + (size_t)(unit * tiles_per_unit + (pass ? p.tiles_c : 0) + t) * kRecBytes;
+              rec = p.save_rec + (size_t)(unit * tiles_per_unit + (pass ? p.tiles_c : 0) + t) * kRecStride;
               uint32_t hh[16];  // direction encoding of this row's ray: features [16*ch, 16*ch+16) -> two 8-feature halves
 #pragma unroll
               for (int e = 0; e < 8; ++e) {
@@ -462,6 +475,18 @@ __global__ void __launch_bounds__(SAVE ? kThreadsSave : kThreads, 1) render_kern
                 const int ka = 16 * ch + 2 * e, kb = ka + 1;
                 *reinterpret_cast<uint16_t*>(img + ka * 128 + ((cr ^ (uint32_t)(ka & 7)) << 4)) = (uint16_t)(hh[e] & 0xFFFFu);
                 *reinterpret_cast<uint16_t*>(img + kb * 128 + ((cr ^ (uint32_t)(kb & 7)) << 4)) = (uint16_t)(hh[e] >> 16);
+              }
+              if constexpr (LO) {
+#pragma unroll
+                for (int e = 0; e < 8; ++e) {
+                  const int ka = 16 * ch + 2 * e, kb = ka + 1;
+                  const float a = (live && rp.valid && ka < kDimDir) ? rp.ped[ka] : 0.f;
+                  const float b = (live && rp.valid && kb < kDimDir) ? rp.ped[kb] : 0.f;
+                  const float2 h = unpack_f16x2(hh[e]);
+                  const uint32_t l = pack_f16x2(a - h.x, b - h.y);
+                  *reinterpret_cast<uint16_t*>(img + kRecLo + ka * 128 + ((cr ^ (uint32_t)(ka & 7)) << 4)) = (uint16_t)(l & 0xFFFFu);
+                  *reinterpret_cast<uint16_t*>(img + kRecLo + kb * 128 + ((cr ^ (uint32_t)(kb & 7)) << 4)) = (uint16_t)(l >> 16);
+                }
               }
             }
           }
@@ -653,7 +678,7 @@ __global__ void __launch_bounds__(SAVE ? kThreadsSave : kThreads, 1) render_kern
         if (pass == 1 && p.nf == 0) break;
         const int n_tiles = pass ? p.tiles_f : p.tiles_c;
         for (int t = 0; t < n_tiles; ++t) {
-          uint8_t* rec = (unit < p.n_units) ? p.save_rec + (size_t)(unit * tiles_per_unit + (pass ? p.tiles_c : 0) + t) * kRecBytes : nullptr;
+          uint8_t* rec = (unit < p.n_units) ? p.save_rec + (size_t)(unit * tiles_per_unit + (pass ? p.tiles_c : 0) + t) * kRecStride : nullptr;
 #pragma unroll 1
           for (int s = 0; s <= 8; ++s) {
             const uint32_t par = (uint32_t)(s & 1);
@@ -669,20 +694,25 @@ __global__ void __launch_bounds__(SAVE ? kThreadsSave : kThreads, 1) render_kern
                 sv_ph ^= bit;
                 tc_fence_after_sync();
               }
-              uint32_t v[32];
-              tmem_ld32(t_reg + 64 * i, v);
-              tmem_wait_ld();
-              if (i == n_slices - 1) {  // the whole region has been read: the MMA warp may overwrite it
-                tc_fence_before_sync();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(bar_saved + par * 8);
-              }
-              if (img) {
-                uint32_t h0[16], h1[16];
+              // LO: two passes per slice (hi columns, then lo columns at +32), so the savers stay at 80 registers
 #pragma unroll
-                for (int j = 0; j < 16; ++j) { h0[j] = v[j]; h1[j] = v[16 + j]; }
-                store_t32(img, row, 64 * i, h0);
-                store_t32(img, row, 64 * i + 32, h1);
+              for (int part = 0; part < (LO ? 2 : 1); ++part) {
+                uint32_t v[32];
+                tmem_ld32(t_reg + 64 * i + 32 * part, v);
+                tmem_wait_ld();
+                if (i == n_slices - 1 && part == (LO ? 1 : 0)) {  // the whole region has been read: the MMA warp may overwrite it
+                  tc_fence_before_sync();
+                  __syncwarp();
+                  if (lane == 0) mbar_arrive(bar_saved + par * 8);
+                }
+                if (img) {
+                  uint8_t* dst = img + part * kRecLo;
+                  uint32_t h0[16], h1[16];
+#pragma unroll
+                  for (int j = 0; j < 16; ++j) { h0[j] = v[j]; h1[j] = v[16 + j]; }
+                  store_t32(dst, row, 64 * i, h0);
+                  store_t32(dst, row, 64 * i + 32, h1);
+                }
               }
             }
           }
@@ -717,15 +747,18 @@ cudaError_t render_kernel_setup() {
   if (e != cudaSuccess) return e;
   e = cudaFuncSetAttribute(render_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
   if (e != cudaSuccess) return e;
-  return cudaFuncSetAttribute(render_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+  e = cudaFuncSetAttribute(render_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+  if (e != cudaSuccess) return e;
+  return cudaFuncSetAttribute(render_kernel<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
 }
 
 cudaError_t launch_render(const RenderParams& p, int precision, int num_sms, cudaStream_t st, long long* launches) {
-  if (p.save_rec) {  // training forward: also writes the per-tile activation records
+  if (p.save_rec) {  // training forward: also writes the per-tile activation records (2: with the lo MiB)
+    if (precision == 2) return launch_clustered(render_kernel<true, true, true>, p, kCluster, kThreadsSave, kSmemBytes, num_sms, st, launches);
     return precision == 1 ? launch_clustered(render_kernel<true, true>, p, kCluster, kThreadsSave, kSmemBytes, num_sms, st, launches)
                           : launch_clustered(render_kernel<false, true>, p, kCluster, kThreadsSave, kSmemBytes, num_sms, st, launches);
   }
-  return precision == 1 ? launch_clustered(render_kernel<true, false>, p, kCluster, kThreads, kSmemBytes, num_sms, st, launches)
+  return precision != 0 ? launch_clustered(render_kernel<true, false>, p, kCluster, kThreads, kSmemBytes, num_sms, st, launches)
                         : launch_clustered(render_kernel<false, false>, p, kCluster, kThreads, kSmemBytes, num_sms, st, launches);
 }
 

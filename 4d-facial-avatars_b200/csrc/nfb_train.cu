@@ -23,6 +23,9 @@
 //                             gradients of each network in the reference's state_dict layout, plus d latent_code.
 //
 // Gradients are carried in FP16 with one power-of-two loss scale per backward call (max |d raw| -> 2^10), FP32 accumulate.
+// After an NFB_PREC_EXACT_GRAD forward the chain and dW kernels run their EXACT variants instead: every operand is split
+// x = hi + lo in FP16 (2 MiB records, nfb_layout.h kRecLo; hi/lo weight stream stream_bwd_x3) and multiplied as
+// hi·hi + hi·lo + lo·hi, ~2^-21 relative operand error, as in the exact forward.
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
@@ -238,10 +241,16 @@ constexpr int kCluster = 2;
 constexpr int kRowThreads = 256;
 constexpr int kOffRing = 0;
 constexpr int kOffOp = kOffRing + kNumSlots * kMaxUnitBytes;  // d raw operand: [128 rows x 64 k] FP16, swizzled (k < 4 used)
-constexpr int kOffBars = kOffOp + kTileM * 128;
+// EXACT (exact-gradient chain): every weight unit is loaded as two ring entries, hi then lo (stream_bwd_x3), and the d raw operand
+// has a lo buffer right after the hi one.
+__host__ __device__ constexpr int op_buffers(bool exact) { return exact ? 2 : 1; }
+__host__ __device__ constexpr int off_bars(bool exact) { return kOffOp + op_buffers(exact) * kTileM * 128; }
 constexpr int kNumBars = 2 * kNumSlots + 4 + 6;  // + bar_sv[2 halves][2 step parities], bar_saved[2 regions]
-constexpr int kOffTmemPtr = kOffBars + kNumBars * 8;
-constexpr int kSmemBytes = kOffTmemPtr + 16;
+__host__ __device__ constexpr int off_tmem_ptr(bool exact) { return off_bars(exact) + kNumBars * 8; }
+__host__ __device__ constexpr int smem_bytes(bool exact) { return off_tmem_ptr(exact) + 16; }
+constexpr int kSmemBytes = smem_bytes(false);
+static_assert(smem_bytes(true) <= 232448, "exact chain exceeds the 227 KB per-CTA shared memory limit");
+static_assert(kMaxUnitBytes >= 256 * 128, "a hi or lo half-unit (<= 256 rows x 128 B) fills one ring slot");
 
 enum : uint32_t { kFromOp = 1u, kWait0 = 2u, kWait1 = 4u, kFirst = 8u, kCommit0 = 16u, kPostWait1 = 64u, kOddRegion = 256u };
 constexpr int total_units() {
@@ -254,7 +263,8 @@ struct ProgEntry { uint32_t x, y, z, w; };
 struct ProgTable { ProgEntry e[32]; };
 static_assert(kTileUnits <= 32, "program table too small");
 constexpr uint32_t region_col_c(int s) { return (s & 1) ? 256u : 0u; }
-constexpr ProgTable make_prog() {
+// exact: w holds the unit's offset in stream_bwd_x3 (hi image; the lo image follows it), otherwise in the FP16 stream.
+constexpr ProgTable make_prog(bool exact = false) {
   ProgTable t{};
   int i = 0;
   for (int s = 0; s < kBwdSteps; ++s) {
@@ -282,17 +292,23 @@ constexpr ProgTable make_prog() {
       t.e[i].x = umma_idesc_f16(kTileM, ui.rows);
       t.e[i].y = d_col | (a_col << 16);
       t.e[i].z = flags;
-      t.e[i].w = ((uint32_t)bwd_unit_offset(s, u) >> 4) | ((uint32_t)ui.rows << 20);
+      t.e[i].w = ((uint32_t)((exact ? 2 : 1) * bwd_unit_offset(s, u)) >> 4) | ((uint32_t)ui.rows << 20);
     }
   }
   return t;
 }
 __constant__ ProgTable c_prog = make_prog();
+// The program a chain kernel runs: c_prog, or c_chain_prog_x3 (defined after the weight-gradient job table, so that table keeps its
+// constant-bank offset).
+template <bool EXACT> __device__ __forceinline__ const ProgTable& prog();
 
 __device__ __forceinline__ uint32_t region_col(int s) { return (s & 1) ? 256u : 0u; }
 
-// One 64-column slice of the accumulator: masked gradient -> FP16 (h a: columns [0,32), h b: [32,64)).
-__device__ __forceinline__ void bwd_epi_slice(uint32_t t_slice, uint2 m, uint32_t (&ha)[16], uint32_t (&hb)[16]) {
+// One 64-column slice of the accumulator: masked gradient -> FP16 (h a: columns [0,32), h b: [32,64)); EXACT: also the lo parts
+// l a, l b (fp16(x - float(hi)), the split of the forward's epilogue).
+template <bool EXACT>
+__device__ __forceinline__ void bwd_epi_slice(uint32_t t_slice, uint2 m, uint32_t (&ha)[16], uint32_t (&hb)[16], uint32_t (&la)[16],
+                                              uint32_t (&lb)[16]) {
   uint32_t va[32], vb[32];
   tmem_ld32(t_slice, va);
   tmem_ld32(t_slice + 32, vb);
@@ -305,22 +321,33 @@ __device__ __forceinline__ void bwd_epi_slice(uint32_t t_slice, uint2 m, uint32_
     const float b1 = ((m.y >> (j + 1)) & 1u) ? __uint_as_float(vb[j + 1]) : 0.f;
     ha[j / 2] = pack_f16x2(a0, a1);
     hb[j / 2] = pack_f16x2(b0, b1);
+    if constexpr (EXACT) {
+      const float2 ga = unpack_f16x2(ha[j / 2]), gb = unpack_f16x2(hb[j / 2]);
+      la[j / 2] = pack_f16x2(a0 - ga.x, a1 - ga.y);
+      lb[j / 2] = pack_f16x2(b0 - gb.x, b1 - gb.y);
+    }
   }
 }
 
+// EXACT: the exact-gradient chain — hi/lo weight units, hi/lo d raw operand, every A operand as hi (+0) and lo (+32) of its slice,
+// hi·W_hi + lo·W_hi + hi·W_lo per K slice as in the exact forward; the savers write the dY images of both record MiBs.
+template <bool EXACT = false>
 __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const __grid_constant__ ChainParams p) {
+  constexpr int NPART = EXACT ? 2 : 1;
+  constexpr long long kRecStride = rec_stride(EXACT);
+  constexpr int kBars = off_bars(EXACT), kTmemPtr = off_tmem_ptr(EXACT);
   extern __shared__ __align__(1024) uint8_t smem[];
   const uint32_t smem_base = smem_u32(smem);
   if ((smem_base & 1023u) != 0u) __trap();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
-  const uint32_t bar_full = smem_base + kOffBars;
+  const uint32_t bar_full = smem_base + kBars;
   const uint32_t bar_empty = bar_full + kNumSlots * 8;
   const uint32_t bar_aready = bar_empty + kNumSlots * 8;  // [2]
   const uint32_t bar_accfull = bar_aready + 16;           // [2] (only [0] used: one commit per step)
   const uint32_t bar_sv = bar_accfull + 16;               // [half][step & 1]: the step's FP16 output is in TMEM -> savers
   const uint32_t bar_saved = bar_sv + 32;                 // [region]: the savers have read the region -> MMA warp
-  volatile uint32_t* tmem_ptr_s = reinterpret_cast<volatile uint32_t*>(smem + kOffTmemPtr);
+  volatile uint32_t* tmem_ptr_s = reinterpret_cast<volatile uint32_t*>(smem + kTmemPtr);
 
   if (threadIdx.x == 0) {
     for (int i = 0; i < kNumSlots; ++i) {
@@ -337,10 +364,10 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const __grid_constan
     mbar_fence_init();
   }
   if (warp == 1) {
-    tmem_alloc(smem_base + kOffTmemPtr, 512);
+    tmem_alloc(smem_base + kTmemPtr, 512);
     tmem_relinquish();
   }
-  for (int i = threadIdx.x; i < kTileM * 128 / 16; i += kThreads)  // operand chunks 1..7 of every row stay zero
+  for (int i = threadIdx.x; i < op_buffers(EXACT) * kTileM * 128 / 16; i += kThreads)  // operand chunks 1..7 of every row stay zero
     reinterpret_cast<uint4*>(smem + kOffOp)[i] = make_uint4(0u, 0u, 0u, 0u);
   tc_fence_before_sync();
   __syncthreads();
@@ -363,17 +390,20 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const __grid_constan
       const int t = j % tpu;
       const uint8_t* base = p.wstream[t < p.tiles_c ? 0 : 1];
       for (int i = 0; i < kTileUnits; ++i) {
-        const uint32_t w = c_prog.e[i].w;
+        const uint32_t w = prog<EXACT>().e[i].w;
         const uint32_t off = (w & 0xFFFFFu) << 4, bytes = (w >> 20) * 128u;
-        mbar_wait(bar_empty + slot * 8, phase ^ 1);
-        if (elect_one()) {
-          mbar_arrive_expect_tx(bar_full + slot * 8, bytes);
-          if ((seq % kCluster) == cta_rank)
-            bulk_g2s_multicast(smem_base + kOffRing + slot * kMaxUnitBytes, base + off, bytes, bar_full + slot * 8, kAllCtas);
+#pragma unroll
+        for (int part = 0; part < NPART; ++part) {  // EXACT: the hi image, then the lo image that follows it in the stream
+          mbar_wait(bar_empty + slot * 8, phase ^ 1);
+          if (elect_one()) {
+            mbar_arrive_expect_tx(bar_full + slot * 8, bytes);
+            if ((seq % kCluster) == cta_rank)
+              bulk_g2s_multicast(smem_base + kOffRing + slot * kMaxUnitBytes, base + off + part * bytes, bytes, bar_full + slot * 8, kAllCtas);
+          }
+          __syncwarp();
+          ++seq;
+          if (++slot == kNumSlots) { slot = 0; phase ^= 1; }
         }
-        __syncwarp();
-        ++seq;
-        if (++slot == kNumSlots) { slot = 0; phase ^= 1; }
       }
     }
   } else if (warp == 1) {
@@ -382,9 +412,10 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const __grid_constan
     uint32_t slot = 0, phase = 0, ph_a0 = 0, ph_a1 = 0;
     uint32_t sv_pending = 0, sv_phase = 0;  // per region bit: a step's output lives there / parity of bar_saved
     const uint64_t op_desc = umma_smem_desc_sw128(smem_base + kOffOp);
+    const uint64_t op_desc_lo = umma_smem_desc_sw128(smem_base + kOffOp + kTileM * 128);  // EXACT only
     for (int j = 0; j < n_tiles_cta; ++j) {
       for (int i = 0; i < kTileUnits; ++i) {
-        const ProgEntry e = c_prog.e[i];
+        const ProgEntry e = prog<EXACT>().e[i];
         if (e.z & kFirst) {  // first unit of a step
           const uint32_t rho = (e.z & kOddRegion) ? 1u : 0u;
           if (sv_pending & (1u << rho)) {
@@ -407,22 +438,30 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const __grid_constan
         const uint32_t d_tmem = tmem_base + (e.y & 0xFFFFu);
         const uint32_t a_tmem = tmem_base + (e.y >> 16);
         const uint32_t first = (e.z & kFirst) ? 0u : 1u;
-        mbar_wait(bar_full + slot * 8, phase);
-        tc_fence_after_sync();
-        const uint64_t b_desc = umma_smem_desc_sw128(smem_base + kOffRing + slot * kMaxUnitBytes);
-        if (elect_one()) {
 #pragma unroll
-          for (int ks = 0; ks < 4; ++ks) {
-            const uint64_t bd = b_desc + (uint64_t)(ks * 2);
-            const uint32_t acc_flag = (first | ks) ? 1u : 0u;
-            if (e.z & kFromOp) umma_ss(d_tmem, op_desc + (uint64_t)(ks * 2), bd, e.x, acc_flag);
-            else umma_ts(d_tmem, a_tmem + ks * 8, bd, e.x, acc_flag);
+        for (int part = 0; part < NPART; ++part) {  // EXACT: part 0 = W_hi (A hi and A lo), part 1 = W_lo (A hi)
+          mbar_wait(bar_full + slot * 8, phase);
+          tc_fence_after_sync();
+          const uint64_t b_desc = umma_smem_desc_sw128(smem_base + kOffRing + slot * kMaxUnitBytes);
+          if (elect_one()) {
+#pragma unroll
+            for (int ks = 0; ks < 4; ++ks) {
+              const uint64_t bd = b_desc + (uint64_t)(ks * 2);
+              const uint32_t acc_flag = (first | part | ks) ? 1u : 0u;
+              if (e.z & kFromOp) {
+                umma_ss(d_tmem, op_desc + (uint64_t)(ks * 2), bd, e.x, acc_flag);
+                if (EXACT && part == 0) umma_ss(d_tmem, op_desc_lo + (uint64_t)(ks * 2), bd, e.x, 1);
+              } else {
+                umma_ts(d_tmem, a_tmem + ks * 8, bd, e.x, acc_flag);
+                if (EXACT && part == 0) umma_ts(d_tmem, a_tmem + 32 + ks * 8, bd, e.x, 1);
+              }
+            }
+            umma_commit_multicast(bar_empty + slot * 8, kAllCtas);
+            if (part == NPART - 1 && (e.z & kCommit0)) umma_commit(bar_accfull);
           }
-          umma_commit_multicast(bar_empty + slot * 8, kAllCtas);
-          if (e.z & kCommit0) umma_commit(bar_accfull);
+          __syncwarp();
+          if (++slot == kNumSlots) { slot = 0; phase ^= 1; }
         }
-        __syncwarp();
-        if (++slot == kNumSlots) { slot = 0; phase ^= 1; }
         if (e.z & kPostWait1) {
           mbar_wait(bar_aready + 8, ph_a1);
           ph_a1 ^= 1;
@@ -449,19 +488,35 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const __grid_constan
         if (real) d = reinterpret_cast<const float4*>(p.draw)[gt * 128 + row];
         const uint32_t h01 = pack_f16x2(d.x * scale, d.y * scale), h23 = pack_f16x2(d.z * scale, d.w * scale);
         *reinterpret_cast<uint4*>(smem + kOffOp + row * 128 + ((0 ^ (row & 7)) << 4)) = make_uint4(h01, h23, 0u, 0u);
+        uint32_t l01 = 0u, l23 = 0u;
+        if constexpr (EXACT) {  // the scale is a power of two: d * scale is exact, its FP16 split as the epilogue's
+          const float2 g01 = unpack_f16x2(h01), g23 = unpack_f16x2(h23);
+          l01 = pack_f16x2(d.x * scale - g01.x, d.y * scale - g01.y);
+          l23 = pack_f16x2(d.z * scale - g23.x, d.w * scale - g23.y);
+          *reinterpret_cast<uint4*>(smem + kOffOp + kTileM * 128 + row * 128 + ((0 ^ (row & 7)) << 4)) = make_uint4(l01, l23, 0u, 0u);
+        }
         if (real) {
-          uint8_t* img = p.rec + gt * kRecBytes + kRecDRaw + img_row_base(16, row);
+          uint8_t* img = p.rec + gt * kRecStride + kRecDRaw + img_row_base(16, row);
           const uint32_t cr = (uint32_t)((row & 63) >> 3);
           *reinterpret_cast<uint16_t*>(img + 0 * 128 + ((cr ^ 0u) << 4)) = (uint16_t)(h01 & 0xFFFFu);
           *reinterpret_cast<uint16_t*>(img + 1 * 128 + ((cr ^ 1u) << 4)) = (uint16_t)(h01 >> 16);
           *reinterpret_cast<uint16_t*>(img + 2 * 128 + ((cr ^ 2u) << 4)) = (uint16_t)(h23 & 0xFFFFu);
           *reinterpret_cast<uint16_t*>(img + 3 * 128 + ((cr ^ 3u) << 4)) = (uint16_t)(h23 >> 16);
+          if constexpr (EXACT) {
+            *reinterpret_cast<uint16_t*>(img + kRecLo + 0 * 128 + ((cr ^ 0u) << 4)) = (uint16_t)(l01 & 0xFFFFu);
+            *reinterpret_cast<uint16_t*>(img + kRecLo + 1 * 128 + ((cr ^ 1u) << 4)) = (uint16_t)(l01 >> 16);
+            *reinterpret_cast<uint16_t*>(img + kRecLo + 2 * 128 + ((cr ^ 2u) << 4)) = (uint16_t)(l23 & 0xFFFFu);
+            *reinterpret_cast<uint16_t*>(img + kRecLo + 3 * 128 + ((cr ^ 3u) << 4)) = (uint16_t)(l23 >> 16);
+          }
         }
       } else if (real) {  // rows 4..15 of the image are zero
-        uint8_t* img = p.rec + gt * kRecBytes + kRecDRaw + img_row_base(16, row);
+        uint8_t* img = p.rec + gt * kRecStride + kRecDRaw + img_row_base(16, row);
         const uint32_t cr = (uint32_t)((row & 63) >> 3);
 #pragma unroll
-        for (int k = 4; k < 16; ++k) *reinterpret_cast<uint16_t*>(img + k * 128 + ((cr ^ (uint32_t)(k & 7)) << 4)) = 0;
+        for (int part = 0; part < NPART; ++part) {
+#pragma unroll
+          for (int k = 4; k < 16; ++k) *reinterpret_cast<uint16_t*>(img + part * kRecLo + k * 128 + ((cr ^ (uint32_t)(k & 7)) << 4)) = 0;
+        }
       }
       fence_proxy_async_smem();
     };
@@ -470,7 +525,7 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const __grid_constan
     for (int j = 0; j < n_tiles_cta; ++j) {
       const int unit = blockIdx.x + (j / tpu) * gridDim.x;
       const bool real = unit < p.n_units;
-      uint8_t* rec = real ? p.rec + ((size_t)unit * tpu + (j % tpu)) * kRecBytes : nullptr;
+      uint8_t* rec = real ? p.rec + ((size_t)unit * tpu + (j % tpu)) * kRecStride : nullptr;
       const uint32_t* masks = reinterpret_cast<const uint32_t*>(rec + kRecMask);
       __syncwarp();
       if (lane == 0) {  // operand of tile j is in place: both gates of step 0
@@ -494,10 +549,14 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const __grid_constan
         {  // half 0: output columns [64 ch, 64 ch + 64).  The FP16 result goes back to TMEM in place: A operand of the next step
            // and (every step, also the last) what the saver warps write to the record.
           const int c0 = 64 * ch;
-          uint32_t ha[16], hb[16];
-          bwd_epi_slice(t_acc + c0, m0, ha, hb);
+          uint32_t ha[16], hb[16], la[16], lb[16];
+          bwd_epi_slice<EXACT>(t_acc + c0, m0, ha, hb, la, lb);
           tmem_st16(t_acc + c0, ha);
           tmem_st16(t_acc + c0 + 16, hb);
+          if constexpr (EXACT) {
+            tmem_st16(t_acc + c0 + 32, la);
+            tmem_st16(t_acc + c0 + 48, lb);
+          }
           tmem_wait_st();
           tc_fence_before_sync();
           __syncwarp();
@@ -508,10 +567,14 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const __grid_constan
         }
         if (two) {  // half 1: columns [128 + 64 ch, ...)
           const int c0 = 128 + 64 * ch;
-          uint32_t ha[16], hb[16];
-          bwd_epi_slice(t_acc + c0, m1, ha, hb);
+          uint32_t ha[16], hb[16], la[16], lb[16];
+          bwd_epi_slice<EXACT>(t_acc + c0, m1, ha, hb, la, lb);
           tmem_st16(t_acc + c0, ha);
           tmem_st16(t_acc + c0 + 16, hb);
+          if constexpr (EXACT) {
+            tmem_st16(t_acc + c0 + 32, la);
+            tmem_st16(t_acc + c0 + 48, lb);
+          }
           tmem_wait_st();
           tc_fence_before_sync();
           __syncwarp();
@@ -539,7 +602,7 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const __grid_constan
     uint32_t sv_ph = 0;  // bit (half * 2 + parity): phase of bar_sv[half][parity]
     for (int j = 0; j < n_tiles_cta; ++j) {
       const int unit = blockIdx.x + (j / tpu) * gridDim.x;
-      uint8_t* rec = unit < p.n_units ? p.rec + ((size_t)unit * tpu + (j % tpu)) * kRecBytes : nullptr;
+      uint8_t* rec = unit < p.n_units ? p.rec + ((size_t)unit * tpu + (j % tpu)) * kRecStride : nullptr;
 #pragma unroll 1
       for (int s = 0; s < kBwdSteps; ++s) {
         const int L = 8 - s, W = rec_width(L);
@@ -556,20 +619,25 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const __grid_constan
             sv_ph ^= bit;
             tc_fence_after_sync();
           }
-          uint32_t v[32];
-          tmem_ld32(t_reg + 64 * i, v);
-          tmem_wait_ld();
-          if (i == n_slices - 1) {  // the whole region has been read
-            tc_fence_before_sync();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(bar_saved + par * 8);
-          }
-          if (img) {
-            uint32_t h0[16], h1[16];
+          // EXACT: two passes per slice (hi columns, then lo columns at +32), so the savers stay at 80 registers
 #pragma unroll
-            for (int k = 0; k < 16; ++k) { h0[k] = v[k]; h1[k] = v[16 + k]; }
-            store_t32(img, row, 64 * i, h0);
-            store_t32(img, row, 64 * i + 32, h1);
+          for (int part = 0; part < NPART; ++part) {
+            uint32_t v[32];
+            tmem_ld32(t_reg + 64 * i + 32 * part, v);
+            tmem_wait_ld();
+            if (i == n_slices - 1 && part == NPART - 1) {  // the whole region has been read
+              tc_fence_before_sync();
+              __syncwarp();
+              if (lane == 0) mbar_arrive(bar_saved + par * 8);
+            }
+            if (img) {
+              uint8_t* dst = img + part * kRecLo;
+              uint32_t h0[16], h1[16];
+#pragma unroll
+              for (int k = 0; k < 16; ++k) { h0[k] = v[k]; h1[k] = v[16 + k]; }
+              store_t32(dst, row, 64 * i, h0);
+              store_t32(dst, row, 64 * i + 32, h1);
+            }
           }
         }
       }
@@ -597,6 +665,15 @@ namespace dw {
 constexpr int kThreads = 192;  // warp 0 producer, warp 1 MMA issuer, warps 2..5 epilogue (one per TMEM lane quadrant)
 constexpr int kStages = 4;
 constexpr int kStageBytes = 16384 + 32768;       // one r-atom (64 sample rows): A [128 features x 128 B], B [<=256 features x 128 B]
+// EXACT (exact-gradient records): a stage holds the hi images as above and the lo images (second record MiB) kStageBytes after
+// them, so 2 stages of 96 KB take the space of 4 x 48 KB.
+__host__ __device__ constexpr int stages(bool exact) { return exact ? 2 : kStages; }
+__host__ __device__ constexpr int stage_bytes(bool exact) { return exact ? 2 * kStageBytes : kStageBytes; }
+__host__ __device__ constexpr int stage_a_off(int part) { return part * kStageBytes; }           // part 0 = hi, 1 = lo
+__host__ __device__ constexpr int stage_b_off(int part) { return part * kStageBytes + 16384; }
+// bytes one stage (one r-atom of one tile) brings in for a job whose B image has b_rows features
+__host__ __device__ constexpr uint32_t stage_tx(bool exact, int b_rows) { return (exact ? 2u : 1u) * (16384u + (uint32_t)b_rows * 128u); }
+static_assert(stages(true) * stage_bytes(true) == kStages * kStageBytes, "both variants share the shared-memory map");
 constexpr int kOffOnes = kStages * kStageBytes;  // [16 rows x 64 r]: row 0 = 1.0 (bias = column sums of dY)
 constexpr int kOffBars = kOffOnes + 2048;
 constexpr int kOffTmemPtr = kOffBars + (2 * kStages + 2) * 8;
@@ -654,7 +731,21 @@ constexpr JobTable make_jobs() {
 static_assert(make_jobs().group_begin[kGroups] == kNumJobs, "job table");
 __constant__ JobTable c_jobs = make_jobs();
 
+}  // namespace dw
+
+__constant__ chain::ProgTable c_chain_prog_x3 = chain::make_prog(true);
+namespace chain {
+template <> __device__ __forceinline__ const ProgTable& prog<false>() { return c_prog; }
+template <> __device__ __forceinline__ const ProgTable& prog<true>() { return c_chain_prog_x3; }
+}  // namespace chain
+
+namespace dw {
+
+// EXACT: exact-gradient records — per ks A_hi·B_hi + A_hi·B_lo + A_lo·B_hi, and A_hi·1 + A_lo·1 for the bias column.
+template <bool EXACT = false>
 __global__ void __launch_bounds__(kThreads, 1) dw_kernel(const __grid_constant__ DwParams p) {
+  constexpr int NSTAGE = stages(EXACT), NPART = EXACT ? 2 : 1;
+  constexpr int kStride = stage_bytes(EXACT);
   extern __shared__ __align__(1024) uint8_t smem[];
   const uint32_t smem_base = smem_u32(smem);
   if ((smem_base & 1023u) != 0u) __trap();
@@ -674,14 +765,14 @@ __global__ void __launch_bounds__(kThreads, 1) dw_kernel(const __grid_constant__
   if (part >= parts || j0 >= j1) return;  // uniform for the whole CTA
   const int job0 = c_jobs.group_begin[group], job1 = c_jobs.group_begin[group + 1];
 
-  const uint32_t bar_full = smem_base + kOffBars;      // [kStages]
-  const uint32_t bar_empty = bar_full + kStages * 8;   // [kStages]
-  const uint32_t bar_accfull = bar_empty + kStages * 8;
+  const uint32_t bar_full = smem_base + kOffBars;      // [NSTAGE]
+  const uint32_t bar_empty = bar_full + NSTAGE * 8;    // [NSTAGE]
+  const uint32_t bar_accfull = bar_empty + NSTAGE * 8;
   const uint32_t bar_accempty = bar_accfull + 8;
   volatile uint32_t* tmem_ptr_s = reinterpret_cast<volatile uint32_t*>(smem + kOffTmemPtr);
 
   if (threadIdx.x == 0) {
-    for (int i = 0; i < kStages; ++i) {
+    for (int i = 0; i < NSTAGE; ++i) {
       mbar_init(bar_full + i * 8, 1);
       mbar_init(bar_empty + i * 8, 1);
     }
@@ -703,7 +794,7 @@ __global__ void __launch_bounds__(kThreads, 1) dw_kernel(const __grid_constant__
 
   auto tile_rec = [&](int j) -> const uint8_t* {
     const int u = j / t_cnt, t = j - u * t_cnt;
-    return p.rec + ((size_t)u * p.tpu + t_base + t) * kRecBytes;
+    return p.rec + ((size_t)u * p.tpu + t_base + t) * rec_stride(EXACT);
   };
 
   if (warp == 0) {
@@ -717,13 +808,17 @@ __global__ void __launch_bounds__(kThreads, 1) dw_kernel(const __grid_constant__
         for (int a = 0; a < 2; ++a) {
           mbar_wait(bar_empty + stage * 8, phase ^ 1);
           if (elect_one()) {
-            const uint32_t sa = smem_base + stage * kStageBytes, sb = sa + 16384;
-            mbar_arrive_expect_tx(bar_full + stage * 8, 16384 + b_bytes);
-            bulk_g2s(sa, rec + J.a_off + a * J.a_rows * 128 + J.a_half * 16384, 16384, bar_full + stage * 8);
-            bulk_g2s(sb, rec + J.b_off + a * J.b_rows * 128, b_bytes, bar_full + stage * 8);
+            const uint32_t st0 = smem_base + stage * kStride;
+            mbar_arrive_expect_tx(bar_full + stage * 8, stage_tx(EXACT, J.b_rows));
+#pragma unroll
+            for (int part = 0; part < NPART; ++part) {  // EXACT: the hi images, then the lo images of the second record MiB
+              const uint8_t* r = rec + part * kRecLo;
+              bulk_g2s(st0 + stage_a_off(part), r + J.a_off + a * J.a_rows * 128 + J.a_half * 16384, 16384, bar_full + stage * 8);
+              bulk_g2s(st0 + stage_b_off(part), r + J.b_off + a * J.b_rows * 128, b_bytes, bar_full + stage * 8);
+            }
           }
           __syncwarp();
-          if (++stage == kStages) { stage = 0; phase ^= 1; }
+          if (++stage == NSTAGE) { stage = 0; phase ^= 1; }
         }
       }
     }
@@ -741,20 +836,29 @@ __global__ void __launch_bounds__(kThreads, 1) dw_kernel(const __grid_constant__
         for (int a = 0; a < 2; ++a) {
           mbar_wait(bar_full + stage * 8, phase);
           tc_fence_after_sync();
-          const uint32_t sa = smem_base + stage * kStageBytes, sb = sa + 16384;
+          const uint32_t sa = smem_base + stage * kStride + stage_a_off(0), sb = smem_base + stage * kStride + stage_b_off(0);
           if (elect_one()) {
             const uint64_t ad = umma_smem_desc_sw128(sa), bd = umma_smem_desc_sw128(sb);
+            const uint32_t sal = smem_base + stage * kStride + stage_a_off(1), sbl = smem_base + stage * kStride + stage_b_off(1);
+            const uint64_t adl = umma_smem_desc_sw128(sal), bdl = umma_smem_desc_sw128(sbl);  // EXACT only
 #pragma unroll
             for (int ks = 0; ks < 4; ++ks) {
               const uint32_t accf = ((j - j0) | a | ks) ? 1u : 0u;
               umma_ss(tmem_base, ad + (uint64_t)(ks * 2), bd + (uint64_t)(ks * 2), idesc, accf);
-              if (J.bias_layer >= 0) umma_ss(tmem_base + kBiasCol, ad + (uint64_t)(ks * 2), ones_desc + (uint64_t)(ks * 2), idesc_bias, accf);
+              if constexpr (EXACT) {
+                umma_ss(tmem_base, ad + (uint64_t)(ks * 2), bdl + (uint64_t)(ks * 2), idesc, 1u);
+                umma_ss(tmem_base, adl + (uint64_t)(ks * 2), bd + (uint64_t)(ks * 2), idesc, 1u);
+              }
+              if (J.bias_layer >= 0) {
+                umma_ss(tmem_base + kBiasCol, ad + (uint64_t)(ks * 2), ones_desc + (uint64_t)(ks * 2), idesc_bias, accf);
+                if (EXACT) umma_ss(tmem_base + kBiasCol, adl + (uint64_t)(ks * 2), ones_desc + (uint64_t)(ks * 2), idesc_bias, 1u);
+              }
             }
             umma_commit(bar_empty + stage * 8);
             if (j == j1 - 1 && a == 1) umma_commit(bar_accfull);
           }
           __syncwarp();
-          if (++stage == kStages) { stage = 0; phase ^= 1; }
+          if (++stage == NSTAGE) { stage = 0; phase ^= 1; }
         }
       }
       acc_phase ^= 1;
@@ -981,10 +1085,46 @@ int debug_jobs_dw(int index, uint32_t* out) {
   return 10;
 }
 
+// Exact-gradient chain program, one entry per LOAD (two per unit: hi, lo): the unit's program entry with w = this part's offset in
+// stream_bwd_x3, then part, the A operand's lo TMEM column (0xFFFFFFFF: from the shared-memory operand), the kernel's shared-memory
+// bytes, ring slot bytes, ring slots, d raw operand buffers.
+int debug_prog_chain_exact(int index, uint32_t* out) {
+  constexpr chain::ProgTable t = chain::make_prog(true);
+  if (index < 0) return 2 * chain::kTileUnits;
+  if (index >= 2 * chain::kTileUnits) return -1;
+  const chain::ProgEntry& e = t.e[index / 2];
+  const uint32_t part = (uint32_t)(index & 1), bytes = (e.w >> 20) * 128u;
+  out[0] = e.x; out[1] = e.y; out[2] = e.z;
+  out[3] = ((((e.w & 0xFFFFFu) << 4) + part * bytes) >> 4) | (e.w & ~0xFFFFFu);
+  out[4] = part;
+  out[5] = (e.z & chain::kFromOp) ? 0xFFFFFFFFu : (e.y >> 16) + 32u;
+  out[6] = (uint32_t)chain::smem_bytes(true); out[7] = (uint32_t)kMaxUnitBytes; out[8] = (uint32_t)chain::kNumSlots;
+  out[9] = (uint32_t)chain::op_buffers(true);
+  return 10;
+}
+// Exact-gradient weight-gradient stage layout, one entry per job: shared-memory offsets inside a stage of A hi, B hi, A lo, B lo,
+// stage bytes, stages, bytes the job loads per tile (two r-atoms), the same for the FP16 kernel, the kernel's shared-memory bytes,
+// record offset of the lo MiB.
+int debug_stages_dw_exact(int index, uint32_t* out) {
+  constexpr dw::JobTable t = dw::make_jobs();
+  if (index < 0) return dw::kNumJobs;
+  if (index >= dw::kNumJobs) return -1;
+  const int b_rows = t.j[index].b_rows;
+  out[0] = dw::stage_a_off(0); out[1] = dw::stage_b_off(0); out[2] = dw::stage_a_off(1); out[3] = dw::stage_b_off(1);
+  out[4] = (uint32_t)dw::stage_bytes(true); out[5] = (uint32_t)dw::stages(true);
+  out[6] = 2u * dw::stage_tx(true, b_rows); out[7] = 2u * dw::stage_tx(false, b_rows);
+  out[8] = (uint32_t)dw::kSmemBytes; out[9] = (uint32_t)kRecLo;
+  return 10;
+}
+
 cudaError_t train_kernels_setup() {
-  cudaError_t e = cudaFuncSetAttribute(chain::chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, chain::kSmemBytes);
+  cudaError_t e = cudaFuncSetAttribute(chain::chain_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, chain::kSmemBytes);
   if (e != cudaSuccess) return e;
-  return cudaFuncSetAttribute(dw::dw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, dw::kSmemBytes);
+  e = cudaFuncSetAttribute(chain::chain_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, chain::smem_bytes(true));
+  if (e != cudaSuccess) return e;
+  e = cudaFuncSetAttribute(dw::dw_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, dw::kSmemBytes);
+  if (e != cudaSuccess) return e;
+  return cudaFuncSetAttribute(dw::dw_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dw::kSmemBytes);
 }
 
 cudaError_t launch_composite_bwd(const CompBwdParams& q, float* scal, cudaStream_t st, long long* launches) {
@@ -996,7 +1136,7 @@ cudaError_t launch_composite_bwd(const CompBwdParams& q, float* scal, cudaStream
   return cudaGetLastError();
 }
 
-cudaError_t launch_chain(const ChainParams& p, int num_sms, cudaStream_t st, long long* launches) {
+cudaError_t launch_chain(const ChainParams& p, bool exact_grad, int num_sms, cudaStream_t st, long long* launches) {
   int grid = p.n_units < num_sms ? p.n_units : num_sms;
   if (grid <= 0) return cudaSuccess;
   grid = (grid + chain::kCluster - 1) / chain::kCluster * chain::kCluster;
@@ -1004,7 +1144,7 @@ cudaError_t launch_chain(const ChainParams& p, int num_sms, cudaStream_t st, lon
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(grid);
   cfg.blockDim = dim3(chain::kThreads);
-  cfg.dynamicSmemBytes = chain::kSmemBytes;
+  cfg.dynamicSmemBytes = exact_grad ? chain::smem_bytes(true) : chain::kSmemBytes;
   cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
@@ -1013,7 +1153,7 @@ cudaError_t launch_chain(const ChainParams& p, int num_sms, cudaStream_t st, lon
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, chain::chain_kernel, p);
+  cudaError_t e = exact_grad ? cudaLaunchKernelEx(&cfg, chain::chain_kernel<true>, p) : cudaLaunchKernelEx(&cfg, chain::chain_kernel<false>, p);
   ++*launches;
   return e != cudaSuccess ? e : cudaGetLastError();
 }
@@ -1041,13 +1181,14 @@ int debug_dw_split(uint32_t* io) {  // in: num_sms, tiles of network 0, tiles of
   return 3;
 }
 
-cudaError_t launch_dw(const DwParams& p_in, int num_sms, cudaStream_t st, long long* launches) {
+cudaError_t launch_dw(const DwParams& p_in, bool exact_grad, int num_sms, cudaStream_t st, long long* launches) {
   DwParams p = p_in;
   const long long tot0 = (long long)p.n_units * p.t_cnt[0], tot1 = (long long)p.n_units * p.t_cnt[1];
   if (tot0 + tot1 <= 0) return cudaSuccess;
   dw_split(num_sms, tot0, tot1, &p.parts[0], &p.parts[1]);
   if (p.parts[0] + p.parts[1] < 1) return cudaSuccess;
-  dw::dw_kernel<<<(p.parts[0] + p.parts[1]) * dw::kGroups, dw::kThreads, dw::kSmemBytes, st>>>(p);
+  if (exact_grad) dw::dw_kernel<true><<<(p.parts[0] + p.parts[1]) * dw::kGroups, dw::kThreads, dw::kSmemBytes, st>>>(p);
+  else dw::dw_kernel<false><<<(p.parts[0] + p.parts[1]) * dw::kGroups, dw::kThreads, dw::kSmemBytes, st>>>(p);
   ++*launches;
   return cudaGetLastError();
 }

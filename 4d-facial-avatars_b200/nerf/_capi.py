@@ -8,7 +8,7 @@ LIB_PATH = os.environ.get("NFB_LIB") or os.path.join(os.path.dirname(_HERE), "li
 
 NFB_OK = 0
 NFB_NET_COARSE, NFB_NET_FINE = 0, 1
-NFB_PREC_FAST, NFB_PREC_EXACT = 0, 1
+NFB_PREC_FAST, NFB_PREC_EXACT, NFB_PREC_EXACT_GRAD = 0, 1, 2
 
 EXPORTS = ["nfb_version", "nfb_strerror", "nfb_last_cuda_error", "nfb_create", "nfb_destroy", "nfb_load_weights",
            "nfb_set_frame", "nfb_render_forward", "nfb_render_frame_host", "nfb_launch_count", "nfb_host_linspace",

@@ -16,14 +16,20 @@ PARAM_ORDER = ([f"layers_xyz.{i}.{k}" for i in range(6) for k in ("weight", "bia
                + ["fc_rgb.weight", "fc_rgb.bias"])
 
 _precision = os.environ.get("NFB_PRECISION", "fast")
+_PREC_CODES = {"fast": capi.NFB_PREC_FAST, "exact": capi.NFB_PREC_EXACT, "exact_grad": capi.NFB_PREC_EXACT_GRAD}
 
 
 def set_precision(mode: str):
-    """'fast' = FP16 operands / FP32 accumulate; 'exact' = 3-pass FP16 hi/lo split (see include/nfb.h)."""
+    """'fast' = FP16 operands / FP32 accumulate; 'exact' = 3-pass FP16 hi/lo split of the forward (see include/nfb.h);
+    'exact_grad' = 'exact', and training gradients computed from hi/lo operands as well (twice the record memory)."""
     global _precision
-    if mode not in ("fast", "exact"):
-        raise ValueError("precision must be 'fast' or 'exact'")
+    if mode not in _PREC_CODES:
+        raise ValueError("precision must be 'fast', 'exact' or 'exact_grad'")
     _precision = mode
+
+
+def _prec_code(prec):
+    return _PREC_CODES.get(prec, capi.NFB_PREC_FAST)
 
 
 def get_precision() -> str:
@@ -157,7 +163,7 @@ class Renderer:
             keep.append(dz)
         prec = precision or _precision
         sm = capi.NfbSampling(num_coarse, num_fine, int(bool(perturb)), float(noise_std), int(bool(white_bkgd)), 0,
-                              capi.NFB_PREC_EXACT if prec == "exact" else capi.NFB_PREC_FAST,
+                              _prec_code(prec),
                               self.linspace(num_coarse).data_ptr(),
                               self.linspace(num_fine).data_ptr() if has_fine else None)
         nz = capi.NfbNoise()
@@ -298,7 +304,7 @@ class Renderer:
         prec = precision or _precision
         has_fine = num_fine > 0
         sm = capi.NfbSampling(num_coarse, num_fine, 0, 0.0, int(bool(white_bkgd)), 0,
-                              capi.NFB_PREC_EXACT if prec == "exact" else capi.NFB_PREC_FAST,
+                              _prec_code(prec),
                               self.linspace(num_coarse).data_ptr(), self.linspace(num_fine).data_ptr() if has_fine else None)
         o = capi.NfbOutputs(views["rgb_coarse"].data_ptr(), views["disp_coarse"].data_ptr(), views["acc_coarse"].data_ptr(),
                             views["rgb_fine"].data_ptr() if has_fine else None,
@@ -318,7 +324,7 @@ class Renderer:
         """Host-buffer end-to-end call (bench e2e leg).  All tensors are CPU (ideally pinned) FP32."""
         prec = precision or _precision
         sm = capi.NfbSampling(num_coarse, num_fine, 0, 0.0, int(bool(white_bkgd)), 0,
-                              capi.NFB_PREC_EXACT if prec == "exact" else capi.NFB_PREC_FAST,
+                              _prec_code(prec),
                               self.linspace(num_coarse).data_ptr(),
                               self.linspace(num_fine).data_ptr() if num_fine > 0 else None)
         pose_a = (C.c_float * 12)(*[float(v) for v in pose.reshape(-1)[:12]])

@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define NFB_VERSION 120
+#define NFB_VERSION 121
 
 typedef struct NfbHandle NfbHandle;
 
@@ -42,10 +42,14 @@ enum {
 enum { NFB_NET_COARSE = 0, NFB_NET_FINE = 1 };
 
 /* Arithmetic used by the tensor-core MLP.
- *   NFB_PREC_FAST  : FP16 operands (round-to-nearest), FP32 accumulate, one tcgen05 pass.
- *   NFB_PREC_EXACT : every operand split x = hi + lo in FP16; hi*hi + hi*lo + lo*hi, FP32
- *                    accumulate (3 tcgen05 passes, ~2^-21 relative operand error). */
-enum { NFB_PREC_FAST = 0, NFB_PREC_EXACT = 1 };
+ *   NFB_PREC_FAST       : FP16 operands (round-to-nearest), FP32 accumulate, one tcgen05 pass.
+ *   NFB_PREC_EXACT      : every operand split x = hi + lo in FP16; hi*hi + hi*lo + lo*hi, FP32
+ *                         accumulate (3 tcgen05 passes, ~2^-21 relative operand error).  In training
+ *                         only the forward: nfb_render_backward carries FP16 operands (~2^-11).
+ *   NFB_PREC_EXACT_GRAD : NFB_PREC_EXACT for rendering (same kernel, bit-identical outputs); after a
+ *                         nfb_render_forward_train in this mode the backward's dX chain and weight-gradient
+ *                         GEMMs use split operands as well (hi+lo records, see nfb_render_forward_train). */
+enum { NFB_PREC_FAST = 0, NFB_PREC_EXACT = 1, NFB_PREC_EXACT_GRAD = 2 };
 
 /* Encoder / conditioning dimensions; mirrors the constructor arguments of
  * ConditionalBlendshapePaperNeRFModel (models.py:193-206).  Only the shipped paper configuration
@@ -165,7 +169,11 @@ int nfb_render_forward(NfbHandle* h, const NfbRays* rays, const NfbSampling* sam
  * Memory: when the records of the whole call would exceed the budget (environment NFB_TRAIN_MEM_MB, default 60 % of the free
  * device memory) — e.g. a full frame rendered with gradients enabled — the forward only renders (evaluation kernel) and the
  * backward re-runs the training forward chunk by chunk inside the budget: same gradients, one extra forward; the caller must
- * then keep the forward's input buffers alive until the backward, and explicit rays are required. */
+ * then keep the forward's input buffers alive until the backward, and explicit rays are required.
+ * NFB_PREC_EXACT_GRAD: each tile record is 2 MiB — the first MiB exactly as in NFB_PREC_EXACT, the second the lo parts
+ * lo = fp16(x - float(hi)) of every image (activations, encodings and the backward's gradients) at the same offsets
+ * (nfb_layout.h kRecLo) — so records take twice the memory (2048 rays at 64+64 samples: 6 GiB), the memory budget above covers
+ * half as many rays per chunk, and the backward moves about twice the record bytes. */
 int nfb_render_forward_train(NfbHandle* h, const NfbRays* rays, const NfbSampling* sampling,
                              const NfbNoise* noise /* nullable */, const NfbOutputs* out, void* stream);
 
@@ -286,7 +294,8 @@ int nfb_host_map_cdf(const NfbRayMap* map, const long long* zeroed_sorted, int n
 
 /* Test hook: device pointers of the training state (valid until the next forward_train on the handle). */
 typedef struct {
-  const uint8_t* records;      /* n_tiles records of record_bytes (layout: nfb_layout.h kRec*) */
+  const uint8_t* records;      /* n_tiles records of record_bytes (layout: nfb_layout.h kRec*; 2 MiB with the lo MiB at kRecLo
+                                  after an NFB_PREC_EXACT_GRAD forward) */
   long long n_tiles;
   int32_t record_bytes;
   const float* d_raw;          /* [n_tiles][128][4] dL/d(rgb_raw, sigma_raw), unscaled */
@@ -314,7 +323,10 @@ int nfb_render_frame_host(NfbHandle* h, const float pose[12], const double intri
  * 1 = two-tile render program (word 4 = half-step group), 2 = backward chain program (each: idesc, TMEM columns, flags,
  * (stream offset / 16) | rows << 20), 3 = weight-gradient jobs (a_off, a_rows, a_half, b_off, b_rows, bias_layer, out_off,
  * out_ld, out_row0, group), 4 = the CTA split of the weight-gradient launch (in/out: out[0..2] = SMs, tiles of network 0, tiles of
- * network 1 -> parts of network 0, parts of network 1, job groups per part), 1000 + 100 n_iter + 10 Tc + Tf = the pipelined render kernel's job sequence for a CTA with n_iter units of work and
+ * network 1 -> parts of network 0, parts of network 1, job groups per part), 5 = exact-gradient chain program (one entry per hi or
+ * lo load: the entry of 2 with the stream_bwd_x3 offset, part, lo A column, shared-memory bytes, slot bytes, slots, operand buffers),
+ * 6 = exact-gradient weight-gradient stages per job (stage offsets of A hi, B hi, A lo, B lo, stage bytes, stages, bytes per tile,
+ * bytes per tile of the FP16 kernel, shared-memory bytes, lo record offset), 1000 + 100 n_iter + 10 Tc + Tf = the pipelined render kernel's job sequence for a CTA with n_iter units of work and
  * Tc / Tf tile pairs per pass (unit iteration, pass, tile, then the kernel's shared-memory bytes and row limits).  index < 0: returns the number of entries; otherwise fills out[0..] (out_words >= 10) and returns
  * the number of words written, or -1. */
 int nfb_debug_schedule(int which, int index, uint32_t* out, int out_words);
