@@ -211,43 +211,13 @@ def test_chain_gradients_exact(ctx):
 def _masked_reference(ctx):
     """The FP32 reference with the kernel's ReLU decisions (decoded from the records) in place of a > 0, so that a
     pre-activation within rounding of zero cannot stand in for arithmetic error.  Returns (grads_c, grads_f, d latent)."""
-    F = torch.nn.functional
     masks = _mask_bits(ctx.records, ctx.n_tiles)
     pc = {k: v.detach().clone().requires_grad_(True) for k, v in ctx.mc.named_parameters()}
     pf = {k: v.detach().clone().requires_grad_(True) for k, v in ctx.mf.named_parameters()}
     lat = ctx.latent.clone().requires_grad_(True)
-    rays, n = ctx.rays, ctx.n
-    ro, rd = rays[:, :3], rays[:, 3:6]
-    dir_cols = torch.cat((rays[:, 5:6], torch.full_like(rays[:, :1], 0.2), torch.full_like(rays[:, :1], 0.8)), dim=-1)
-
-    def mlp(p, x, pas):
-        tile, row = ctx.map[pas]
-        m = [_layer_mask(masks, tile, row, layer).float() for layer in range(9)]
-        xyz, dirs = x[..., :63], x[..., 63:]
-        rows = xyz.shape[0]
-        cond = torch.cat(((ctx.expr * 1 / 3).reshape(1, -1).expand(rows, -1), lat.reshape(1, -1).expand(rows, -1)), dim=1)
-        initial = torch.cat((xyz, cond), dim=1)
-        h = initial
-        for i in range(6):
-            h = F.linear(torch.cat((initial, h), dim=-1) if i == 3 else h, p[f"layers_xyz.{i}.weight"], p[f"layers_xyz.{i}.bias"]) * m[i]
-        feat = F.linear(h, p["fc_feat.weight"], p["fc_feat.bias"])
-        sigma = F.linear(feat, p["fc_alpha.weight"], p["fc_alpha.bias"])
-        g = F.linear(torch.cat((feat, dirs), dim=-1), p["layers_dir.0.weight"], p["layers_dir.0.bias"]) * m[6]
-        g = F.linear(g, p["layers_dir.1.weight"], p["layers_dir.1.bias"]) * m[7]
-        g = F.linear(g, p["layers_dir.2.weight"], p["layers_dir.2.bias"]) * m[8]
-        return torch.cat((F.linear(g, p["fc_rgb.weight"], p["fc_rgb.bias"]), sigma), dim=-1)
-
-    def one_pass(p, z, pas, noise):
-        s = z.shape[1]
-        pts = ro[:, None, :] + rd[:, None, :] * z[:, :, None]
-        x = torch.cat((TR._posenc(pts.reshape(-1, 3), 10, True),
-                       TR._posenc(dir_cols[:, None, :].expand(n, s, 3).reshape(-1, 3), 4, False)), dim=-1)
-        raw = mlp(p, x, pas).reshape(n, s, 4)
-        return TR._composite(raw, z, rd, 0.1, noise, False, ctx.bg)
-
-    rgb_c, disp_c, acc_c, _ = one_pass(pc, ctx.z_c, 0, ctx.nz["n_c"])
-    rgb_f, disp_f, acc_f, w = one_pass(pf, ctx.z_f, 1, ctx.nz["n_f"])
-    outs = [rgb_c, disp_c, acc_c, rgb_f, disp_f, acc_f, w[:, -1]]
+    m = {key: [_layer_mask(masks, *ctx.map[pas], layer) for layer in range(9)] for pas, key in ((0, "coarse"), (1, "fine"))}
+    outs = TR.render_at_depths(ctx.rays, pc, pf, ctx.expr, lat, ctx.z_c, ctx.z_f, 0.2, 0.8, 0.1, ctx.nz, False, ctx.bg, None,
+                               masks=m)
     torch.autograd.backward(outs, ctx.gouts)
     return [pc[k].grad for k in TR.PARAM_ORDER], [pf[k].grad for k in TR.PARAM_ORDER], lat.grad
 

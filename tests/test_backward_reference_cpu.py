@@ -96,3 +96,47 @@ def test_torch_reference_gradients_equal_reference_autograd(name, monkeypatch):
     lat_ref = g("grad_latent")
     close(lat.grad, lat_ref, "latent")
     assert float(lat_ref.abs().max()) > 0
+
+
+@pytest.mark.parametrize("white,use_bg", [(False, True), (True, False)], ids=["bg", "white_nobg"])
+def test_masked_reference_reproduces_unmasked_gradients(white, use_bg):
+    """render_at_depths(masks=...) with the ReLU decisions a > 0 of an unmasked run gives, in FP64, the unmasked run's outputs and
+    gradients exactly: the masked reference the GPU tests evaluate with the kernel's own decisions differs from the plain one only
+    where those decisions differ."""
+    torch.manual_seed(0)
+    n, nc, nf, near, far = 5, 16, 24, 0.2, 0.8
+    fr = O.synthetic_frame(7, 1, n)
+    ro, rd = (t.reshape(-1, 3).double() for t in O.ray_bundle(1, n, fr["intrinsics"], fr["pose"]))
+    rays = torch.cat((ro, rd, torch.full((n, 1), near, dtype=torch.float64), torch.full((n, 1), far, dtype=torch.float64)), dim=-1)
+    z_c = near + (far - near) * torch.sort(torch.rand(n, nc, dtype=torch.float64), dim=-1).values
+    z_f = torch.sort(torch.cat((z_c, near + (far - near) * torch.rand(n, nf, dtype=torch.float64)), dim=-1), dim=-1).values
+    noise = {"n_c": torch.randn(n, nc, dtype=torch.float64), "n_f": torch.randn(n, nc + nf, dtype=torch.float64)}
+    bg = fr["bg"].reshape(-1, 3).double() if use_bg else None
+    dir_z = torch.rand(n, dtype=torch.float64) * 2.0 - 1.0
+    expr = fr["expr"].double()
+    params = [{k: v.double() for k, v in O.random_init_params(seed).items()} for seed in (100, 101)]
+
+    def run(masks):
+        lc, lf = ({k: v.clone().requires_grad_(True) for k, v in p.items()} for p in params)
+        lat = fr["latent"].double().requires_grad_(True)
+        taps = {}
+        out = TR.render_at_depths(rays, lc, lf, expr, lat, z_c, z_f, near, far, 0.1, noise, white, bg, dir_z, taps, masks)
+        gen = torch.Generator().manual_seed(3)
+        torch.autograd.backward(out, [torch.randn(o.shape, generator=gen, dtype=torch.float64) for o in out])
+        grads = [leaves[k].grad for leaves in (lc, lf) for k in TR.PARAM_ORDER] + [lat.grad]
+        return [o.detach() for o in out], grads, taps
+
+    out, grads, taps = run(None)
+    masks = {key: [taps[key][f"a{i}"].detach() > 0 for i in range(9)] for key in ("coarse", "fine")}
+    assert all(bool(m.any()) and not bool(m.all()) for ms in masks.values() for m in ms)
+    m_out, m_grads, m_taps = run(masks)
+    for a, b in zip(out, m_out):
+        assert torch.equal(a, b)
+    for k, a, b in zip([f"coarse {k}" for k in TR.PARAM_ORDER] + [f"fine {k}" for k in TR.PARAM_ORDER] + ["latent"], grads, m_grads):
+        assert (a is None) == (b is None), k
+        if a is not None:
+            assert a.dtype == torch.float64 and torch.equal(a, b), k
+    for key in ("coarse", "fine"):
+        for i in range(9):
+            assert torch.equal(taps[key][f"a{i}"].grad, m_taps[key][f"a{i}"].grad), (key, i)
+        assert torch.equal(taps[key]["raw"].grad, m_taps[key]["raw"].grad), key

@@ -1,6 +1,6 @@
-"""Plain-PyTorch FP32 restatement of one training forward/backward of the render path AT GIVEN sample depths — test
-infrastructure only (the floating-point reference for the fused backward kernels; runs on whatever device its inputs live
-on).  Follows train_utils.py:36-162, volume_rendering_utils.py:7-75, models.py:236-261; resampled depths carry no
+"""Plain-PyTorch restatement of one training forward/backward of the render path AT GIVEN sample depths — test
+infrastructure only (the floating-point reference for the fused backward kernels; runs on whatever device and in whatever
+floating-point type its inputs have: FP32 or FP64).  Follows train_utils.py:36-162, volume_rendering_utils.py:7-75, models.py:236-261; resampled depths carry no
 gradient (`z_samples.detach()`, train_utils.py:124)."""
 import torch
 
@@ -17,8 +17,9 @@ def _posenc(x, n_freq, include_input):
     return torch.cat(parts, dim=-1)
 
 
-def _mlp(p, x, expr, latent, taps=None):
-    """taps (dict): receives the post-activation outputs h0..h5, g0..g2 and the pre-activations a0..a8 (retain_grad)."""
+def _mlp(p, x, expr, latent, taps=None, masks=None):
+    """taps (dict): receives the post-activation outputs h0..h5, g0..g2 and the pre-activations a0..a8 (retain_grad).
+    masks: None, or the nine ReLU decisions ([rows, width] bool, layers a0..a8) to apply in place of a > 0."""
     F = torch.nn.functional
     xyz, dirs = x[..., :63], x[..., 63:]
     rows = xyz.shape[0]
@@ -29,7 +30,7 @@ def _mlp(p, x, expr, latent, taps=None):
         if taps is not None:
             a.retain_grad()
             taps[name_pre] = a
-        h = F.relu(a)
+        h = F.relu(a) if masks is None else a * masks[int(name_pre[1:])]
         if taps is not None:
             taps[name_post] = h
         return h
@@ -74,12 +75,12 @@ def _composite(raw, z, rd, noise_std, noise, white_bkgd, bg):
     return rgb, disp, acc, w
 
 
-def _pass(p, z, rays, dir_cols, expr, latent, noise_std, noise, white_bkgd, bg, taps=None):
+def _pass(p, z, rays, dir_cols, expr, latent, noise_std, noise, white_bkgd, bg, taps=None, masks=None):
     ro, rd = rays[:, :3], rays[:, 3:6]
     n, s = z.shape
     pts = ro[:, None, :] + rd[:, None, :] * z[:, :, None]
     x = torch.cat((_posenc(pts.reshape(-1, 3), 10, True), _posenc(dir_cols[:, None, :].expand(n, s, 3).reshape(-1, 3), 4, False)), dim=-1)
-    raw = _mlp(p, x, expr, latent, taps).reshape(n, s, 4)
+    raw = _mlp(p, x, expr, latent, taps, masks).reshape(n, s, 4)
     if taps is not None:
         raw.retain_grad()
         taps["raw"] = raw
@@ -87,17 +88,21 @@ def _pass(p, z, rays, dir_cols, expr, latent, noise_std, noise, white_bkgd, bg, 
 
 
 def render_at_depths(rays, params_c, params_f, expr, latent, z_c, z_f, near, far, noise_std=0.0, noise=None,
-                     white_bkgd=False, bg=None, dir_z=None, taps=None):
+                     white_bkgd=False, bg=None, dir_z=None, taps=None, masks=None):
     """rays [N,8]; params_*: dict name -> tensor (requires_grad leaves).  Returns the 7-tuple as differentiable tensors.
-    `taps` (dict): receives per-pass intermediate tensors under "coarse"/"fine"."""
+    `taps` (dict): receives per-pass intermediate tensors under "coarse"/"fine".  `masks` (dict): per pass ("coarse"/"fine")
+    the nine [N*S, width] ReLU decisions to use instead of a > 0 (rows ray-major: ray i, sample j at i*S + j)."""
     dir_cols = torch.cat((dir_z.reshape(-1, 1) if dir_z is not None else rays[:, 5:6],
                           torch.full_like(rays[:, :1], near), torch.full_like(rays[:, :1], far)), dim=-1)
     nz = noise or {}
+    mk = masks or {}
     tc = taps.setdefault("coarse", {}) if taps is not None else None
-    rgb_c, disp_c, acc_c, w = _pass(params_c, z_c, rays, dir_cols, expr, latent, noise_std, nz.get("n_c"), white_bkgd, bg, tc)
+    rgb_c, disp_c, acc_c, w = _pass(params_c, z_c, rays, dir_cols, expr, latent, noise_std, nz.get("n_c"), white_bkgd, bg, tc,
+                                    mk.get("coarse"))
     outs = [rgb_c, disp_c, acc_c, None, None, None, w[:, -1]]
     if params_f is not None:
         tf = taps.setdefault("fine", {}) if taps is not None else None
-        rgb_f, disp_f, acc_f, w = _pass(params_f, z_f, rays, dir_cols, expr, latent, noise_std, nz.get("n_f"), white_bkgd, bg, tf)
+        rgb_f, disp_f, acc_f, w = _pass(params_f, z_f, rays, dir_cols, expr, latent, noise_std, nz.get("n_f"), white_bkgd, bg, tf,
+                                        mk.get("fine"))
         outs[3:7] = [rgb_f, disp_f, acc_f, w[:, -1]]
     return outs
